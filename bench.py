@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — critic pairs/sec, fused fwd+bwd MI critic/estimator (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one pass of the hot path (single pass: sampled softmax references -> score tiles -> loss statistics and
@@ -24,6 +24,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the source tree (it may be read-only)
 # NCCL prints its version banner on stdout at NCCL_DEBUG=VERSION; the contract is ONE JSON line there
 if os.environ.get("NCCL_DEBUG", "").upper() in ("", "VERSION"):
     os.environ["NCCL_DEBUG"] = "WARN"
@@ -47,7 +48,15 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-variants", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned to DIR/<name>.npy: the loss "
+                         "statistics, dW and a fixed seeded sample of the rows of dX and dY, at most 64 MB in all")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return a
 
 
 def peaks():
@@ -99,7 +108,7 @@ def time_cpu(a, steps, warmup, budget_s=25.0):
         t0 = time.perf_counter()
         step()
         ts.append(time.perf_counter() - t0)
-        if time.time() - t_start > budget_s:
+        if budget_s is not None and time.time() - t_start > budget_s:
             break
     t = sum(ts) / len(ts)
     return {"value": B * B / t, "unit": UNIT, "cores": torch.get_num_threads(), "kind": "port",
@@ -137,7 +146,7 @@ def run_reference(a):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    cb = time_cpu(a, a.steps, a.warmup, budget_s=120.0)
+    cb = time_cpu(a, a.steps, a.warmup, budget_s=None)        # --steps timed steps, however long they take
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus,
         "steps": cb["steps"], "warmup": max(1, a.warmup), "ms_per_step": cb["ms_per_step"], "higher_is_better": True,
@@ -241,6 +250,53 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons),
                 "source": "NVML in-process, 50 ms period" if self.nvml is not None else "nvidia-smi -lms 100"}
+
+
+# ------------------------------------------------------------------------------------------- outputs
+DUMP_BYTES = 64 << 20          # what --dump-outputs may write in all
+
+
+def dump_outputs(path, last, B, off, world, rank):
+    """Writes what the timed call returned in its last step as ``path/<name>.npy`` (fp32 / fp64), so that two builds run
+    with the same arguments (hence the same seeded inputs) can be compared output for output:
+      loss_out (N = 1: the fp64 [8] loss vector) or one fp64 file per entry of the statistics dict (N > 1);
+      dX, dY: rows of the global batch, dW: rows of the [D, D] gradient (summed over ranks).
+    Each of dX, dY, dW keeps at most a third of DUMP_BYTES: a larger one is cut to a fixed seeded sample of its rows, the
+    same rows for the same --batch / --dim, sorted (256 MB each of dX and dY at the default size).  dX and dY are gathered
+    from every rank's shard, so every rank calls this; rank 0 writes."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    stats, dX, dY, dW = last
+    Bl, D = dX.shape
+    cap = (DUMP_BYTES - (1 << 20)) // (3 * 4 * D)      # fp32 rows per array; 1 MB left for the statistics and file headers
+
+    def sample(n):
+        if n <= cap:
+            return torch.arange(n)
+        return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:cap].sort().values
+
+    rows = sample(B)
+    mine = (rows >= off) & (rows < off + Bl)
+    out = {}
+    for name, g in (("dX", dX), ("dY", dY)):
+        s = torch.zeros(len(rows), D, dtype=g.dtype, device=g.device)
+        s[mine.to(g.device)] = g[(rows[mine] - off).to(g.device)]
+        if world > 1:
+            dist.all_reduce(s)                         # every sampled row is held by exactly one rank, zeros elsewhere
+        out[name] = s
+    if dW is not None:
+        out["dW"] = dW[sample(D).to(dW.device)]
+    if isinstance(stats, dict):
+        out.update(stats)
+    else:
+        out["loss_out"] = stats
+    if rank != 0:
+        return
+    os.makedirs(path, exist_ok=True)
+    for name, t in out.items():
+        t = torch.as_tensor(t).detach().cpu()
+        np.save(os.path.join(path, name + ".npy"), (t if t.dtype == torch.float64 else t.float()).numpy())
 
 
 # ------------------------------------------------------------------------------------------- GPU arm
@@ -353,6 +409,8 @@ def run_ours(a):
     lib.mi_profile_read(ms, cnt)
     lib.mi_set_profiling(0)
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, last, B, off, world, rank)
     ms_per_step = total_ms / a.steps
     value = B * B / (ms_per_step * 1e-3)
     if world == 1:
