@@ -11,6 +11,8 @@ point is the critic slot:
     --critic fused   mi_b200.FusedCritic + dv_bound_loss on the PairBatch handle  (this repo)
     --critic mlp     mi_b200.FusedMLPCritic(768, (1024, 512)): the reference's OWN mi_discriminator (main_utils.py:77), fused
     --critic mlp_pairs  the same nn.Sequential on the explicit pair tensor (what the reference executes, torch ops)
+    --critic mlp_sharded  FusedMLPCritic through sharded_mi_loss: at N > 1 the loss of the GLOBAL batch (every rank's rows
+                     against every rank's texts), not per-rank batches
     --critic pairs   the same separable critic on the explicit [B + N_neg, 2D] pair tensor (torch ops;
                      the reference's formulation with the O(B^2) loop replaced by one gather)
 
@@ -78,7 +80,7 @@ class TextEncoder(nn.Module):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--critic", default="fused", choices=["fused", "pairs", "mlp", "mlp_pairs"])
+    ap.add_argument("--critic", default="fused", choices=["fused", "pairs", "mlp", "mlp_pairs", "mlp_sharded"])
     ap.add_argument("--estimator", default="dv")
     ap.add_argument("--batch", type=int, default=256, help="per GPU")
     ap.add_argument("--steps", type=int, default=5)
@@ -99,7 +101,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     torch.manual_seed(0)
     img_enc, txt_enc = ImageEncoder().to(dev), TextEncoder(a.bert_layers).to(dev)
-    if a.critic in ("mlp", "mlp_pairs"):                            # the mi_discriminator slot (main_utils.py:77)
+    if a.critic in ("mlp", "mlp_pairs", "mlp_sharded"):             # the mi_discriminator slot (main_utils.py:77)
         critic = mi_b200.FusedMLPCritic(768, (1024, 512), precision="fast").to(dev)
     else:
         critic = mi_b200.FusedCritic(768, "bilinear").to(dev)
@@ -126,9 +128,9 @@ def main():
         emb_img, emb_txt = img_enc(img), txt_enc(ids, mask, seg)     # main_utils.py:218-219
         torch.cuda.synchronize()
         t1 = time.perf_counter()
-        if world > 1 and a.critic in ("fused", "pairs"):
+        if world > 1 and a.critic in ("fused", "pairs", "mlp_sharded"):     # global batch over the ranks (both critics)
             loss = mi_b200.sharded_mi_loss(emb_img, emb_txt, critic, study, a.estimator)
-        elif a.critic in ("fused", "mlp"):                            # (N > 1 with the MLP critic: per-rank batches, as the reference's DDP)
+        elif a.critic in ("fused", "mlp", "mlp_sharded"):             # (N > 1 with --critic mlp: per-rank batches, as the reference's DDP)
             mi_input = mi_b200.create_mi_pairs(emb_img, emb_txt, study.tolist(), dev)      # :220-221
             loss = mi_critic(critic(mi_input), B, dev)                                     # :222-224
         else:
@@ -164,9 +166,9 @@ def main():
         for step in range(a.throughput_steps):
             img_opt.zero_grad(); txt_opt.zero_grad(); mi_opt.zero_grad()
             emb_img, emb_txt = img_enc(img), txt_enc(ids, mask, seg)
-            if world > 1 and a.critic in ("fused", "pairs"):
+            if world > 1 and a.critic in ("fused", "pairs", "mlp_sharded"):
                 loss = mi_b200.sharded_mi_loss(emb_img, emb_txt, critic, study, a.estimator)
-            elif a.critic in ("fused", "mlp"):
+            elif a.critic in ("fused", "mlp", "mlp_sharded"):
                 loss = mi_critic(critic(mi_b200.create_mi_pairs(emb_img, emb_txt, study_list, dev)), B, dev)
             else:
                 loss = mi_critic(critic(mi_b200.create_mi_pairs_tensor(emb_img, emb_txt, study_list, dev)), B, dev)

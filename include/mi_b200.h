@@ -281,6 +281,53 @@ int mi_mlp_critic_loss_fwd_bwd(const float* X, const float* Y, const float* W1, 
                                double* loss_out, float* S_out, float* dX, float* dY, float* dW1, float* db1, float* dW2, float* db2,
                                float* dW3, float* db3, void* workspace, size_t workspace_bytes, mi_stream_t stream);
 
+/* The MLP critic over a ROW BLOCK: the stage ops of the batch-sharded step (DESIGN 8.4; mi_b200.dist drives them with
+ * its own collectives).  Rank r holds image rows X [Bq, D] at global rows [q_offset, q_offset + Bq) and has all-gathered
+ * the Bk text rows Y [Bk, D] of the batch (Bk = B_global) and their ids sid_k [Bk]; sid_q [Bq] = the ids of its own rows.
+ * The six parameters are replicated.  Every call is asynchronous on `stream` and never synchronises.  Per step:
+ *   1. mi_mlp_block_ref_logit  (single pass only) -> ref_out[1]: the maximum logit of a sample of the block's OWN pairs
+ *      (image rows x the text rows at the same global indices); the caller takes the maximum over the ranks.
+ *   2. mi_mlp_block_fwd        the block's pass over its Bq x Bk pairs -> scal_out[8], the block's scalar row in the
+ *      mi_score_stats layout (slot 7: the block's sum of the softmax weights in reference units, single pass only).
+ *      two_pass = 0: the single pass against `ref` (same value on every rank); 1: the logits are formed first (exact).
+ *   3. (caller) all-gather of the scalar rows -> scal_all [world, 8]
+ *   4. mi_mlp_block_merge      -> loss_out[8] of the batch (mi_mlp_critic_loss_fwd_bwd's layout) and merged[8] (the merged
+ *      row, slot 7 summed).  Single pass: loss_out[7] != 0 when the global weight sum left [1e-30, 1e30] while negatives
+ *      exist — the same verdict on every rank; the caller then repeats the step with two_pass = 1.
+ *   5. mi_mlp_block_bwd        -> dX of the block's rows, dC_part [Bk, H1] (the block's contribution to dL/dC for EVERY
+ *      text row, to be summed over ranks), the image half of dW1 ([H1, 2D] pitch, columns [0, D)), db1, dW2, db2, dW3,
+ *      db3: the block's shares (sum over ranks = the gradient of the global loss).
+ *   6. (caller) reduce-scatter of dC_part -> dC [Bq, H1] of the own text rows;
+ *      mi_mlp_input_grad(dC, Y_own, W1, side = 1) -> dY of the own rows and the text half of dW1; all-reduce of the
+ *      parameter gradients.
+ * `state` (mi_mlp_block_state_bytes) is caller-owned and carries the block from fwd to bwd; `workspace`
+ * (mi_mlp_block_workspace_bytes, covers every stage and mi_mlp_input_grad with R = Bq) is scratch that may be reused in
+ * between.  Sizes are 0 for unsupported shapes (D, H1, H2 multiples of 8, H2 <= 512). */
+size_t mi_mlp_block_workspace_bytes(int64_t Bq, int64_t Bk, int64_t D, int64_t H1, int64_t H2, int precision);
+size_t mi_mlp_block_state_bytes(int64_t Bq, int64_t Bk, int64_t D, int64_t H1, int64_t H2, int precision);
+int mi_mlp_block_ref_logit(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                           const float* W3, const float* b3, int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2,
+                           int precision, float* ref_out, void* workspace, size_t workspace_bytes, mi_stream_t stream);
+int mi_mlp_block_fwd(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                     const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                     int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                     const float* ref, int two_pass, double* scal_out, void* state, size_t state_bytes,
+                     void* workspace, size_t workspace_bytes, mi_stream_t stream);
+int mi_mlp_block_merge(const double* scal_all, int world, int64_t B_global, int estimator, int two_pass, double* loss_out,
+                       double* merged, mi_stream_t stream);
+int mi_mlp_block_bwd(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                     const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                     int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                     int two_pass, const double* loss, const double* merged, void* state, size_t state_bytes,
+                     float* dX, float* dC_part, float* dW1, float* db1, float* dW2, float* db2, float* dW3, float* db3,
+                     void* workspace, size_t workspace_bytes, mi_stream_t stream);
+/* Layer-1 backward of one side of the MLP critic over R rows: dZ [R, H1] = dL/d(W1side in), In [R, D], W1 the full [H1, 2D]
+ * weight; side 0 = image (W1x, columns [0, D)), 1 = text (W1y, columns [D, 2D)).  dIn = dZ W1side [R, D], the side's
+ * half of dW1 [H1, 2D] = dZ^T In, db1 (optional) = column sums of dZ.  Any output may be NULL. */
+size_t mi_mlp_input_grad_workspace_bytes(int64_t R, int64_t D, int64_t H1, int precision);
+int mi_mlp_input_grad(const float* dZ, const float* In, const float* W1, int side, int64_t R, int64_t D, int64_t H1, int precision,
+                      float* dIn, float* dW1, float* db1, void* workspace, size_t workspace_bytes, mi_stream_t stream);
+
 /* ---- Generalised Discrimination Value (validate.py:16-49, gdv_calculation; SURVEY 8f-3) ----------------- */
 
 /* pos [Np, D], neg [Nn, D]: fp32 device matrices of the two classes' embeddings (validate.py:118-127).  Each class is
@@ -318,6 +365,7 @@ void mi_set_mlp_panel_pairs(int64_t pairs); /* pairs per row panel of the MLP-cr
  * device-predicated two-pass repeat if the guard trips); bit 1: the dZ1 reductions are fused into their GEMM's epilogue.
  * Default 3; 0 = the two-pass sequence for every estimator; negative = default. */
 void mi_set_mlp_mode(int mode);
+int mi_get_mlp_mode(void);                  /* the current MLP-critic mode (0..3) */
 /* Multi-GPU overlap: the tile-engine launches that follow `event_after_outk` inside mi_score_single_pass / mi_score_grad
  * use (SM count - n) SMs, so the collective the caller starts at that event (reduce-scatter of the dY contributions)
  * finds free SMs instead of queueing behind a persistent 148-CTA grid.  0 (default) = use every SM. */

@@ -24,6 +24,7 @@ PROTOTYPES = {
     "mi_set_overlap_reserve_sms": (None, [c_int]),
     "mi_set_mlp_panel_pairs": (None, [c_i64]),
     "mi_set_mlp_mode": (None, [c_int]),
+    "mi_get_mlp_mode": (c_int, []),
     "mi_plan_ksplit": (c_int, [c_i64, c_int, c_i64]),
     "mi_plan_mlp_walk": (c_i64, [c_i64, c_i64, c_i64, c_vp, c_i64]),
     "mi_get_cta_group": (c_int, []),
@@ -70,6 +71,15 @@ PROTOTYPES = {
                                                c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_int, c_vp]),
     "mi_mlp_critic_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64, c_i64, c_int]),
     "mi_mlp_critic_loss_fwd_bwd": (c_int, [c_vp] * 9 + [c_i64, c_i64, c_i64, c_i64, c_int, c_int] + [c_vp] * 10 + [c_vp, c_sz, c_vp]),
+    "mi_mlp_block_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64, c_i64, c_i64, c_int]),
+    "mi_mlp_block_state_bytes": (c_sz, [c_i64, c_i64, c_i64, c_i64, c_i64, c_int]),
+    "mi_mlp_block_ref_logit": (c_int, [c_vp] * 8 + [c_i64] * 6 + [c_int, c_vp, c_vp, c_sz, c_vp]),
+    "mi_mlp_block_fwd": (c_int, [c_vp] * 10 + [c_i64] * 6 + [c_int, c_int, c_vp, c_int, c_vp, c_vp, c_sz, c_vp, c_sz, c_vp]),
+    "mi_mlp_block_merge": (c_int, [c_vp, c_int, c_i64, c_int, c_int, c_vp, c_vp, c_vp]),
+    "mi_mlp_block_bwd": (c_int, [c_vp] * 10 + [c_i64] * 6 + [c_int, c_int, c_int, c_vp, c_vp, c_vp, c_sz] + [c_vp] * 8
+                         + [c_vp, c_sz, c_vp]),
+    "mi_mlp_input_grad_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64, c_int]),
+    "mi_mlp_input_grad": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "mi_gdv_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64, c_int]),
     "mi_gdv": (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_sz, c_vp]),
     "mi_critic_host_scratch_bytes": (c_sz, [c_i64, c_i64, c_int, c_int, c_int, c_int]),

@@ -164,17 +164,51 @@ class _ShardedFusedCriticLoss(torch.autograd.Function):
         return gx, gy, gw, None, None, None, None, None, None
 
 
+class _ShardedFusedMLPCriticLoss(torch.autograd.Function):
+    """Data-parallel form of the concat-MLP critic: every rank passes its row shard; the loss is the GLOBAL-batch
+    estimator (identical on all ranks), embedding gradients are those of the local rows, the six parameter gradients are
+    already summed over ranks (the gradient of the global loss)."""
+
+    @staticmethod
+    def forward(ctx, X, Y, W1, b1, W2, b2, W3, b3, sid, estimator, precision, group, grad_scale):
+        from . import dist as mdist
+        tensors = (X, Y, W1, b1, W2, b2, W3, b3)
+        need = any(t.requires_grad for t in tensors)
+        out, dX, dY, grads = mdist.sharded_mlp_critic_loss_fwd_bwd(X, Y, (W1, b1, W2, b2, W3, b3), sid, estimator, precision,
+                                                                   need_grads=need, group=group)
+        ctx.grads = None if dX is None else (dX, dY) + tuple(grads[n] for n in mdist.MLP_GRAD_NAMES)
+        ctx.dtypes = tuple(t.dtype for t in tensors)
+        ctx.grad_scale = grad_scale
+        ctx.stats = out
+        return out["loss"].to(torch.float32)
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        if ctx.grads is None:
+            return (None,) * 13
+        g = grad_out.to(torch.float32)
+        ge = g * ctx.grad_scale          # encoder grads: DDP averages over ranks, the global loss needs the sum
+        scales = (ge, ge) + (g,) * 6
+        outs = tuple((t * s).to(dt) for t, s, dt in zip(ctx.grads, scales, ctx.dtypes))
+        return outs + (None,) * 5
+
+
 def sharded_mi_loss(embedding_img, embedding_txt, critic: "FusedCritic", study_id, estimator: str = "dv",
                     group=None, ddp_mean_correction: bool = True) -> torch.Tensor:
     """Global-batch MI loss when every rank holds a row shard of the batch (SURVEY 8e / 8f-4).
     ``study_id`` is this rank's integer id tensor (raw int64 ids are relabelled consistently across ranks).
     With ``ddp_mean_correction`` the embedding gradients are multiplied by the world size so that
-    DistributedDataParallel's gradient averaging of the encoders yields the gradient of the global loss."""
+    DistributedDataParallel's gradient averaging of the encoders yields the gradient of the global loss; parameter
+    gradients are those of the global loss, not scaled.  ``critic`` is a ``FusedCritic`` or a ``FusedMLPCritic``."""
     import torch.distributed as tdist
     world = tdist.get_world_size(group) if tdist.is_available() and tdist.is_initialized() else 1
     sid = study_id if torch.is_tensor(study_id) else torch.tensor([int(s) for s in study_id], dtype=torch.int64)
     sid = sid.to(embedding_img.device)
     scale = float(world) if ddp_mean_correction else 1.0
+    if isinstance(critic, FusedMLPCritic):
+        c = critic
+        return _ShardedFusedMLPCriticLoss.apply(embedding_img, embedding_txt, c[0].weight, c[0].bias, c[2].weight, c[2].bias,
+                                                c[4].weight, c[4].bias, sid, estimator, c.precision, group, scale)
     return _ShardedFusedCriticLoss.apply(embedding_img, embedding_txt, critic.W, sid, estimator, critic.precision,
                                          critic.inv_tau, group, scale)
 

@@ -1064,7 +1064,8 @@ struct EpiMlpDz {
 //      pass (g~ = incl e^{S - ref}; every gradient is linear in g~, the caller multiplies by e^{ref - LSE} at the end),
 //      so nothing has to wait for the global log-sum-exp and Z2 is never recomputed.
 //      Rows are pairs in the padded panel order p = il * Bp + j (Bp = B rounded up to the M block): an M block has ONE
-//      image row i = r0 + il and consecutive text columns j.  Joint policy: pass1 forms this warp's share of the logit
+//      image row i = r0 + il and consecutive text columns j.  The image rows may be a block of a larger batch (sharded
+//      step): local row i is global row q_off + i, so its positive pair is text column j = q_off + i.  Joint policy: pass1 forms this warp's share of the logit
 //      (64 of the up to 512 columns per tile), `mid` adds the four column quarters through shared memory (one named
 //      barrier of the 16 epilogue warps per unit, double-buffered slots), derives g~ and the row statistics, and the
 //      second pass is EpiMlpDz's chunk with that g~.
@@ -1081,18 +1082,20 @@ struct EpiMlpSp {
     const float* w3;       // [n_ntile * 256] zero padded
     const float* b3;       // [1]
     const float* ref;      // [1] maximum logit of the sample (the reference logit is this + kMlpSpMargin)
-    const int* sid;        // [B] study ids (negatives: sid[i] != sid[j], main_utils.py:105)
-    int B, Bp, r0, rr;     // batch, padded batch, first image row of the panel, image rows in the panel
+    const int* sid_q;      // [rows] study ids of the image rows (negatives: sid_q[i] != sid_k[j], main_utils.py:105)
+    const int* sid_k;      // [B] study ids of the text rows
+    int B, Bp, r0, rr;     // text rows, padded text rows, first image row of the panel, image rows in the panel
+    int q_off;             // global index of local image row 0
     int cols;              // H2
     __nv_bfloat16* dz;     // [rr * Bp, pitch]  g~ w3 [Z2 + b2 > 0]
     __nv_bfloat16* dz_lo;  // residual half (strict) or nullptr
     long long pitch;
     float* dw3;            // [n_ntile * 256] accumulators (atomicAdd), in g~ units
     float* db2;
-    float* rowsum;         // [B] += sum_j g~          (atomicAdd)
-    float* rowcnt;         // [B] += number of negatives of the row
-    float* diag_out;       // [B] logit of the positive pair
-    float* S_out;          // optional [B, B]: every logit
+    float* rowsum;         // [rows] += sum_j g~          (atomicAdd)
+    float* rowcnt;         // [rows] += number of negatives of the row
+    float* diag_out;       // [rows] logit of the positive pair
+    float* S_out;          // optional [rows, B]: every logit
   };
   struct State { uint8_t* stage_smem; float acc; float g; int slot; float sw[kMaxTiles][2]; float sb[kMaxTiles][2]; };
   static __device__ __forceinline__ void init(const Params&, State& st) {
@@ -1126,7 +1129,7 @@ struct EpiMlpSp {
     st.slot ^= 1;       // the next unit writes the other slot; this one is rewritten two barriers from now
     const int il = row / p.Bp, j = row - il * p.Bp, i = p.r0 + il;
     const bool valid = j < p.B && il < p.rr;
-    const bool incl = valid && __ldg(p.sid + i) != __ldg(p.sid + j);
+    const bool incl = valid && __ldg(p.sid_q + i) != __ldg(p.sid_k + j);
     // e^{S - ref} with ref = (sample maximum) + 69 ln 2: the subtraction stays near the logits (no absolute rounding at
     // the size of the margin) and the margin is an exact power of two
     const float g = incl ? expf(S - __ldg(p.ref)) * kMlpSpScale : 0.f;
@@ -1134,7 +1137,7 @@ struct EpiMlpSp {
     if (colq == 0) {
       if (valid) {
         if (p.S_out != nullptr) p.S_out[(size_t)i * p.B + j] = S;
-        if (i == j) p.diag_out[i] = S;
+        if (j == p.q_off + i) p.diag_out[i] = S;
       }
       float gs = g;
 #pragma unroll
@@ -1238,10 +1241,10 @@ struct EpiMlpDa {
   struct Params {
     const uint32_t* mask;  // [rr * Bp][wpr]
     int wpr;               // mask words per pair = ceil(H1 / 32) rounded up to an even number (8 B loads)
-    int B, Bp, r0, rr;
+    int B, Bp, r0, rr;     // text rows, padded text rows, first image row of the panel, image rows in the panel
     int cols;              // H1
-    float* dA;             // [B, cols]   (atomicAdd)
-    float* dC;             // [B, cols]   (atomicAdd)
+    float* dA;             // [image rows, cols]   (atomicAdd)
+    float* dC;             // [B, cols]            (atomicAdd)
   };
   struct State { uint8_t* stage_smem; float dc[64]; uint32_t mw0, mw1; int il; };
   static __device__ __forceinline__ void init(const Params&, State&) {}

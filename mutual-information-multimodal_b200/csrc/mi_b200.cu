@@ -789,18 +789,19 @@ __global__ void flag_to_scal_kernel(const int* __restrict__ flag, double* __rest
   scal[6] = static_cast<double>(flag[0]);
 }
 
-// ranks' reduced scalars [world][8] -> one row of the same layout (global max / rescaled sum-exp, plain sums)
+// ranks' reduced scalars [world][8] -> one row of the same layout (global max / rescaled sum-exp, plain sums).
+// Slot 7 is summed too: the MLP critic's sharded single pass carries each block's sum of g~ there (0 everywhere else).
 __global__ void merge_scal_kernel(const double* __restrict__ scal_all, int world, double* __restrict__ out) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   double gm = -INFINITY;
   for (int r = 0; r < world; ++r) gm = fmax(gm, scal_all[r * 8]);
-  double s = 0, t[5] = {0, 0, 0, 0, 0};
+  double s = 0, t[6] = {0, 0, 0, 0, 0, 0};
   for (int r = 0; r < world; ++r) {
     const double* v = scal_all + r * 8;
     if (isfinite(v[0])) s += v[1] * exp(v[0] - gm);
-    for (int k = 0; k < 5; ++k) t[k] += v[2 + k];
+    for (int k = 0; k < 6; ++k) t[k] += v[2 + k];
   }
-  out[0] = gm; out[1] = s; out[2] = t[0]; out[3] = t[1]; out[4] = t[2]; out[5] = t[3]; out[6] = t[4]; out[7] = 0;
+  out[0] = gm; out[1] = s; out[2] = t[0]; out[3] = t[1]; out[4] = t[2]; out[5] = t[3]; out[6] = t[4]; out[7] = t[5];
 }
 
 // fused glue: loss from the reduced scalars (fp64), and the scalar references as floats
@@ -826,7 +827,7 @@ __global__ void loss_finalize_kernel(const double* __restrict__ scal_row, const 
       !(fabs((double)lambda[0] - lse) <= 60.0)) guard += 1.0;
   loss_out[0] = loss; loss_out[1] = pos; loss_out[2] = lse; loss_out[3] = n_neg;
   loss_out[4] = loss_row; loss_out[5] = loss_col; loss_out[6] = scal_row[5]; loss_out[7] = guard;
-  *lse_f = (float)lse;
+  if (lse_f) *lse_f = (float)lse;
 }
 // flag[0] = (loss_out[7] != 0): the device predicate of the exact fallback
 __global__ void guard_to_flag_kernel(const double* __restrict__ loss_out, int* __restrict__ flag, double* __restrict__ guard_a) {
@@ -1893,6 +1894,7 @@ void mi_set_mlp_panel_pairs(int64_t pairs) {      // bounded: pair indices insid
   g_mlp_max_pairs = pairs > 0 ? (pairs < (1LL << 27) ? pairs : (1LL << 27)) : (1LL << 20);
 }
 void mi_set_mlp_mode(int mode) { g_mlp_mode.store(mode < 0 ? 3 : (mode & 3), std::memory_order_relaxed); }
+int mi_get_mlp_mode(void) { return g_mlp_mode.load(std::memory_order_relaxed); }
 void mi_set_cta_group(int g) { g_cta_group.store((g == 1) ? 1 : 2, std::memory_order_relaxed); }
 int mi_get_cta_group(void) { return cta_group(); }
 
@@ -2355,6 +2357,98 @@ int mi_mlp_critic_loss_fwd_bwd(const float* X, const float* Y, const float* W1, 
   Bump ws(workspace, workspace_bytes, false);
   return mlp_impl(X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, sid, MlpDims{B, D, H1, H2}, estimator, precision, loss_out, S_out,
                   MlpGrads{dX, dY, dW1, db1, dW2, db2, dW3, db3}, ws, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// ---- the MLP critic over a row block: the stage ops of the batch-sharded step (DESIGN 8.4)
+// (the size queries plan every stage of both sequences: the path is chosen per step)
+size_t mi_mlp_block_workspace_bytes(int64_t Bq, int64_t Bk, int64_t D, int64_t H1, int64_t H2, int precision) {
+  const MlpBlock blk{Bq, Bk, 0, Bk, nullptr, nullptr};
+  const MlpDims d{Bk, D, H1, H2};
+  size_t peak = 0;
+  const int stages[5][2] = {{kMlpStageRef, 0}, {kMlpStageFwd, 0}, {kMlpStageFwd, 1}, {kMlpStageBwd, 0}, {kMlpStageBwd, 1}};
+  for (const auto& st : stages) {
+    Bump ws(nullptr, 0, true), keep(nullptr, 0, true);
+    MlpBlockIO io{};
+    io.two_pass = st[1];
+    // the reference stage keeps nothing: its state comes from the workspace
+    if (mlp_block_impl(st[0], nullptr, nullptr, MlpParams{}, blk, d, MI_EST_DV, precision, io, ws, st[0] == kMlpStageRef ? ws : keep,
+                       nullptr) != MI_OK)
+      return 0;
+    if (ws.peak > peak) peak = ws.peak;
+  }
+  Bump ws(nullptr, 0, true);
+  if (mlp_input_grad_impl(nullptr, nullptr, nullptr, 1, Bq, D, H1, precision, nullptr, nullptr, nullptr, ws, nullptr) != MI_OK) return 0;
+  if (ws.peak > peak) peak = ws.peak;
+  return peak + 256;
+}
+size_t mi_mlp_block_state_bytes(int64_t Bq, int64_t Bk, int64_t D, int64_t H1, int64_t H2, int precision) {
+  Bump ws(nullptr, 0, true), keep(nullptr, 0, true);
+  if (mlp_block_impl(kMlpStageFwd, nullptr, nullptr, MlpParams{}, MlpBlock{Bq, Bk, 0, Bk, nullptr, nullptr}, MlpDims{Bk, D, H1, H2},
+                     MI_EST_DV, precision, MlpBlockIO{}, ws, keep, nullptr) != MI_OK) return 0;
+  return keep.peak + 256;
+}
+int mi_mlp_block_ref_logit(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                           const float* W3, const float* b3, int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2,
+                           int precision, float* ref_out, void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+  MI_TRY(device_check());
+  Bump ws(workspace, workspace_bytes, false);
+  MlpBlockIO io{};
+  io.ref_out = ref_out;
+  return mlp_block_impl(kMlpStageRef, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, nullptr, nullptr},
+                        MlpDims{Bk, D, H1, H2}, MI_EST_DV, precision, io, ws, ws, reinterpret_cast<cudaStream_t>(stream));
+}
+int mi_mlp_block_fwd(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                     const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                     int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                     const float* ref, int two_pass, double* scal_out, void* state, size_t state_bytes,
+                     void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+  MI_TRY(device_check());
+  Bump ws(workspace, workspace_bytes, false), keep(state, state_bytes, false);
+  MlpBlockIO io{};
+  io.ref = ref; io.two_pass = two_pass; io.scal_out = scal_out;
+  return mlp_block_impl(kMlpStageFwd, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, sid_q, sid_k},
+                        MlpDims{Bk, D, H1, H2}, estimator, precision, io, ws, keep, reinterpret_cast<cudaStream_t>(stream));
+}
+int mi_mlp_block_merge(const double* scal_all, int world, int64_t B_global, int estimator, int two_pass, double* loss_out, double* merged,
+                       mi_stream_t stream_) {
+  MI_TRY(device_check());
+  if (!scal_all || world <= 0 || B_global <= 0 || !loss_out || !merged ||
+      (estimator != MI_EST_DV && estimator != MI_EST_INFONCE_REF && estimator != MI_EST_INFONCE_ROW)) return MI_ERR_BAD_ARG;
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  merge_scal_kernel<<<1, 32, 0, stream>>>(scal_all, world, merged);
+  MI_LAUNCH_CHECK("merge_scal_kernel");
+  loss_finalize_kernel<<<1, 32, 0, stream>>>(merged, nullptr, B_global, estimator, loss_out, nullptr, nullptr, nullptr);
+  MI_LAUNCH_CHECK("loss_finalize_kernel");
+  if (!two_pass) {
+    mlp_block_guard_kernel<<<1, 1, 0, stream>>>(merged, loss_out);
+    MI_LAUNCH_CHECK("mlp_block_guard_kernel");
+  }
+  return MI_OK;
+}
+int mi_mlp_block_bwd(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                     const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                     int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                     int two_pass, const double* loss, const double* merged, void* state, size_t state_bytes,
+                     float* dX, float* dC_part, float* dW1, float* db1, float* dW2, float* db2, float* dW3, float* db3,
+                     void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+  MI_TRY(device_check());
+  Bump ws(workspace, workspace_bytes, false), keep(state, state_bytes, false);
+  MlpBlockIO io{};
+  io.two_pass = two_pass; io.loss = loss; io.merged = merged; io.dC_part = dC_part;
+  io.gr = MlpGrads{dX, nullptr, dW1, db1, dW2, db2, dW3, db3};
+  return mlp_block_impl(kMlpStageBwd, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, sid_q, sid_k},
+                        MlpDims{Bk, D, H1, H2}, estimator, precision, io, ws, keep, reinterpret_cast<cudaStream_t>(stream));
+}
+size_t mi_mlp_input_grad_workspace_bytes(int64_t R, int64_t D, int64_t H1, int precision) {
+  Bump ws(nullptr, 0, true);
+  if (mlp_input_grad_impl(nullptr, nullptr, nullptr, 0, R, D, H1, precision, nullptr, nullptr, nullptr, ws, nullptr) != MI_OK) return 0;
+  return ws.peak + 256;
+}
+int mi_mlp_input_grad(const float* dZ, const float* In, const float* W1, int side, int64_t R, int64_t D, int64_t H1, int precision,
+                      float* dIn, float* dW1, float* db1, void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+  MI_TRY(device_check());
+  Bump ws(workspace, workspace_bytes, false);
+  return mlp_input_grad_impl(dZ, In, W1, side, R, D, H1, precision, dIn, dW1, db1, ws, reinterpret_cast<cudaStream_t>(stream));
 }
 
 // ---- introspection of the host-side scheduling decisions (CPU tests; no device needed)

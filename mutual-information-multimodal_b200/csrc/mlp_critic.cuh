@@ -55,15 +55,15 @@ __global__ void fill_f32_kernel(float* __restrict__ p, long long n, float v) {
   if (i < n) p[i] = v;
 }
 // H[p, k] = relu(A[i, k] + C[j, k]) as bf16 hi (+ lo at column Hp), 8 columns per thread;
-// pairs p = (i - r0) Bk + j of a row panel, or the positive pairs i = j = p (diag)
+// pairs p = (i - r0) Bk + j of a row panel, or the positive pairs i = p, j = q_off + p (diag)
 __global__ void mlp_gen_kernel(const float* __restrict__ A, const float* __restrict__ Cm, long long H1, long long Bk, long long r0,
                                long long P, __nv_bfloat16* __restrict__ H, long long pitch, long long Hp, int split, int diag,
-                               const int* __restrict__ run_if) {
+                               long long q_off, const int* __restrict__ run_if) {
   MI_PRED(run_if);
   const long long h8 = H1 >> 3;
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < P * h8; idx += (long long)gridDim.x * blockDim.x) {
     const long long p = idx / h8, k = (idx - p * h8) << 3;
-    const long long i = diag ? p : r0 + p / Bk, j = diag ? p : p % Bk;
+    const long long i = diag ? p : r0 + p / Bk, j = diag ? q_off + p : p % Bk;
     const float4* a4 = reinterpret_cast<const float4*>(A + i * H1 + k);
     const float4* c4 = reinterpret_cast<const float4*>(Cm + j * H1 + k);
     const float4 a0 = __ldg(a4), a1 = __ldg(a4 + 1), c0 = __ldg(c4), c1 = __ldg(c4 + 1);
@@ -168,18 +168,20 @@ __global__ void mlp_logit_merge_kernel(const float* __restrict__ part, int rows_
   for (int q = 0; q < mi::kColQuarters; ++q) a += part[(size_t)q * rows_padded + p];
   S[p] = a;
 }
-// one warp per row of S: {lse over the negatives, #negatives, S_ii, lse over negatives and the positive}
-__global__ void mlp_row_stats_kernel(const float* __restrict__ S, const int* __restrict__ sid, long long B, float4* __restrict__ row_out,
+// one warp per row of S [Bq, Bk] (image rows at q_off): {lse over the negatives, #negatives, S[i, q_off + i],
+// lse over negatives and the positive}
+__global__ void mlp_row_stats_kernel(const float* __restrict__ S, const int* __restrict__ sid_q, const int* __restrict__ sid_k,
+                                     long long Bq, long long Bk, long long q_off, float4* __restrict__ row_out,
                                      const int* __restrict__ run_if) {
   MI_PRED(run_if);
   const long long row = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  if (row >= B) return;
-  const int my = sid[row];
+  if (row >= Bq) return;
+  const int my = sid_q[row];
   float m = mi::neg_inf(), s = 0.f, cnt = 0.f;
-  for (long long j = lane; j < B; j += 32) {
-    if (sid[j] != my) {                                   // main_utils.py:105 (the diagonal has equal ids)
-      const float v = S[row * B + j];
+  for (long long j = lane; j < Bk; j += 32) {
+    if (sid_k[j] != my) {                                 // main_utils.py:105 (the diagonal has equal ids)
+      const float v = S[row * Bk + j];
       const float mn = fmaxf(m, v);
       s = s * expf(m - mn) + expf(v - mn); m = mn; cnt += 1.f;
     }
@@ -192,7 +194,7 @@ __global__ void mlp_row_stats_kernel(const float* __restrict__ S, const int* __r
     m = mn;
   }
   if (lane == 0) {
-    const float diag = S[row * B + row];
+    const float diag = S[row * Bk + q_off + row];
     const float lse_neg = (cnt > 0.f && s > 0.f) ? m + logf(s) : mi::neg_inf();
     const float hi = fmaxf(lse_neg, diag), lo = fminf(lse_neg, diag);
     row_out[row] = make_float4(lse_neg, cnt, diag, hi + log1pf(expf(lo - hi)));
@@ -212,20 +214,22 @@ __global__ void mlp_rows_from_sums_kernel(const float* __restrict__ rowsum, cons
   const float hi = fmaxf(lse_neg, d), lo = fminf(lse_neg, d);
   row_out[i] = make_float4(lse_neg, cnt, d, hi + log1pf(expf(lo - hi)));
 }
-// G = dL/dS.  dv / infonce (mi_critics.py:3-23): softmax over ALL negatives, -1/B on the diagonal;
-// row InfoNCE: (1/B) softmax over {positive} u negatives of the row, minus 1/B on the diagonal.
-__global__ void mlp_g_kernel(const float* __restrict__ S, const int* __restrict__ sid, long long B, int dv_like,
-                             const float* __restrict__ lse, const float4* __restrict__ rows, float* __restrict__ G,
-                             const int* __restrict__ run_if) {
+// G = dL/dS over a block [Bq, Bk] (image rows at q_off) of a batch of Bg.  dv / infonce (mi_critics.py:3-23): softmax
+// over ALL negatives (lse = the global log-sum-exp), -1/Bg on the diagonal; row InfoNCE: (1/Bg) softmax over {positive} u
+// negatives of the row, minus 1/Bg on the diagonal.
+__global__ void mlp_g_kernel(const float* __restrict__ S, const int* __restrict__ sid_q, const int* __restrict__ sid_k, long long Bq,
+                             long long Bk, long long q_off, long long Bg, int dv_like, const float* __restrict__ lse,
+                             const float4* __restrict__ rows, float* __restrict__ G, const int* __restrict__ run_if) {
   MI_PRED(run_if);
   const long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  if (idx >= B * B) return;
-  const long long i = idx / B, j = idx - i * B;
-  const float inv_b = 1.f / static_cast<float>(B);
-  const bool neg = sid[i] != sid[j];
+  if (idx >= Bq * Bk) return;
+  const long long i = idx / Bk, j = idx - i * Bk;
+  const float inv_b = 1.f / static_cast<float>(Bg);
+  const bool neg = sid_q[i] != sid_k[j];
+  const bool pos = j == q_off + i;
   float g = 0.f;
-  if (dv_like) g = neg ? expf(S[idx] - lse[0]) : (i == j ? -inv_b : 0.f);
-  else if (neg || i == j) g = inv_b * expf(S[idx] - rows[i].w) - (i == j ? inv_b : 0.f);
+  if (dv_like) g = neg ? expf(S[idx] - lse[0]) : (pos ? -inv_b : 0.f);
+  else if (neg || pos) g = inv_b * expf(S[idx] - rows[i].w) - (pos ? inv_b : 0.f);
   G[idx] = g;
 }
 // One read of the dZ1 panel gives both reductions.  A block owns a slab [32 rows il] x [all j] x [64 columns]:
@@ -307,12 +311,15 @@ __global__ void sum_reduce_kernel(const float* __restrict__ in, long long n, flo
   __syncthreads();
   if (threadIdx.x == 0) { double t = 0.0; for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += sh[i]; out[0] = static_cast<float>(t); }
 }
-// one block, after loss_finalize_kernel: total = sum of g~ over all negatives (fp64).  The softmax weights are g~ / total,
-// so cfac = 1 / total takes the sums from reference units to weights without going through e^{ref - LSE}.
-// Guard (loss_out[7] = 1, cfac = 0): total outside [1e-30, 1e30] (overflow of some e^{S - ref}, or every negative
-// flushed to zero) while negatives exist.  db3 = sum of dL/dlogit over all pairs = total cfac - 1 (analytically 0).
-__global__ void mlp_weights_kernel(const float* __restrict__ rowsum, long long n, float* __restrict__ cfac, float* __restrict__ db3,
-                                   double* __restrict__ loss_out) {
+// one block, after loss_finalize_kernel: t = sum of g~ over the rows' negatives (fp64); total = t, or the sum over every
+// row block of the batch (`total_in`, sharded step).  The softmax weights are g~ / total, so cfac = 1 / total takes the
+// sums from reference units to weights without going through e^{ref - LSE}.
+// Guard (guard_out = 1, cfac = 0): total outside [1e-30, 1e30] (overflow of some e^{S - ref}, or every negative
+// flushed to zero) while negatives exist (n_neg[0] > 0).  db3 = the block's share of sum of dL/dlogit over all pairs:
+// t cfac - frac, frac = Bq / Bg (the positive pairs of the block); summed over the blocks: 1 - 1 (analytically 0).
+__global__ void mlp_weights_kernel(const float* __restrict__ rowsum, long long n, const double* __restrict__ total_in, double frac,
+                                   const double* __restrict__ n_neg, float* __restrict__ cfac, float* __restrict__ db3,
+                                   double* __restrict__ guard_out) {
   __shared__ double sh[32];
   double a = 0.0;
   for (long long i = threadIdx.x; i < n; i += blockDim.x) a += rowsum[i];
@@ -322,14 +329,33 @@ __global__ void mlp_weights_kernel(const float* __restrict__ rowsum, long long n
   if (threadIdx.x == 0) {
     double t = 0.0;
     for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += sh[i];
-    const bool any_neg = loss_out[3] > 0.0;
-    const bool ok = t >= 1e-30 && t <= 1e30;
-    const float c = (any_neg && ok) ? static_cast<float>(1.0 / t) : 0.f;
+    const double total = total_in ? total_in[0] : t;
+    const bool any_neg = n_neg[0] > 0.0;
+    const bool ok = total >= 1e-30 && total <= 1e30;
+    const float c = (any_neg && ok) ? static_cast<float>(1.0 / total) : 0.f;
     cfac[0] = c;
-    db3[0] = any_neg ? static_cast<float>(t * static_cast<double>(c) - 1.0) : -1.f;
-    if (any_neg && !ok) loss_out[7] = 1.0;
+    db3[0] = any_neg ? static_cast<float>(t * static_cast<double>(c) - frac) : static_cast<float>(-frac);
+    if (any_neg && !ok && guard_out) guard_out[0] = 1.0;
   }
 }
+// one block: out[0] = sum in[0..n) in fp64 (the block's sum of g~ travels in slot 7 of its scalar row)
+__global__ void sum_f64_kernel(const float* __restrict__ in, long long n, double* __restrict__ out) {
+  __shared__ double sh[32];
+  double a = 0.0;
+  for (long long i = threadIdx.x; i < n; i += blockDim.x) a += in[i];
+  for (int o = 16; o; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = a;
+  __syncthreads();
+  if (threadIdx.x == 0) { double t = 0.0; for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += sh[i]; out[0] = t; }
+}
+// sharded step, after the merge of the blocks' scalar rows: the single pass' guard on the global sum of g~ (merged[7]),
+// the same window as mlp_weights_kernel
+__global__ void mlp_block_guard_kernel(const double* __restrict__ merged, double* __restrict__ loss_out) {
+  const double t = merged[7];
+  if (loss_out[3] > 0.0 && !(t >= 1e-30 && t <= 1e30)) loss_out[7] += 1.0;
+}
+// the global log-sum-exp as the float the estimator's G uses (loss_finalize_kernel's lse_f)
+__global__ void lse_from_loss_kernel(const double* __restrict__ loss_out, float* __restrict__ lse_f) { lse_f[0] = (float)loss_out[2]; }
 __global__ void copy_f32_kernel(const float* __restrict__ in, float* __restrict__ out, long long n) {
   long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i < n) out[i] = in[i];
@@ -348,6 +374,8 @@ __global__ void mlp_add_diag_kernel(const float* __restrict__ z, long long n, fl
 }
 
 struct MlpDims { long long B, D, H1, H2; };
+// Bq image rows (global rows q_off ..) against Bk text rows of a batch of Bg (single GPU: Bq = Bk = Bg, q_off = 0)
+struct MlpBlock { long long Bq, Bk, q_off, Bg; const int *sid_q, *sid_k; };
 struct MlpParams { const float *W1, *b1, *W2, *b2, *W3, *b3; };
 struct MlpGrads { float *dX, *dY, *dW1, *db1, *dW2, *db2, *dW3, *db3; };
 
@@ -379,9 +407,9 @@ int zero_async(void* p, size_t bytes, cudaStream_t stream) {
 
 // everything the two sequences share: dimensions, operands, scratch
 struct MlpCtx {
-  long long B, D, H1, H2, Dp, Hp, H2p, pX, pH, pZ, eX, eH, eZ, h2_pad;
+  long long Bq, Bk, q_off, Bg, D, H1, H2, Dp, Hp, H2p, pX, pH, pZ, eX, eH, eZ, h2_pad;
   int sp, nt2, estimator;
-  const int* sid;
+  const int *sid_q, *sid_k;
   MlpParams prm;
   __nv_bfloat16 *X16, *Y16, *W1x, *W1y, *W2h, *Hpan, *DZ2, *DZ1h, *dA16, *dC16;
   float *A32, *C32, *b2p, *w3p, *S, *rows_r, *lse_f, *part, *G, *DZ1, *dA32, *dC32, *acc_w3, *acc_b2, *dW2, *db3v;
@@ -445,7 +473,7 @@ int mlp_reduce_panel(const MlpCtx& c, long long cols, long long rr, long long r0
 }
 int mlp_zero_accumulators(const MlpCtx& c, long long dc_rows) {
   MI_TRY(zero_async(c.dC32, static_cast<size_t>(dc_rows) * c.H1 * sizeof(float), c.stream));
-  MI_TRY(zero_async(c.dA32, static_cast<size_t>(c.B) * c.H1 * sizeof(float), c.stream));
+  MI_TRY(zero_async(c.dA32, static_cast<size_t>(c.Bq) * c.H1 * sizeof(float), c.stream));
   MI_TRY(zero_async(c.acc_w3, static_cast<size_t>(c.h2_pad) * sizeof(float), c.stream));
   MI_TRY(zero_async(c.acc_b2, static_cast<size_t>(c.h2_pad) * sizeof(float), c.stream));
   return MI_OK;
@@ -453,76 +481,92 @@ int mlp_zero_accumulators(const MlpCtx& c, long long dc_rows) {
 
 // ---- the two-pass sequence: logits of every pair -> estimator -> recompute Z2 for the backward.  Exact for every input
 //      (running-max statistics); every estimator.  All launches carry this thread's launch predicate.
-int mlp_two_pass(const MlpCtx& c, bool plan, Bump& ws) {
-  const long long B = c.B, H1 = c.H1, H2 = c.H2;
+int mlp_tp_gen_panel(const MlpCtx& c, long long r0, long long P) {
+  mlp_gen_kernel<<<blocks_capped(P * (c.H1 >> 3), 256), 256, 0, c.stream>>>(c.A32, c.C32, c.H1, c.Bk, r0, P, c.Hpan, c.pH, c.Hp, c.sp, 0, 0,
+                                                                           t_run_if);
+  MI_LAUNCH_CHECK("mlp_gen_kernel");
+  return MI_OK;
+}
+// forward: the logits S [Bq, Bk] of the block, its row statistics (c.rows_r) and its scalar row (c.scal)
+int mlp_tp_fwd(const MlpCtx& c, bool dry) {
+  if (dry) return MI_OK;
+  const long long Bq = c.Bq, Bk = c.Bk, H2 = c.H2;
+  cudaStream_t stream = c.stream;
+  const long long R = mlp_panel_rows(Bq, Bk);
+  for (long long r0 = 0; r0 < Bq; r0 += R) {
+    const long long rr = (Bq - r0 < R) ? (Bq - r0) : R, P = rr * Bk;
+    MI_TRY(mlp_tp_gen_panel(c, r0, P));
+    Sched sc; mlp_z2_sched(c, P, sc);
+    mi::EpiMlpFwd::Params ep;
+    ep.b2 = c.b2p; ep.w3 = c.w3p; ep.part = c.part; ep.rows_padded = sc.n_mblk * rows_per_mblk();
+    MI_TRY(launch_engine<mi::EpiMlpFwd>(MapSpec{c.Hpan, P, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
+    mlp_logit_merge_kernel<<<blocks_for(P, 256), 256, 0, stream>>>(c.part, ep.rows_padded, P, c.prm.b3, c.S + r0 * Bk, t_run_if);
+    MI_LAUNCH_CHECK("mlp_logit_merge_kernel");
+  }
+  // ---- estimator on S (same reductions and fp64 finalisation as the separable critics)
+  mlp_row_stats_kernel<<<blocks_for(Bq * 32, 256), 256, 0, stream>>>(c.S, c.sid_q, c.sid_k, Bq, Bk, c.q_off,
+                                                                     reinterpret_cast<float4*>(c.rows_r), t_run_if);
+  MI_LAUNCH_CHECK("mlp_row_stats_kernel");
+  stats_reduce_kernel<<<1, 1024, 0, stream>>>(reinterpret_cast<const float4*>(c.rows_r), static_cast<int>(Bq), c.scal, t_run_if);
+  MI_LAUNCH_CHECK("stats_reduce_kernel");
+  return MI_OK;
+}
+// backward, once the loss is known (c.lse_f: the global log-sum-exp; c.rows_r: the block's row statistics): G, then Z2
+// recomputed panel by panel.  `resident`: the forward's only panel is still in c.Hpan.
+int mlp_tp_bwd(const MlpCtx& c, bool resident, Bump& ws) {
+  const long long Bq = c.Bq, Bk = c.Bk, H2 = c.H2;
   const bool dry = ws.dry;
   cudaStream_t stream = c.stream;
-  const long long R = mlp_panel_rows(B, B);
-  const long long n_panels = cdiv(B, R);
-  auto gen_panel = [&](long long r0, long long P) -> int {
-    mlp_gen_kernel<<<blocks_capped(P * (H1 >> 3), 256), 256, 0, stream>>>(c.A32, c.C32, H1, B, r0, P, c.Hpan, c.pH, c.Hp, c.sp, 0, t_run_if);
-    MI_LAUNCH_CHECK("mlp_gen_kernel");
-    return MI_OK;
-  };
-  if (!dry) {
-    // ---- forward: logits of every pair
-    for (long long r0 = 0; r0 < B; r0 += R) {
-      const long long rr = (B - r0 < R) ? (B - r0) : R, P = rr * B;
-      MI_TRY(gen_panel(r0, P));
-      Sched sc; mlp_z2_sched(c, P, sc);
-      mi::EpiMlpFwd::Params ep;
-      ep.b2 = c.b2p; ep.w3 = c.w3p; ep.part = c.part; ep.rows_padded = sc.n_mblk * rows_per_mblk();
-      MI_TRY(launch_engine<mi::EpiMlpFwd>(MapSpec{c.Hpan, P, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
-      mlp_logit_merge_kernel<<<blocks_for(P, 256), 256, 0, stream>>>(c.part, ep.rows_padded, P, c.prm.b3, c.S + r0 * B, t_run_if);
-      MI_LAUNCH_CHECK("mlp_logit_merge_kernel");
-    }
-    // ---- estimator on S (same reductions and fp64 finalisation as the separable critics)
-    mlp_row_stats_kernel<<<blocks_for(B * 32, 256), 256, 0, stream>>>(c.S, c.sid, B, reinterpret_cast<float4*>(c.rows_r), t_run_if);
-    MI_LAUNCH_CHECK("mlp_row_stats_kernel");
-    stats_reduce_kernel<<<1, 1024, 0, stream>>>(reinterpret_cast<const float4*>(c.rows_r), static_cast<int>(B), c.scal, t_run_if);
-    MI_LAUNCH_CHECK("stats_reduce_kernel");
-    loss_finalize_kernel<<<1, 32, 0, stream>>>(c.scal, nullptr, B, c.estimator, c.loss_out, c.lse_f, nullptr, t_run_if);
-    MI_LAUNCH_CHECK("loss_finalize_kernel");
-  }
-  if (!plan) return MI_OK;
+  const long long R = mlp_panel_rows(Bq, Bk);
   if (!dry) {
     const int dv_like = (c.estimator == MI_EST_DV || c.estimator == MI_EST_INFONCE_REF) ? 1 : 0;
-    mlp_g_kernel<<<blocks_for(B * B, 256), 256, 0, stream>>>(c.S, c.sid, B, dv_like, c.lse_f, reinterpret_cast<const float4*>(c.rows_r), c.G, t_run_if);
+    mlp_g_kernel<<<blocks_for(Bq * Bk, 256), 256, 0, stream>>>(c.S, c.sid_q, c.sid_k, Bq, Bk, c.q_off, c.Bg, dv_like, c.lse_f,
+                                                               reinterpret_cast<const float4*>(c.rows_r), c.G, t_run_if);
     MI_LAUNCH_CHECK("mlp_g_kernel");
-    MI_TRY(mlp_zero_accumulators(c, B));
+    MI_TRY(mlp_zero_accumulators(c, Bk));
   }
-  // ---- backward, panel by panel
-  for (long long r0 = 0; r0 < B; r0 += R) {
-    const long long rr = (B - r0 < R) ? (B - r0) : R, P = rr * B;
+  for (long long r0 = 0; r0 < Bq; r0 += R) {
+    const long long rr = (Bq - r0 < R) ? (Bq - r0) : R, P = rr * Bk;
     if (!dry) {
-      if (n_panels > 1) MI_TRY(gen_panel(r0, P));                 // a single panel is still resident from the forward
+      if (!resident) MI_TRY(mlp_tp_gen_panel(c, r0, P));
       Sched sc; mlp_z2_sched(c, P, sc);
       mi::EpiMlpDz::Params ep;
-      ep.b2 = c.b2p; ep.w3 = c.w3p; ep.g = c.G + r0 * B; ep.rows = static_cast<int>(P); ep.cols = static_cast<int>(H2);
+      ep.b2 = c.b2p; ep.w3 = c.w3p; ep.g = c.G + r0 * Bk; ep.rows = static_cast<int>(P); ep.cols = static_cast<int>(H2);
       ep.dz = c.DZ2; ep.dz_lo = c.sp == 2 ? c.DZ2 + c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
       MI_TRY(launch_engine<mi::EpiMlpDz>(MapSpec{c.Hpan, P, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
     }
     MI_TRY(mlp_dw2_gemm(c, P, r0 > 0, ws));
     MI_TRY(mlp_dz1_gemm(c, P, c.sp == 2 ? c.DZ1 : nullptr, c.sp == 1 ? c.DZ1h : nullptr, ws));
-    if (!dry) MI_TRY(mlp_reduce_panel(c, B, rr, r0));
+    if (!dry) MI_TRY(mlp_reduce_panel(c, Bk, rr, r0));
   }
   if (!dry) {
-    sum_reduce_kernel<<<1, 1024, 0, stream>>>(c.G, B * B, c.db3v, t_run_if);
+    sum_reduce_kernel<<<1, 1024, 0, stream>>>(c.G, Bq * Bk, c.db3v, t_run_if);
     MI_LAUNCH_CHECK("sum_reduce_kernel");
   }
   return MI_OK;
 }
+// the whole two-pass step of one GPU (the block is the batch)
+int mlp_two_pass(const MlpCtx& c, bool plan, Bump& ws) {
+  MI_TRY(mlp_tp_fwd(c, ws.dry));
+  if (!ws.dry) {
+    loss_finalize_kernel<<<1, 32, 0, c.stream>>>(c.scal, nullptr, c.Bg, c.estimator, c.loss_out, c.lse_f, nullptr, t_run_if);
+    MI_LAUNCH_CHECK("loss_finalize_kernel");
+  }
+  if (!plan) return MI_OK;
+  return mlp_tp_bwd(c, mlp_panel_rows(c.Bq, c.Bk) >= c.Bq, ws);
+}
 
-// reference of the single pass: the maximum logit over an n x n strided sample of the pairs (the margin is added in the epilogue)
+// reference of the single pass: the maximum logit over an n x n strided sample of the block's OWN pairs (image rows
+// x the text rows at the same global indices; the margin is added in the epilogue)
 constexpr long long kMlpRefSample = 256;
 int mlp_reference_logit(const MlpCtx& c, float* As, float* Cs, float* Ssmp, float* ref) {
-  const long long ns = c.B < kMlpRefSample ? c.B : kMlpRefSample, stride = c.B / ns, P = ns * ns;
+  const long long ns = c.Bq < kMlpRefSample ? c.Bq : kMlpRefSample, stride = c.Bq / ns, P = ns * ns;
   cudaStream_t stream = c.stream;
   gather_rows_kernel<<<blocks_for(ns * c.H1, 256), 256, 0, stream>>>(c.A32, stride, c.H1, As, ns);
   MI_LAUNCH_CHECK("gather_rows_kernel");
-  gather_rows_kernel<<<blocks_for(ns * c.H1, 256), 256, 0, stream>>>(c.C32, stride, c.H1, Cs, ns);
+  gather_rows_kernel<<<blocks_for(ns * c.H1, 256), 256, 0, stream>>>(c.C32 + c.q_off * c.H1, stride, c.H1, Cs, ns);
   MI_LAUNCH_CHECK("gather_rows_kernel");
-  mlp_gen_kernel<<<blocks_capped(P * (c.H1 >> 3), 256), 256, 0, stream>>>(As, Cs, c.H1, ns, 0, P, c.Hpan, c.pH, c.Hp, c.sp, 0, nullptr);
+  mlp_gen_kernel<<<blocks_capped(P * (c.H1 >> 3), 256), 256, 0, stream>>>(As, Cs, c.H1, ns, 0, P, c.Hpan, c.pH, c.Hp, c.sp, 0, 0, nullptr);
   MI_LAUNCH_CHECK("mlp_gen_kernel");
   Sched sc; mlp_z2_sched(c, P, sc);
   mi::EpiMlpFwd::Params ep;
@@ -551,34 +595,36 @@ void mlp_da_chunks(long long rr, long long per_chunk_units, int& chunk_len, int&
 
 // ---- the single pass (dv / infonce): see the header of this file
 struct MlpSpBuf { float *As, *Cs, *Ssmp, *ref, *cfac, *rowsum, *rowcnt, *diag, *gd, *DZ1d; uint32_t* mask; int* flag; double* guard_a; };
-int mlp_single_pass(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws) {
-  const long long B = c.B, H1 = c.H1, H2 = c.H2;
+// the panels against the reference sb.ref: raw accumulators in reference units (dW2, dA, dC, dw3, db2), the rows' sums of
+// g~ (sb.rowsum) and the block's scalar row (c.scal)
+int mlp_sp_panels(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws) {
+  const long long Bq = c.Bq, Bk = c.Bk, H1 = c.H1, H2 = c.H2;
   const bool dry = ws.dry;
   cudaStream_t stream = c.stream;
-  const long long Bp = round_up(B, rows_per_mblk());
-  const long long R = mlp_panel_rows(B, Bp);
+  const long long Bp = round_up(Bk, rows_per_mblk());
+  const long long R = mlp_panel_rows(Bq, Bp);
   const int wpr = static_cast<int>(round_up(cdiv(H1, 32), 2));          // even: the epilogue reads word pairs
   const bool fused_da = (g_mlp_mode.load(std::memory_order_relaxed) & 2) != 0;
   if (!dry) {
-    MI_TRY(mlp_reference_logit(c, sb.As, sb.Cs, sb.Ssmp, sb.ref));
     MI_TRY(mlp_zero_accumulators(c, Bp));
-    MI_CUDA(cudaMemsetAsync(sb.rowsum, 0, static_cast<size_t>(2 * B) * sizeof(float), stream));      // rowsum | rowcnt
+    MI_CUDA(cudaMemsetAsync(sb.rowsum, 0, static_cast<size_t>(2 * Bq) * sizeof(float), stream));      // rowsum | rowcnt
   }
-  for (long long r0 = 0; r0 < B; r0 += R) {
-    const long long rr = (B - r0 < R) ? (B - r0) : R, P = rr * Bp;
+  for (long long r0 = 0; r0 < Bq; r0 += R) {
+    const long long rr = (Bq - r0 < R) ? (Bq - r0) : R, P = rr * Bp;
     if (!dry) {
       {
         dim3 gg(blocks_for(cdiv(Bp, kGenJ) * 4 * wpr, 256), 1, 1);
         long long ny = cdiv(16LL * num_sms(), gg.x);              // enough blocks in flight to saturate the HBM writes
         if (ny > rr) ny = rr;
         gg.y = static_cast<unsigned>(ny < 1 ? 1 : ny);
-        mlp_gen2_kernel<<<gg, 256, 0, stream>>>(c.A32, c.C32, H1, B, Bp, r0, rr, c.Hpan, c.pH, c.Hp, c.sp, sb.mask, wpr);
+        mlp_gen2_kernel<<<gg, 256, 0, stream>>>(c.A32, c.C32, H1, Bk, Bp, r0, rr, c.Hpan, c.pH, c.Hp, c.sp, sb.mask, wpr);
         MI_LAUNCH_CHECK("mlp_gen2_kernel");
       }
       Sched sc; mlp_z2_sched(c, P, sc);
       mi::EpiMlpSp::Params ep;
-      ep.b2 = c.b2p; ep.w3 = c.w3p; ep.b3 = c.prm.b3; ep.ref = sb.ref; ep.sid = c.sid;
-      ep.B = static_cast<int>(B); ep.Bp = static_cast<int>(Bp); ep.r0 = static_cast<int>(r0); ep.rr = static_cast<int>(rr);
+      ep.b2 = c.b2p; ep.w3 = c.w3p; ep.b3 = c.prm.b3; ep.ref = sb.ref; ep.sid_q = c.sid_q; ep.sid_k = c.sid_k;
+      ep.B = static_cast<int>(Bk); ep.Bp = static_cast<int>(Bp); ep.r0 = static_cast<int>(r0); ep.rr = static_cast<int>(rr);
+      ep.q_off = static_cast<int>(c.q_off);
       ep.cols = static_cast<int>(H2);
       ep.dz = c.DZ2; ep.dz_lo = c.sp == 2 ? c.DZ2 + c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
       ep.rowsum = sb.rowsum; ep.rowcnt = sb.rowcnt; ep.diag_out = sb.diag; ep.S_out = S_out;
@@ -598,7 +644,7 @@ int mlp_single_pass(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws)
         sc.k_blocks = kb; sc.seg_len = kb;
         if (c.sp == 2) { sc.k_blocks = 3 * kb; sc.a_seg[1] = kb; sc.b_noff[2] = static_cast<int>(c.Hp); }
         mi::EpiMlpDa::Params ep;
-        ep.mask = sb.mask; ep.wpr = wpr; ep.B = static_cast<int>(B); ep.Bp = static_cast<int>(Bp);
+        ep.mask = sb.mask; ep.wpr = wpr; ep.B = static_cast<int>(Bk); ep.Bp = static_cast<int>(Bp);
         ep.r0 = static_cast<int>(r0); ep.rr = static_cast<int>(rr); ep.cols = static_cast<int>(H1);
         ep.dA = c.dA32; ep.dC = c.dC32;
         MI_TRY((launch_engine<mi::EpiMlpDa, false, true>(MapSpec{c.DZ2, P, c.eZ, c.pZ}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream)));
@@ -609,121 +655,140 @@ int mlp_single_pass(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws)
     }
   }
   if (!dry) {
-    // ---- estimator: row statistics from the sums, the shared fp64 finalisation (its guard checks |ref - LSE|)
-    mlp_rows_from_sums_kernel<<<blocks_for(B, 256), 256, 0, stream>>>(sb.rowsum, sb.rowcnt, sb.diag, sb.ref, B, reinterpret_cast<float4*>(c.rows_r));
+    // ---- estimator: row statistics from the sums, reduced like the separable critics' rows
+    mlp_rows_from_sums_kernel<<<blocks_for(Bq, 256), 256, 0, stream>>>(sb.rowsum, sb.rowcnt, sb.diag, sb.ref, Bq, reinterpret_cast<float4*>(c.rows_r));
     MI_LAUNCH_CHECK("mlp_rows_from_sums_kernel");
-    stats_reduce_kernel<<<1, 1024, 0, stream>>>(reinterpret_cast<const float4*>(c.rows_r), static_cast<int>(B), c.scal, nullptr);
+    stats_reduce_kernel<<<1, 1024, 0, stream>>>(reinterpret_cast<const float4*>(c.rows_r), static_cast<int>(Bq), c.scal, nullptr);
     MI_LAUNCH_CHECK("stats_reduce_kernel");
-    loss_finalize_kernel<<<1, 32, 0, stream>>>(c.scal, nullptr, B, c.estimator, c.loss_out, c.lse_f, nullptr, nullptr);
-    MI_LAUNCH_CHECK("loss_finalize_kernel");
-    mlp_weights_kernel<<<1, 1024, 0, stream>>>(sb.rowsum, B, sb.cfac, c.db3v, c.loss_out);
+  }
+  return MI_OK;
+}
+// the rest of the single pass once the loss is known (c.loss_out: n_neg of the batch; `total`: the sum of g~ over every
+// row block, NULL = this block is the batch; `guard_out`: where a trip of the weights' guard is reported, or NULL):
+// softmax weights, reference units -> weights, and the block's positive pairs (i, q_off + i): dL/dlogit = -1/Bg
+// (mi_critics.py:6,18), one panel of Bq pairs
+int mlp_sp_finish(const MlpCtx& c, const MlpSpBuf& sb, const double* total, double* guard_out, Bump& ws) {
+  const long long Bq = c.Bq, Bk = c.Bk, H1 = c.H1, H2 = c.H2;
+  const bool dry = ws.dry;
+  cudaStream_t stream = c.stream;
+  if (!dry) {
+    mlp_weights_kernel<<<1, 1024, 0, stream>>>(sb.rowsum, Bq, total, static_cast<double>(Bq) / static_cast<double>(c.Bg), c.loss_out + 3,
+                                               sb.cfac, c.db3v, guard_out);
     MI_LAUNCH_CHECK("mlp_weights_kernel");
-    // ---- reference units -> softmax weights
     float* bufs[5] = {c.dW2, c.dA32, c.dC32, c.acc_w3, c.acc_b2};
-    const long long lens[5] = {H2 * H1, B * H1, B * H1, c.h2_pad, c.h2_pad};
+    const long long lens[5] = {H2 * H1, Bq * H1, Bk * H1, c.h2_pad, c.h2_pad};
     for (int t = 0; t < 5; ++t) {
       mlp_rescale_kernel<<<blocks_capped(lens[t], 256), 256, 0, stream>>>(bufs[t], lens[t], sb.cfac);
       MI_LAUNCH_CHECK("mlp_rescale_kernel");
     }
-    // ---- the positive pairs (i, i): dL/dlogit = -1/B (mi_critics.py:6,18), one panel of B pairs
-    mlp_gen_kernel<<<blocks_capped(B * (H1 >> 3), 256), 256, 0, stream>>>(c.A32, c.C32, H1, B, 0, B, c.Hpan, c.pH, c.Hp, c.sp, 1, nullptr);
+    mlp_gen_kernel<<<blocks_capped(Bq * (H1 >> 3), 256), 256, 0, stream>>>(c.A32, c.C32, H1, Bk, 0, Bq, c.Hpan, c.pH, c.Hp, c.sp, 1, c.q_off,
+                                                                          nullptr);
     MI_LAUNCH_CHECK("mlp_gen_kernel");
-    fill_f32_kernel<<<blocks_for(B, 256), 256, 0, stream>>>(sb.gd, B, -1.f / static_cast<float>(B));
+    fill_f32_kernel<<<blocks_for(Bq, 256), 256, 0, stream>>>(sb.gd, Bq, -1.f / static_cast<float>(c.Bg));
     MI_LAUNCH_CHECK("fill_f32_kernel");
-    Sched sc; mlp_z2_sched(c, B, sc);
+    Sched sc; mlp_z2_sched(c, Bq, sc);
     mi::EpiMlpDz::Params ep;
-    ep.b2 = c.b2p; ep.w3 = c.w3p; ep.g = sb.gd; ep.rows = static_cast<int>(B); ep.cols = static_cast<int>(H2);
+    ep.b2 = c.b2p; ep.w3 = c.w3p; ep.g = sb.gd; ep.rows = static_cast<int>(Bq); ep.cols = static_cast<int>(H2);
     ep.dz = c.DZ2; ep.dz_lo = c.sp == 2 ? c.DZ2 + c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
-    MI_TRY(launch_engine<mi::EpiMlpDz>(MapSpec{c.Hpan, B, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
+    MI_TRY(launch_engine<mi::EpiMlpDz>(MapSpec{c.Hpan, Bq, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
   }
-  MI_TRY(mlp_dw2_gemm(c, B, true, ws));
-  MI_TRY(mlp_dz1_gemm(c, B, sb.DZ1d, nullptr, ws));
+  MI_TRY(mlp_dw2_gemm(c, Bq, true, ws));
+  MI_TRY(mlp_dz1_gemm(c, Bq, sb.DZ1d, nullptr, ws));
   if (!dry) {
-    mlp_add_diag_kernel<<<blocks_capped(B * H1, 256), 256, 0, stream>>>(sb.DZ1d, B * H1, c.dA32, c.dC32);
+    mlp_add_diag_kernel<<<blocks_capped(Bq * H1, 256), 256, 0, stream>>>(sb.DZ1d, Bq * H1, c.dA32, c.dC32 + c.q_off * H1);
     MI_LAUNCH_CHECK("mlp_add_diag_kernel");
   }
   return MI_OK;
 }
 
-int mlp_impl(const float* X, const float* Y, const MlpParams& prm, const int* sid, const MlpDims& d, int estimator, int precision,
-             double* loss_out, float* S_out, const MlpGrads& gr, Bump& ws, cudaStream_t stream) {
-  const long long B = d.B, D = d.D, H1 = d.H1, H2 = d.H2;
-  if (B <= 0 || D <= 0 || H1 <= 0 || H2 <= 0 || (D % 8) != 0 || (H1 % 8) != 0 || (H2 % 8) != 0) return MI_ERR_BAD_ARG;
-  if (H2 > mi::EpiMlpDz::kMaxTiles * mi::TILE_N) return MI_ERR_BAD_ARG;
-  if (estimator != MI_EST_DV && estimator != MI_EST_INFONCE_REF && estimator != MI_EST_INFONCE_ROW) return MI_ERR_BAD_ARG;
-  typedef __nv_bfloat16 bf;
-  const bool grads = gr.dX || gr.dY || gr.dW1 || gr.db1 || gr.dW2 || gr.db2 || gr.dW3 || gr.db3;
-  const bool plan = grads || ws.dry;
-  const bool dv_like = estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF;
-  // the workspace is planned for both sequences (the size query does not know the estimator's path)
-  const bool single = dv_like && plan && (g_mlp_mode.load(std::memory_order_relaxed) & 1) != 0;
-  MlpCtx c;
-  c.B = B; c.D = D; c.H1 = H1; c.H2 = H2; c.estimator = estimator; c.sid = sid; c.prm = prm; c.stream = stream; c.loss_out = loss_out;
+void mlp_ctx_dims(MlpCtx& c, long long D, long long H1, long long H2, int precision) {
+  c.D = D; c.H1 = H1; c.H2 = H2;
   c.sp = (precision & 1) == MI_PREC_BF16_STRICT ? 2 : 1;
   const int sp = c.sp;
   c.Dp = round_up(D, kSplitAlign); c.Hp = round_up(H1, kSplitAlign); c.H2p = round_up(H2, kSplitAlign);
   c.pX = sp == 2 ? 2 * c.Dp : D; c.pH = sp == 2 ? 2 * c.Hp : H1; c.pZ = sp == 2 ? 2 * c.H2p : H2;
   c.eX = sp == 2 ? c.Dp + D : D; c.eH = sp == 2 ? c.Hp + H1 : H1; c.eZ = sp == 2 ? c.H2p + H2 : H2;   // TMA extents
-  const long long Bp = round_up(B, rows_per_mblk());
-  const long long Pmax1 = mlp_panel_rows(B, B) * B, Pmax2 = mlp_panel_rows(B, Bp) * Bp;
-  const long long ns_ref = B < kMlpRefSample ? B : kMlpRefSample;        // the reference-logit sample is a panel too
-  long long Pmax = Pmax1 > Pmax2 ? Pmax1 : Pmax2;
-  if (Pmax < ns_ref * ns_ref) Pmax = ns_ref * ns_ref;
   c.nt2 = static_cast<int>(cdiv(H2, mi::TILE_N));
   c.h2_pad = static_cast<long long>(c.nt2) * mi::TILE_N;
+}
+bool mlp_dims_ok(const MlpDims& d, int estimator) {
+  if (d.B <= 0 || d.D <= 0 || d.H1 <= 0 || d.H2 <= 0 || (d.D % 8) != 0 || (d.H1 % 8) != 0 || (d.H2 % 8) != 0) return false;
+  if (d.H2 > mi::EpiMlpDz::kMaxTiles * mi::TILE_N) return false;
+  return estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF || estimator == MI_EST_INFONCE_ROW;
+}
+// fp32 [R, C] (pitch ld_in) -> the bf16 operand (hi, + lo in strict mode) of pitch `pitch`, lo half at column Cp
+int mlp_split(const MlpCtx& c, const float* in, long long ld_in, __nv_bfloat16* out, long long pitch, long long Cp, long long R, long long C) {
+  split_f32_kernel<<<blocks_for(R * pitch, 256), 256, 0, c.stream>>>(in, ld_in, out, pitch, c.sp, Cp, R, C, nullptr);
+  MI_LAUNCH_CHECK("split_f32_kernel");
+  return MI_OK;
+}
+
+// Carves the buffers of the MLP path over a block and runs its prologue: bf16 operands, layer 1 (A = X W1x^T + b1 for the
+// Bq image rows, C = Y W1y^T for the Bk text rows; fp32 out).  What the sharded step keeps between its forward and its
+// backward call (logits, row statistics, raw accumulators) comes from `keep`, the caller-owned state; on a single GPU
+// `keep` is the workspace itself.  `args_ok`: the caller's own pointer checks (reported after the workspace check).
+int mlp_setup(MlpCtx& c, MlpSpBuf& sb, const float* X, const float* Y, const MlpParams& prm, const MlpBlock& blk, const MlpDims& d,
+              int estimator, int precision, bool plan, float* S_out, float* dW2_out, double* loss_out, bool args_ok,
+              Bump& ws, Bump& keep, cudaStream_t stream) {
+  if (blk.Bq <= 0 || blk.Bk <= 0 || blk.q_off < 0 || blk.q_off + blk.Bq > blk.Bk || blk.Bk > blk.Bg) return MI_ERR_BAD_ARG;
+  typedef __nv_bfloat16 bf;
+  const long long Bq = blk.Bq, Bk = blk.Bk, D = d.D, H1 = d.H1, H2 = d.H2;
+  c.Bq = Bq; c.Bk = Bk; c.q_off = blk.q_off; c.Bg = blk.Bg; c.sid_q = blk.sid_q; c.sid_k = blk.sid_k;
+  c.estimator = estimator; c.prm = prm; c.stream = stream; c.loss_out = loss_out;
+  mlp_ctx_dims(c, D, H1, H2, precision);
+  const int sp = c.sp;
+  const long long Bp = round_up(Bk, rows_per_mblk());
+  const long long Pmax1 = mlp_panel_rows(Bq, Bk) * Bk, Pmax2 = mlp_panel_rows(Bq, Bp) * Bp;
+  const long long ns_ref = Bq < kMlpRefSample ? Bq : kMlpRefSample;      // the reference-logit sample is a panel too
+  long long Pmax = Pmax1 > Pmax2 ? Pmax1 : Pmax2;
+  if (Pmax < ns_ref * ns_ref) Pmax = ns_ref * ns_ref;
   const long long rows_padded_max = cdiv(Pmax, rows_per_mblk()) * rows_per_mblk();
   const long long pX = c.pX, pH = c.pH, pZ = c.pZ;
 
-  c.X16 = ws.take<bf>(B * pX); c.Y16 = ws.take<bf>(B * pX);
+  c.X16 = ws.take<bf>(Bq * pX); c.Y16 = ws.take<bf>(Bk * pX);
   c.W1x = ws.take<bf>(H1 * pX); c.W1y = ws.take<bf>(H1 * pX);
   c.W2h = ws.take<bf>(H2 * pH);
-  c.A32 = ws.take<float>(B * H1); c.C32 = ws.take<float>(B * H1);
+  c.A32 = ws.take<float>(Bq * H1); c.C32 = ws.take<float>(Bk * H1);
   c.b2p = ws.take<float>(c.h2_pad); c.w3p = ws.take<float>(c.h2_pad);
-  c.S = S_out ? S_out : ws.take<float>(B * B);
-  c.rows_r = ws.take<float>(B * 4);
+  c.S = S_out ? S_out : keep.take<float>(Bq * Bk);
+  c.rows_r = keep.take<float>(Bq * 4);
   c.scal = ws.take<double>(8);
   c.lse_f = ws.take<float>(1);
   c.db3v = ws.take<float>(1);
   c.Hpan = ws.take<bf>(Pmax * pH);
   c.part = ws.take<float>(mi::kColQuarters * rows_padded_max);
-  c.G = plan ? ws.take<float>(B * B) : nullptr;
+  c.G = plan ? ws.take<float>(Bq * Bk) : nullptr;
   c.DZ2 = plan ? ws.take<bf>(Pmax * pZ) : nullptr;
   // dZ1 panel: bf16 in fast mode (half the bytes of the HBM-write-bound masked contraction), fp32 in strict mode
   c.DZ1 = (plan && sp == 2) ? ws.take<float>(Pmax * H1) : nullptr;
   c.DZ1h = (plan && sp == 1) ? ws.take<bf>(Pmax * H1) : nullptr;
-  c.dA32 = plan ? ws.take<float>(B * H1) : nullptr; c.dC32 = plan ? ws.take<float>(Bp * H1) : nullptr;
-  c.dA16 = plan ? ws.take<bf>(B * pH) : nullptr; c.dC16 = plan ? ws.take<bf>(B * pH) : nullptr;
-  c.acc_w3 = plan ? ws.take<float>(c.h2_pad) : nullptr; c.acc_b2 = plan ? ws.take<float>(c.h2_pad) : nullptr;
-  float* dW2_tmp = (plan && !gr.dW2) ? ws.take<float>(H2 * H1) : nullptr;
-  MlpSpBuf sb{};
+  c.dA32 = plan ? keep.take<float>(Bq * H1) : nullptr; c.dC32 = plan ? keep.take<float>(Bp * H1) : nullptr;
+  c.dA16 = plan ? ws.take<bf>(Bq * pH) : nullptr; c.dC16 = plan ? ws.take<bf>(Bk * pH) : nullptr;
+  c.acc_w3 = plan ? keep.take<float>(c.h2_pad) : nullptr; c.acc_b2 = plan ? keep.take<float>(c.h2_pad) : nullptr;
+  float* dW2_tmp = (plan && !dW2_out) ? keep.take<float>(H2 * H1) : nullptr;
   if (plan) {
     const long long ns = ns_ref;
     sb.As = ws.take<float>(ns * H1); sb.Cs = ws.take<float>(ns * H1); sb.Ssmp = ws.take<float>(ns * ns);
     sb.ref = ws.take<float>(1); sb.cfac = ws.take<float>(1);
-    sb.rowsum = ws.take<float>(2 * B); sb.rowcnt = sb.rowsum ? sb.rowsum + B : nullptr;
-    sb.diag = ws.take<float>(B); sb.gd = ws.take<float>(B);
-    sb.DZ1d = ws.take<float>(B * H1);
+    sb.rowsum = keep.take<float>(2 * Bq); sb.rowcnt = sb.rowsum ? sb.rowsum + Bq : nullptr;
+    sb.diag = keep.take<float>(Bq); sb.gd = ws.take<float>(Bq);
+    sb.DZ1d = ws.take<float>(Bq * H1);
     sb.mask = ws.take<uint32_t>(Pmax2 * round_up(cdiv(H1, 32), 2));
     sb.flag = ws.take<int>(1); sb.guard_a = ws.take<double>(1);
   }
-  if (!ws.ok()) return MI_ERR_WORKSPACE;
+  if (!ws.ok() || !keep.ok()) return MI_ERR_WORKSPACE;
   c.mk = ws.mark();
-  c.dW2 = gr.dW2 ? gr.dW2 : dW2_tmp;
+  c.dW2 = dW2_out ? dW2_out : dW2_tmp;
   const size_t mk = c.mk;
   const bool dry = ws.dry;
-  if (!dry && (!X || !Y || !sid || !loss_out || !prm.W1 || !prm.b1 || !prm.W2 || !prm.b2 || !prm.W3 || !prm.b3)) return MI_ERR_BAD_ARG;
+  if (!dry && (!args_ok || !X || !Y || !prm.W1 || !prm.b1 || !prm.W2 || !prm.b2 || !prm.W3 || !prm.b3)) return MI_ERR_BAD_ARG;
 
-  auto split = [&](const float* in, long long ld_in, bf* out, long long pitch, long long Cp, long long Rr, long long Cc) -> int {
-    split_f32_kernel<<<blocks_for(Rr * pitch, 256), 256, 0, stream>>>(in, ld_in, out, pitch, sp, Cp, Rr, Cc, nullptr);
-    MI_LAUNCH_CHECK("split_f32_kernel");
-    return MI_OK;
-  };
   if (!dry) {
-    MI_TRY(split(X, D, c.X16, pX, c.Dp, B, D));
-    MI_TRY(split(Y, D, c.Y16, pX, c.Dp, B, D));
-    MI_TRY(split(prm.W1, 2 * D, c.W1x, pX, c.Dp, H1, D));            // W1 = [W1x | W1y]  (nn.Linear weight [H1, 2D])
-    MI_TRY(split(prm.W1 + D, 2 * D, c.W1y, pX, c.Dp, H1, D));
-    MI_TRY(split(prm.W2, H1, c.W2h, pH, c.Hp, H2, H1));
+    MI_TRY(mlp_split(c, X, D, c.X16, pX, c.Dp, Bq, D));
+    MI_TRY(mlp_split(c, Y, D, c.Y16, pX, c.Dp, Bk, D));
+    MI_TRY(mlp_split(c, prm.W1, 2 * D, c.W1x, pX, c.Dp, H1, D));            // W1 = [W1x | W1y]  (nn.Linear weight [H1, 2D])
+    MI_TRY(mlp_split(c, prm.W1 + D, 2 * D, c.W1y, pX, c.Dp, H1, D));
+    MI_TRY(mlp_split(c, prm.W2, H1, c.W2h, pH, c.Hp, H2, H1));
     pad_f32_kernel<<<blocks_for(c.h2_pad, 256), 256, 0, stream>>>(prm.b2, c.b2p, H2, c.h2_pad);
     MI_LAUNCH_CHECK("pad_f32_kernel");
     pad_f32_kernel<<<blocks_for(c.h2_pad, 256), 256, 0, stream>>>(prm.W3, c.w3p, H2, c.h2_pad);
@@ -735,16 +800,82 @@ int mlp_impl(const float* X, const float* Y, const MlpParams& prm, const int* si
   // ---- layer 1: A = X W1x^T + b1, C = Y W1y^T  (fp32 out)
   for (int side = 0; side < 2; ++side) {
     GemmArgs g;
-    g.a = MapSpec{side == 0 ? c.X16 : c.Y16, B, c.eX, pX};
+    const long long rows = side == 0 ? Bq : Bk;
+    g.a = MapSpec{side == 0 ? c.X16 : c.Y16, rows, c.eX, pX};
     g.b = MapSpec{side == 0 ? c.W1x : c.W1y, H1, c.eX, pX};
-    g.M = B; g.N = H1; kk_segments(g, sp, D);
+    g.M = rows; g.N = H1; kk_segments(g, sp, D);
     g.out_f32 = side == 0 ? c.A32 : c.C32; g.ld_out = H1;
     g.bias = side == 0 ? prm.b1 : nullptr;
     MI_TRY(run_gemm(g, ws, stream));
     ws.release(mk);
   }
+  return MI_OK;
+}
+
+// ---- layer 1 backward of ONE side over R rows (image side: dZ = dA, In = X, W1x; text side: dZ = dC, In = Y, W1y):
+//      dIn = dZ W1side, dW1[:, side] = dZ^T In (dW1_side points at the side's first column of the [H1, 2D] gradient),
+//      db1 = column sums of dZ (optional).  dZ comes as fp32 and as its bf16 operand; In16 / W16 are the bf16 operands.
+int mlp_layer1_bwd(const MlpCtx& c, long long R, const float* dZ32, __nv_bfloat16* dZ16, __nv_bfloat16* In16, __nv_bfloat16* W16,
+                   float* dIn, float* dW1_side, float* db1, Bump& ws) {
+  const long long D = c.D, H1 = c.H1, pX = c.pX, pH = c.pH;
+  const int sp = c.sp;
+  const bool dry = ws.dry;
+  const size_t mk = ws.mark();
+  if (db1 && !dry) { colsum_kernel<<<blocks_for(H1, 32), 256, 0, c.stream>>>(dZ32, R, H1, db1); MI_LAUNCH_CHECK("colsum_kernel"); }
+  if (dIn || dry) {   // dIn = dZ W1side : W1side [H1, D] read in place as the MN-major B operand
+    GemmArgs g;
+    g.a = MapSpec{dZ16, R, c.eH, pH};
+    g.b_mn = true; g.b = MapSpec{W16, H1, c.eX, pX};
+    g.M = R; g.N = D;
+    const int kb = static_cast<int>(sp == 2 ? c.Hp / bk() : cdiv(H1, bk()));
+    g.k_blocks = kb; g.seg_len = kb;
+    if (sp == 2) { g.k_blocks = 3 * kb; g.a_seg[1] = kb; g.b_noff[2] = static_cast<int>(c.Dp); }
+    g.out_f32 = dIn; g.ld_out = D;
+    if (dry) { g.out_f32 = reinterpret_cast<float*>(16); }
+    MI_TRY(run_gemm(g, ws, c.stream));
+    ws.release(mk);
+  }
+  if (dW1_side || dry) {   // dW1[:, side] = dZ^T In : contraction over the rows, both operands MN-major
+    GemmArgs g;
+    const int kb = static_cast<int>(cdiv(R, bk()));
+    g.a_mn = true; g.a = MapSpec{dZ16, R, c.eH, pH};
+    g.b_mn = true; g.b = MapSpec{In16, R, c.eX, pX};
+    g.M = H1; g.N = D; g.k_blocks = kb; g.seg_len = kb;
+    if (sp == 2) { g.k_blocks = 3 * kb; g.a_moff[1] = static_cast<int>(c.Hp); g.b_noff[2] = static_cast<int>(c.Dp); }
+    const long long tiles = cdiv(H1, rows_per_mblk()) * cdiv(D, mi::TILE_N);
+    g.ksplit = choose_ksplit(tiles, g.k_blocks);
+    g.out_f32 = dW1_side; g.ld_out = 2 * D;
+    if (dry) { g.out_f32 = reinterpret_cast<float*>(16); }
+    MI_TRY(run_gemm(g, ws, c.stream));
+    ws.release(mk);
+  }
+  return MI_OK;
+}
+
+// ---- the single-GPU step: the block form with Bq = Bk = Bg = B, q_off = 0, one id vector
+int mlp_impl(const float* X, const float* Y, const MlpParams& prm, const int* sid, const MlpDims& d, int estimator, int precision,
+             double* loss_out, float* S_out, const MlpGrads& gr, Bump& ws, cudaStream_t stream) {
+  if (!mlp_dims_ok(d, estimator)) return MI_ERR_BAD_ARG;
+  const long long B = d.B, D = d.D, H1 = d.H1, H2 = d.H2;
+  const bool grads = gr.dX || gr.dY || gr.dW1 || gr.db1 || gr.dW2 || gr.db2 || gr.dW3 || gr.db3;
+  const bool plan = grads || ws.dry;
+  const bool dv_like = estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF;
+  // the workspace is planned for both sequences (the size query does not know the estimator's path)
+  const bool single = dv_like && plan && (g_mlp_mode.load(std::memory_order_relaxed) & 1) != 0;
+  MlpCtx c;
+  MlpSpBuf sb{};
+  MI_TRY(mlp_setup(c, sb, X, Y, prm, MlpBlock{B, B, 0, B, sid, sid}, d, estimator, precision, plan, S_out, gr.dW2, loss_out,
+                   sid && loss_out, ws, ws, stream));
+  const bool dry = ws.dry;
   if (single || dry) {
-    MI_TRY(mlp_single_pass(c, sb, S_out, ws));
+    if (!dry) MI_TRY(mlp_reference_logit(c, sb.As, sb.Cs, sb.Ssmp, sb.ref));
+    MI_TRY(mlp_sp_panels(c, sb, S_out, ws));
+    if (!dry) {
+      // the shared fp64 finalisation (its guard checks |ref - LSE|)
+      loss_finalize_kernel<<<1, 32, 0, stream>>>(c.scal, nullptr, B, estimator, loss_out, c.lse_f, nullptr, nullptr);
+      MI_LAUNCH_CHECK("loss_finalize_kernel");
+    }
+    MI_TRY(mlp_sp_finish(c, sb, nullptr, dry ? nullptr : loss_out + 7, ws));
     if (!dry) {
       guard_to_flag_kernel<<<1, 1, 0, stream>>>(loss_out, sb.flag, sb.guard_a);
       MI_LAUNCH_CHECK("guard_to_flag_kernel");
@@ -765,43 +896,94 @@ int mlp_impl(const float* X, const float* Y, const MlpParams& prm, const int* si
     if (gr.dW3) { copy_f32_kernel<<<blocks_for(H2, 256), 256, 0, stream>>>(c.acc_w3, gr.dW3, H2); MI_LAUNCH_CHECK("copy_f32_kernel"); }
     if (gr.db2) { copy_f32_kernel<<<blocks_for(H2, 256), 256, 0, stream>>>(c.acc_b2, gr.db2, H2); MI_LAUNCH_CHECK("copy_f32_kernel"); }
     if (gr.db3) { copy_f32_kernel<<<1, 32, 0, stream>>>(c.db3v, gr.db3, 1); MI_LAUNCH_CHECK("copy_f32_kernel"); }
-    if (gr.db1) { colsum_kernel<<<blocks_for(H1, 32), 256, 0, stream>>>(c.dA32, B, H1, gr.db1); MI_LAUNCH_CHECK("colsum_kernel"); }
-    MI_TRY(split(c.dA32, H1, c.dA16, pH, c.Hp, B, H1));
-    MI_TRY(split(c.dC32, H1, c.dC16, pH, c.Hp, B, H1));
+    MI_TRY(mlp_split(c, c.dA32, H1, c.dA16, c.pH, c.Hp, B, H1));
+    MI_TRY(mlp_split(c, c.dC32, H1, c.dC16, c.pH, c.Hp, B, H1));
   }
-  // ---- layer 1 backward
-  for (int side = 0; side < 2; ++side) {
-    float* dIn = side == 0 ? gr.dX : gr.dY;
-    bf* dAc = side == 0 ? c.dA16 : c.dC16;
-    bf* Wside = side == 0 ? c.W1x : c.W1y;
-    bf* In16 = side == 0 ? c.X16 : c.Y16;
-    if (dIn || dry) {   // dX = dA W1x : W1x [H1, D] read in place as the MN-major B operand
-      GemmArgs g;
-      g.a = MapSpec{dAc, B, c.eH, pH};
-      g.b_mn = true; g.b = MapSpec{Wside, H1, c.eX, pX};
-      g.M = B; g.N = D;
-      const int kb = static_cast<int>(sp == 2 ? c.Hp / bk() : cdiv(H1, bk()));
-      g.k_blocks = kb; g.seg_len = kb;
-      if (sp == 2) { g.k_blocks = 3 * kb; g.a_seg[1] = kb; g.b_noff[2] = static_cast<int>(c.Dp); }
-      g.out_f32 = dIn; g.ld_out = D;
-      if (dry) { g.out_f32 = reinterpret_cast<float*>(16); }
-      MI_TRY(run_gemm(g, ws, stream));
-      ws.release(mk);
-    }
-    if (gr.dW1 || dry) {   // dW1[:, side] = dA^T X : contraction over the batch, both operands MN-major
-      GemmArgs g;
-      const int kb = static_cast<int>(cdiv(B, bk()));
-      g.a_mn = true; g.a = MapSpec{dAc, B, c.eH, pH};
-      g.b_mn = true; g.b = MapSpec{In16, B, c.eX, pX};
-      g.M = H1; g.N = D; g.k_blocks = kb; g.seg_len = kb;
-      if (sp == 2) { g.k_blocks = 3 * kb; g.a_moff[1] = static_cast<int>(c.Hp); g.b_noff[2] = static_cast<int>(c.Dp); }
-      const long long tiles = cdiv(H1, rows_per_mblk()) * cdiv(D, mi::TILE_N);
-      g.ksplit = choose_ksplit(tiles, g.k_blocks);
-      g.out_f32 = gr.dW1 ? gr.dW1 + side * D : nullptr; g.ld_out = 2 * D;
-      if (dry) { g.out_f32 = reinterpret_cast<float*>(16); }
-      MI_TRY(run_gemm(g, ws, stream));
-      ws.release(mk);
-    }
-  }
+  MI_TRY(mlp_layer1_bwd(c, B, c.dA32, c.dA16, c.X16, c.W1x, gr.dX, gr.dW1, gr.db1, ws));
+  MI_TRY(mlp_layer1_bwd(c, B, c.dC32, c.dC16, c.Y16, c.W1y, gr.dY, gr.dW1 ? gr.dW1 + D : nullptr, nullptr, ws));
   return MI_OK;
+}
+
+// ---- the stages of the batch-sharded step (DESIGN 8.4): one row block of Bq image rows against all Bk = Bg text rows.
+//      The caller's collectives go between the stages; everything that must survive from the forward to the backward
+//      lives in the caller-owned `state` (the scratch workspace is reused by whatever runs in between).
+enum MlpStage { kMlpStageRef = 0, kMlpStageFwd = 1, kMlpStageBwd = 2 };
+struct MlpBlockIO {
+  float* ref_out;           // stage ref: [1] maximum logit of the sample of the block's own pairs
+  const float* ref;         // stage fwd (single pass): [1] the reference of every block (maximum over the blocks)
+  int two_pass;
+  double* scal_out;         // stage fwd: [8] the block's scalar row (mi_score_stats layout, slot 7 = its sum of g~)
+  const double* loss;       // stage bwd: [8] loss_out of the batch (mi_mlp_block_merge)
+  const double* merged;     // stage bwd: [8] merged scalar row (slot 7 = the batch's sum of g~)
+  float* dC_part;           // stage bwd: [Bk, H1] the block's contribution to dL/dC
+  MlpGrads gr;              // stage bwd: dX (the block's rows), dW1 (image half), db1, dW2, db2, dW3, db3 of the block
+};
+int mlp_block_impl(int stage, const float* X, const float* Y, const MlpParams& prm, const MlpBlock& blk, const MlpDims& d,
+                   int estimator, int precision, const MlpBlockIO& io, Bump& ws, Bump& keep, cudaStream_t stream) {
+  if (!mlp_dims_ok(d, estimator)) return MI_ERR_BAD_ARG;
+  const long long H1 = d.H1, H2 = d.H2;
+  bool args_ok = true;
+  if (stage == kMlpStageRef) args_ok = io.ref_out != nullptr;
+  else if (stage == kMlpStageFwd) args_ok = blk.sid_q && blk.sid_k && io.scal_out && (io.two_pass || io.ref);
+  else if (stage == kMlpStageBwd) args_ok = blk.sid_q && blk.sid_k && io.loss && io.dC_part && (io.two_pass || io.merged);
+  else return MI_ERR_BAD_ARG;
+  MlpCtx c;
+  MlpSpBuf sb{};
+  MI_TRY(mlp_setup(c, sb, X, Y, prm, blk, d, estimator, precision, true, nullptr, nullptr, const_cast<double*>(io.loss), args_ok,
+                   ws, keep, stream));
+  const bool dry = ws.dry;
+  if (stage == kMlpStageRef) {
+    if (!dry) MI_TRY(mlp_reference_logit(c, sb.As, sb.Cs, sb.Ssmp, io.ref_out));
+    return MI_OK;
+  }
+  if (stage == kMlpStageFwd) {
+    if (!dry) c.scal = io.scal_out;
+    if (io.two_pass) return mlp_tp_fwd(c, dry);
+    sb.ref = const_cast<float*>(io.ref);
+    MI_TRY(mlp_sp_panels(c, sb, nullptr, ws));
+    if (!dry) {
+      sum_f64_kernel<<<1, 1024, 0, stream>>>(sb.rowsum, c.Bq, c.scal + 7);
+      MI_LAUNCH_CHECK("sum_f64_kernel");
+    }
+    return MI_OK;
+  }
+  if (io.two_pass) {
+    if (!dry) {
+      lse_from_loss_kernel<<<1, 1, 0, stream>>>(io.loss, c.lse_f);
+      MI_LAUNCH_CHECK("lse_from_loss_kernel");
+    }
+    MI_TRY(mlp_tp_bwd(c, false, ws));
+  } else {
+    MI_TRY(mlp_sp_finish(c, sb, io.merged ? io.merged + 7 : nullptr, nullptr, ws));
+  }
+  const MlpGrads& gr = io.gr;
+  if (!dry) {
+    if (gr.dW3) { copy_f32_kernel<<<blocks_for(H2, 256), 256, 0, stream>>>(c.acc_w3, gr.dW3, H2); MI_LAUNCH_CHECK("copy_f32_kernel"); }
+    if (gr.db2) { copy_f32_kernel<<<blocks_for(H2, 256), 256, 0, stream>>>(c.acc_b2, gr.db2, H2); MI_LAUNCH_CHECK("copy_f32_kernel"); }
+    if (gr.db3) { copy_f32_kernel<<<1, 32, 0, stream>>>(c.db3v, gr.db3, 1); MI_LAUNCH_CHECK("copy_f32_kernel"); }
+    if (gr.dW2) { copy_f32_kernel<<<blocks_for(H2 * H1, 256), 256, 0, stream>>>(c.dW2, gr.dW2, H2 * H1); MI_LAUNCH_CHECK("copy_f32_kernel"); }
+    MI_CUDA(cudaMemcpyAsync(io.dC_part, c.dC32, static_cast<size_t>(c.Bk) * H1 * sizeof(float), cudaMemcpyDeviceToDevice, stream));
+    MI_TRY(mlp_split(c, c.dA32, H1, c.dA16, c.pH, c.Hp, c.Bq, H1));
+  }
+  return mlp_layer1_bwd(c, c.Bq, c.dA32, c.dA16, c.X16, c.W1x, gr.dX, gr.dW1, gr.db1, ws);
+}
+// layer-1 backward of one side from fp32 inputs (the text side of the sharded step, after the exchange of dC)
+int mlp_input_grad_impl(const float* dZ, const float* In, const float* W1, int side, long long R, long long D, long long H1, int precision,
+                        float* dIn, float* dW1, float* db1, Bump& ws, cudaStream_t stream) {
+  if (R <= 0 || D <= 0 || H1 <= 0 || (D % 8) != 0 || (H1 % 8) != 0 || (side != 0 && side != 1)) return MI_ERR_BAD_ARG;
+  typedef __nv_bfloat16 bf;
+  MlpCtx c;
+  c.stream = stream;
+  mlp_ctx_dims(c, D, H1, 8, precision);
+  bf* dZ16 = ws.take<bf>(R * c.pH);
+  bf* In16 = ws.take<bf>(R * c.pX);
+  bf* W16 = ws.take<bf>(H1 * c.pX);
+  if (!ws.ok()) return MI_ERR_WORKSPACE;
+  if (!ws.dry) {
+    if (!dZ || !In || !W1) return MI_ERR_BAD_ARG;
+    MI_TRY(mlp_split(c, dZ, H1, dZ16, c.pH, c.Hp, R, H1));
+    MI_TRY(mlp_split(c, In, D, In16, c.pX, c.Dp, R, D));
+    MI_TRY(mlp_split(c, W1 + side * D, 2 * D, W16, c.pX, c.Dp, H1, D));
+  }
+  return mlp_layer1_bwd(c, R, dZ, dZ16, In16, W16, dIn, dW1 ? dW1 + side * D : nullptr, db1, ws);
 }

@@ -414,3 +414,102 @@ def sharded_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor, W:
     if rs_work is not None:
         rs_work.wait()                                # current (compute) stream waits for the collective
     return out, dX, dY, dW
+
+
+# ---- the reference's own critic, make_mlp(2D, [H1, H2]) (DESIGN 8.4): the same row-block sharding over stage ops
+#
+#   1. reference logit from a sample of the rank's OWN block (single pass only; no exchange needed), then ONE small
+#      all-gather of the study ids with the reference packed in (all-reduce MAX for int64 ids), and the all-gather of Y
+#   2. the block pass over Bl x Bg pairs (mi_mlp_block_fwd) -> the rank's scalar row (slot 7: its sum of the weights)
+#   3. all-gather of the 8 fp64 scalars, merge (mi_mlp_block_merge): the global loss and the single pass' guard — the same
+#      on every rank; a tripped guard repeats the step with the two-pass sequence
+#   4. the block's backward (mi_mlp_block_bwd): dX_r, the image half of dW1, partial dW2 / db2 / dW3 / db3 / db1 and the
+#      rank's contribution dC_part [Bg, H1] to dL/dC of every text row
+#   5. reduce-scatter of dC_part -> dC_r; dY_r and the text half of dW1 (mi_mlp_input_grad); ONE all-reduce of the flat
+#      parameter gradients
+
+MLP_GRAD_NAMES = ("dW1", "db1", "dW2", "db2", "dW3", "db3")
+
+
+def sharded_mlp_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor, params, sid_local: torch.Tensor,
+                                    estimator: str = "dv", precision: str = "fast", need_grads: bool = True, group=None,
+                                    backend=None, two_pass: bool = False, check_guard: bool = True):
+    """Global-batch loss of the concat-MLP critic when every rank holds a row shard (all ranks the same number of rows);
+    ``params`` = (W1 [H1, 2D], b1, W2 [H2, H1], b2, W3 [1, H2], b3), replicated.  Returns (stats dict of 0-d fp64 tensors
+    incl. 'loss' and 'guard', dX_local, dY_local, grads dict dW1 ... db3 already summed over ranks) — the gradients are
+    None without ``need_grads``.
+
+    dv / infonce with gradients take the single pass (unless mi_set_mlp_mode cleared bit 0); its guard is read on the host
+    after the scalar exchange and, if it tripped on the global weight sum, every rank repeats the step with the two-pass
+    sequence and reports guard = 1.  ``check_guard=False`` skips that host read; the verdict is then left in
+    stats['guard'] for the caller to act on.  infonce_row, forward-only calls and ``two_pass=True`` use the two-pass
+    sequence."""
+    if backend is None:
+        from . import ops as backend  # the CUDA path; raises if the library / device is missing
+    if estimator not in ("dv", "infonce", "infonce_ref", "infonce_row"):
+        raise ValueError(f"the MLP critic supports the dv, infonce and infonce_row estimators, not {estimator!r}")
+    world, rank = _world(group)
+    Bl, D = X_local.shape
+    Bg = Bl * world
+    off = rank * Bl
+    dv_like = estimator != "infonce_row"
+    single = need_grads and dv_like and not two_pass and (backend.get_mlp_mode() & 1) != 0
+    nccl = world > 1 and dist.get_backend(group) != "gloo"
+    X, Y = X_local.detach(), Y_local.detach()
+    params = tuple(p.detach() for p in params)
+
+    ref = backend.mlp_block_ref_logit(X, Y, params, 0, precision) if single else None
+    if sid_local.dtype == torch.int32:
+        if single and world > 1:
+            # ONE small all-gather carries the study ids and the reference (raw float bits)
+            meta = torch.cat((sid_local.reshape(-1), ref.reshape(1).to(torch.float32).view(torch.int32)))
+            meta_all = _all_gather_rows(meta.reshape(1, Bl + 1), world, group)
+            sid_all = meta_all[:, :Bl].reshape(-1).contiguous()
+            ref = meta_all[:, Bl].contiguous().view(torch.float32).max().reshape(1)
+        else:
+            sid_all = _all_gather_rows(sid_local.contiguous(), world, group)
+    else:                                                        # identical relabelling on every rank, no host sync
+        sid_all = dense_labels(_all_gather_rows(sid_local.to(torch.int64).contiguous(), world, group))
+        if single and world > 1:
+            ref = ref.clone()
+            dist.all_reduce(ref, op=dist.ReduceOp.MAX, group=group)
+    sid_loc = sid_all[off:off + Bl].contiguous()
+    Y_all = _all_gather_rows(Y.contiguous(), world, group)
+
+    # ---- the block pass and the scalar exchange
+    scal, state = backend.mlp_block_fwd(X, Y_all, params, sid_loc, sid_all, off, estimator, precision, ref, not single)
+    scal_all = _all_gather_rows(scal.reshape(1, 8), world, group)
+    loss, merged = backend.mlp_block_merge(scal_all, Bg, estimator, not single)
+    if single and check_guard and float(loss[7]) != 0.0:
+        # every rank sees the same merged rows: all of them repeat the step with exact statistics
+        out, dX, dY, grads = sharded_mlp_critic_loss_fwd_bwd(X_local, Y_local, params, sid_local, estimator, precision,
+                                                             need_grads, group, backend, two_pass=True)
+        out["guard"] = torch.ones((), dtype=torch.float64, device=out["loss"].device)
+        return out, dX, dY, grads
+    out = {"loss": loss[0], "pos_mean": loss[1], "lse_neg": loss[2], "n_neg": loss[3], "loss_row": loss[4],
+           "rows_without_negatives": loss[6], "guard": loss[7]}
+    if not need_grads:
+        return out, None, None, None
+
+    # ---- backward of the block, exchange of the dC contributions, layer 1 of the own text rows
+    g = backend.mlp_block_bwd(X, Y_all, params, sid_loc, sid_all, off, estimator, precision, not single, loss, merged, state)
+    ev = None
+    if nccl:
+        ev = torch.cuda.Event()
+        ev.record()
+    dC, rs_work = _reduce_scatter_rows(g["dC_part"], Bl, off, world, group, nccl, ev)
+    if rs_work is not None:
+        rs_work.wait()
+    if isinstance(dC, _A2ASum):
+        dC = dC.resolve()
+    dY, dW1, _ = backend.mlp_input_grad(dC, Y, params[0], 1, precision, dW1=g["dW1"])
+    grads = {"dW1": dW1, "db1": g["db1"], "dW2": g["dW2"], "db2": g["db2"], "dW3": g["dW3"], "db3": g["db3"]}
+    if world > 1:
+        flat = torch.cat([grads[n].reshape(-1) for n in MLP_GRAD_NAMES])
+        dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=group)
+        o = 0
+        for n in MLP_GRAD_NAMES:
+            k = grads[n].numel()
+            grads[n] = flat[o:o + k].view(grads[n].shape)
+            o += k
+    return out, g["dX"], dY, grads

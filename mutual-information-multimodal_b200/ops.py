@@ -590,6 +590,126 @@ def set_mlp_mode(mode: int) -> None:
     _lib.load().mi_set_mlp_mode(int(mode))
 
 
+def get_mlp_mode() -> int:
+    return int(_lib.load().mi_get_mlp_mode())
+
+
+# ---- the MLP critic over a row block: stage ops of the batch-sharded step (mi_b200.dist.sharded_mlp_critic_loss_fwd_bwd)
+
+def _mlp_operands(X, Y, params):
+    _need_cuda(X, Y, *params)
+    f32 = lambda t: t.detach().to(torch.float32).contiguous()
+    X, Y = f32(X), f32(Y)
+    W1, b1, W2, b2, W3, b3 = (f32(t) for t in params)
+    D = X.shape[1]
+    H1, H2 = W1.shape[0], W2.shape[0]
+    if (Y.shape[1] != D or W1.shape != (H1, 2 * D) or W2.shape != (H2, H1) or W3.numel() != H2 or b1.numel() != H1
+            or b2.numel() != H2 or b3.numel() != 1):
+        raise MIError("MLP critic parameters do not have the make_mlp(2D, [H1, H2]) shapes")
+    return X, Y, (W1, b1, W2, b2, W3, b3), D, H1, H2
+
+
+def _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev):
+    nbytes = _lib.load().mi_mlp_block_workspace_bytes(Bq, Bk, D, H1, H2, prec)
+    if nbytes == 0:
+        raise MIError("mi_mlp_block_workspace_bytes: unsupported shape (D, H1, H2 multiples of 8, H2 <= 512)")
+    return workspace(nbytes, dev)
+
+
+def _mlp_estimator(estimator):
+    if estimator not in ("dv", "infonce", "infonce_ref", "infonce_row"):
+        raise MIError("the MLP critic supports the dv, infonce and infonce_row estimators")
+    return ESTIMATOR[estimator]
+
+
+def mlp_block_ref_logit(X: torch.Tensor, Y: torch.Tensor, params, q_offset: int, precision: str = "fast") -> torch.Tensor:
+    """Maximum logit of a sample of the block's own pairs (image rows X against the text rows of Y at q_offset ..)
+    (mi_mlp_block_ref_logit) -> fp32 [1]."""
+    X, Y, prm, D, H1, H2 = _mlp_operands(X, Y, params)
+    Bq, Bk, prec = X.shape[0], Y.shape[0], PRECISION[precision]
+    ref = torch.empty(1, dtype=torch.float32, device=X.device)
+    ws = _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, X.device)
+    _check(_lib.load().mi_mlp_block_ref_logit(*(_ptr(t) for t in (X, Y) + prm), Bq, Bk, q_offset, D, H1, H2, prec, _ptr(ref),
+                                              _ptr(ws), ws.numel(), _stream()), "mi_mlp_block_ref_logit")
+    return ref
+
+
+def mlp_block_fwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor, sid_k: torch.Tensor, q_offset: int,
+                  estimator: str, precision: str, ref: Optional[torch.Tensor], two_pass: bool):
+    """The block's pass over its Bq x Bk pairs (mi_mlp_block_fwd) -> (scalar row fp64 [8], state).  ``state`` is an
+    opaque device buffer that carries the block to ``mlp_block_bwd``."""
+    X, Y, prm, D, H1, H2 = _mlp_operands(X, Y, params)
+    _need_cuda(sid_q, sid_k, ref)
+    Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), PRECISION[precision]
+    lib = _lib.load()
+    dev = X.device
+    sid_q, sid_k = sid_q.to(torch.int32).contiguous(), sid_k.to(torch.int32).contiguous()
+    ws = _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev)
+    state = torch.empty(lib.mi_mlp_block_state_bytes(Bq, Bk, D, H1, H2, prec), dtype=torch.uint8, device=dev)
+    scal = torch.empty(8, dtype=torch.float64, device=dev)
+    _check(lib.mi_mlp_block_fwd(*(_ptr(t) for t in (X, Y) + prm), _ptr(sid_q), _ptr(sid_k), Bq, Bk, q_offset, D, H1, H2, est, prec,
+                                _ptr(ref), int(two_pass), _ptr(scal), _ptr(state), state.numel(), _ptr(ws), ws.numel(), _stream()),
+           "mi_mlp_block_fwd")
+    return scal, state
+
+
+def mlp_block_merge(scal_all: torch.Tensor, b_global: int, estimator: str, two_pass: bool):
+    """Blocks' scalar rows [world, 8] -> (loss_out fp64 [8] of the batch, merged row fp64 [8]) (mi_mlp_block_merge)."""
+    _need_cuda(scal_all)
+    scal_all = scal_all.contiguous()
+    loss = torch.empty(8, dtype=torch.float64, device=scal_all.device)
+    merged = torch.empty(8, dtype=torch.float64, device=scal_all.device)
+    _check(_lib.load().mi_mlp_block_merge(_ptr(scal_all), scal_all.shape[0], b_global, _mlp_estimator(estimator), int(two_pass),
+                                          _ptr(loss), _ptr(merged), _stream()), "mi_mlp_block_merge")
+    return loss, merged
+
+
+def mlp_block_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor, sid_k: torch.Tensor, q_offset: int,
+                  estimator: str, precision: str, two_pass: bool, loss: torch.Tensor, merged: torch.Tensor, state: torch.Tensor) -> dict:
+    """The block's backward once the loss of the batch is known (mi_mlp_block_bwd).  Returns dX of the block's rows,
+    dC_part [Bk, H1] (the block's contribution to dL/dC of every text row), dW1 (image half filled), db1, dW2, db2, dW3, db3
+    (the block's shares)."""
+    X, Y, prm, D, H1, H2 = _mlp_operands(X, Y, params)
+    _need_cuda(sid_q, sid_k, loss, merged, state)
+    Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), PRECISION[precision]
+    dev = X.device
+    sid_q, sid_k = sid_q.to(torch.int32).contiguous(), sid_k.to(torch.int32).contiguous()
+    shapes = {"dX": (Bq, D), "dC_part": (Bk, H1), "dW1": (H1, 2 * D), "db1": (H1,), "dW2": (H2, H1), "db2": (H2,),
+              "dW3": (1, H2), "db3": (1,)}
+    g = {k: torch.empty(v, dtype=torch.float32, device=dev) for k, v in shapes.items()}
+    ws = _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev)
+    _check(_lib.load().mi_mlp_block_bwd(*(_ptr(t) for t in (X, Y) + prm), _ptr(sid_q), _ptr(sid_k), Bq, Bk, q_offset, D, H1, H2,
+                                        est, prec, int(two_pass), _ptr(loss), _ptr(merged), _ptr(state), state.numel(),
+                                        *(_ptr(g[k]) for k in shapes), _ptr(ws), ws.numel(), _stream()), "mi_mlp_block_bwd")
+    return g
+
+
+def mlp_input_grad(dZ: torch.Tensor, In: torch.Tensor, W1: torch.Tensor, side: int, precision: str = "fast",
+                   dW1: Optional[torch.Tensor] = None, want_db1: bool = False):
+    """Layer-1 backward of one side (mi_mlp_input_grad): dIn = dZ W1side; the side's half of dW1 [H1, 2D] is written
+    into ``dW1`` (allocated when None); db1 = column sums of dZ when asked.  Returns (dIn, dW1, db1 or None)."""
+    _need_cuda(dZ, In, W1, dW1)
+    dZ, In, W1 = (t.detach().to(torch.float32).contiguous() for t in (dZ, In, W1))
+    R, D = In.shape
+    H1 = W1.shape[0]
+    if dZ.shape != (R, H1) or W1.shape != (H1, 2 * D):
+        raise MIError("mlp_input_grad: dZ [R, H1], In [R, D], W1 [H1, 2D] expected")
+    if dW1 is None:
+        dW1 = torch.zeros((H1, 2 * D), dtype=torch.float32, device=In.device)
+    elif dW1.shape != (H1, 2 * D) or dW1.dtype != torch.float32 or not dW1.is_contiguous():
+        raise MIError("mlp_input_grad: dW1 must be a contiguous fp32 [H1, 2D] tensor")
+    dIn = torch.empty((R, D), dtype=torch.float32, device=In.device)
+    db1 = torch.empty(H1, dtype=torch.float32, device=In.device) if want_db1 else None
+    prec = PRECISION[precision]
+    nbytes = _lib.load().mi_mlp_input_grad_workspace_bytes(R, D, H1, prec)
+    if nbytes == 0:
+        raise MIError("mi_mlp_input_grad_workspace_bytes: unsupported shape (D, H1 multiples of 8)")
+    ws = workspace(nbytes, In.device)
+    _check(_lib.load().mi_mlp_input_grad(_ptr(dZ), _ptr(In), _ptr(W1), int(side), R, D, H1, prec, _ptr(dIn), _ptr(dW1), _ptr(db1),
+                                         _ptr(ws), ws.numel(), _stream()), "mi_mlp_input_grad")
+    return dIn, dW1, db1
+
+
 def gdv(pos: torch.Tensor, neg: torch.Tensor, precision: str = "strict") -> torch.Tensor:
     """mi_gdv: fp64[4] = {gdv, intra_pos, intra_neg, inter} of two [N, D] fp32 embedding sets (validate.py:16-49)."""
     _need_cuda(pos, neg)
