@@ -266,11 +266,13 @@ int mi_sharded_critic_loss_fwd_bwd(mi_dist_ctx* ctx, const void* X_local, const 
  * (main_utils.py:220-226) without building the [B + N_neg, 2D] pair tensor.  All tensors fp32, row-major, on the
  * device, in nn.Linear layout:  W1 [H1, 2D] (columns [0,D) act on the image embedding, [D,2D) on the text
  * embedding), b1 [H1], W2 [H2, H1], b2 [H2], W3 [1, H2], b3 [1].   D, H1, H2 multiples of 8, H2 <= 512.
- * estimator: MI_EST_DV, MI_EST_INFONCE_REF or MI_EST_INFONCE_ROW.  precision: MI_PREC_BF16_FAST (bf16 operands of
- * the tensor-core contractions, fp32 accumulate) or MI_PREC_BF16_STRICT (hi/lo bf16 pairs, 16 significant bits).
- * loss_out (fp64[8]) as mi_critic_loss_fwd_bwd.  dv / infonce with gradients run as a single pass (softmax weights against
+ * estimator: MI_EST_DV, MI_EST_INFONCE_REF, MI_EST_INFONCE_ROW or MI_EST_INFONCE_SYM.  precision: MI_PREC_BF16_FAST
+ * (bf16 operands of the tensor-core contractions, fp32 accumulate) or MI_PREC_BF16_STRICT (hi/lo bf16 pairs, 16
+ * significant bits).  loss_out (fp64[8]) as mi_critic_loss_fwd_bwd (slot 4 = loss_row, slot 5 = loss_col of
+ * MI_EST_INFONCE_SYM).  dv / infonce with gradients run as a single pass (softmax weights against
  * the maximum logit of a sample of pairs, Z2 formed once; see mi_set_mlp_mode); if its guard trips, the two-pass sequence
- * repeats the step behind a device-side predicate and loss_out[7] > 0 reports it.  The call never synchronises.
+ * repeats the step behind a device-side predicate and loss_out[7] > 0 reports it.  infonce_row and infonce_sym always run
+ * the two-pass sequence (their row / column normalisers need every logit first).  The call never synchronises.
  * S_out (optional, [B, B]) receives the logit of EVERY pair
  * (S[i,j] = mlp([x_i ; y_j]); the reference's logits are its diagonal followed by its negatives in gap-major
  * order).  Every gradient pointer may be NULL; all NULL = forward only. */
@@ -290,13 +292,19 @@ int mi_mlp_critic_loss_fwd_bwd(const float* X, const float* Y, const float* W1, 
  *   2. mi_mlp_block_fwd        the block's pass over its Bq x Bk pairs -> scal_out[8], the block's scalar row in the
  *      mi_score_stats layout (slot 7: the block's sum of the softmax weights in reference units, single pass only).
  *      two_pass = 0: the single pass against `ref` (same value on every rank); 1: the logits are formed first (exact).
- *   3. (caller) all-gather of the scalar rows -> scal_all [world, 8]
+ *      mi_mlp_block_fwd_rc (MI_EST_INFONCE_SYM, two_pass = 1 only) also writes col_lse_out [Bk]: for every text row j the
+ *      log-sum-exp of the block's logits S[i, j] over its negatives and, when j = q_offset + i lies in the block, the
+ *      positive pair (-inf if the set is empty).  The column of the batch is the log-sum-exp of the ranks' values.
+ *   3. (caller) all-gather of the scalar rows -> scal_all [world, 8] (MI_EST_INFONCE_SYM: and of the column partials)
  *   4. mi_mlp_block_merge      -> loss_out[8] of the batch (mi_mlp_critic_loss_fwd_bwd's layout) and merged[8] (the merged
  *      row, slot 7 summed).  Single pass: loss_out[7] != 0 when the global weight sum left [1e-30, 1e30] while negatives
  *      exist — the same verdict on every rank; the caller then repeats the step with two_pass = 1.
+ *      MI_EST_INFONCE_SYM (two_pass = 1 only): every slot as for MI_EST_INFONCE_ROW; the caller completes slot 5
+ *      (loss_col = (sum_j c_j - B_global * slot 1) / B_global, c = the merged columns) and slot 0 (= (slot 4 + slot 5) / 2).
  *   5. mi_mlp_block_bwd        -> dX of the block's rows, dC_part [Bk, H1] (the block's contribution to dL/dC for EVERY
  *      text row, to be summed over ranks), the image half of dW1 ([H1, 2D] pitch, columns [0, D)), db1, dW2, db2, dW3,
- *      db3: the block's shares (sum over ranks = the gradient of the global loss).
+ *      db3: the block's shares (sum over ranks = the gradient of the global loss).  mi_mlp_block_bwd_rc takes col_lse [Bk],
+ *      the merged columns of the batch (MI_EST_INFONCE_SYM; NULL otherwise).
  *   6. (caller) reduce-scatter of dC_part -> dC [Bq, H1] of the own text rows;
  *      mi_mlp_input_grad(dC, Y_own, W1, side = 1) -> dY of the own rows and the text half of dW1; all-reduce of the
  *      parameter gradients.
@@ -313,6 +321,11 @@ int mi_mlp_block_fwd(const float* X, const float* Y, const float* W1, const floa
                      int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
                      const float* ref, int two_pass, double* scal_out, void* state, size_t state_bytes,
                      void* workspace, size_t workspace_bytes, mi_stream_t stream);
+int mi_mlp_block_fwd_rc(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                        const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                        int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                        const float* ref, int two_pass, double* scal_out, float* col_lse_out, void* state, size_t state_bytes,
+                        void* workspace, size_t workspace_bytes, mi_stream_t stream);
 int mi_mlp_block_merge(const double* scal_all, int world, int64_t B_global, int estimator, int two_pass, double* loss_out,
                        double* merged, mi_stream_t stream);
 int mi_mlp_block_bwd(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
@@ -321,6 +334,12 @@ int mi_mlp_block_bwd(const float* X, const float* Y, const float* W1, const floa
                      int two_pass, const double* loss, const double* merged, void* state, size_t state_bytes,
                      float* dX, float* dC_part, float* dW1, float* db1, float* dW2, float* db2, float* dW3, float* db3,
                      void* workspace, size_t workspace_bytes, mi_stream_t stream);
+int mi_mlp_block_bwd_rc(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                        const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                        int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                        int two_pass, const double* loss, const double* merged, const float* col_lse, void* state, size_t state_bytes,
+                        float* dX, float* dC_part, float* dW1, float* db1, float* dW2, float* db2, float* dW3, float* db3,
+                        void* workspace, size_t workspace_bytes, mi_stream_t stream);
 /* Layer-1 backward of one side of the MLP critic over R rows: dZ [R, H1] = dL/d(W1side in), In [R, D], W1 the full [H1, 2D]
  * weight; side 0 = image (W1x, columns [0, D)), 1 = text (W1y, columns [D, 2D)).  dIn = dZ W1side [R, D], the side's
  * half of dW1 [H1, 2D] = dZ^T In, db1 (optional) = column sums of dZ.  Any output may be NULL. */

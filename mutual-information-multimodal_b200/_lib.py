@@ -75,9 +75,13 @@ PROTOTYPES = {
     "mi_mlp_block_state_bytes": (c_sz, [c_i64, c_i64, c_i64, c_i64, c_i64, c_int]),
     "mi_mlp_block_ref_logit": (c_int, [c_vp] * 8 + [c_i64] * 6 + [c_int, c_vp, c_vp, c_sz, c_vp]),
     "mi_mlp_block_fwd": (c_int, [c_vp] * 10 + [c_i64] * 6 + [c_int, c_int, c_vp, c_int, c_vp, c_vp, c_sz, c_vp, c_sz, c_vp]),
+    "mi_mlp_block_fwd_rc": (c_int, [c_vp] * 10 + [c_i64] * 6 + [c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_sz, c_vp, c_sz,
+                                                               c_vp]),
     "mi_mlp_block_merge": (c_int, [c_vp, c_int, c_i64, c_int, c_int, c_vp, c_vp, c_vp]),
     "mi_mlp_block_bwd": (c_int, [c_vp] * 10 + [c_i64] * 6 + [c_int, c_int, c_int, c_vp, c_vp, c_vp, c_sz] + [c_vp] * 8
                          + [c_vp, c_sz, c_vp]),
+    "mi_mlp_block_bwd_rc": (c_int, [c_vp] * 10 + [c_i64] * 6 + [c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_sz] + [c_vp] * 8
+                            + [c_vp, c_sz, c_vp]),
     "mi_mlp_input_grad_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64, c_int]),
     "mi_mlp_input_grad": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "mi_gdv_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64, c_int]),

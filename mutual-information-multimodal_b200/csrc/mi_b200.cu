@@ -2397,27 +2397,39 @@ int mi_mlp_block_ref_logit(const float* X, const float* Y, const float* W1, cons
   return mlp_block_impl(kMlpStageRef, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, nullptr, nullptr},
                         MlpDims{Bk, D, H1, H2}, MI_EST_DV, precision, io, ws, ws, reinterpret_cast<cudaStream_t>(stream));
 }
+int mi_mlp_block_fwd_rc(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                        const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                        int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                        const float* ref, int two_pass, double* scal_out, float* col_lse_out, void* state, size_t state_bytes,
+                        void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+  MI_TRY(device_check());
+  Bump ws(workspace, workspace_bytes, false), keep(state, state_bytes, false);
+  MlpBlockIO io{};
+  io.ref = ref; io.two_pass = two_pass; io.scal_out = scal_out; io.col_lse_out = col_lse_out;
+  return mlp_block_impl(kMlpStageFwd, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, sid_q, sid_k},
+                        MlpDims{Bk, D, H1, H2}, estimator, precision, io, ws, keep, reinterpret_cast<cudaStream_t>(stream));
+}
 int mi_mlp_block_fwd(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
                      const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
                      int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
                      const float* ref, int two_pass, double* scal_out, void* state, size_t state_bytes,
                      void* workspace, size_t workspace_bytes, mi_stream_t stream) {
-  MI_TRY(device_check());
-  Bump ws(workspace, workspace_bytes, false), keep(state, state_bytes, false);
-  MlpBlockIO io{};
-  io.ref = ref; io.two_pass = two_pass; io.scal_out = scal_out;
-  return mlp_block_impl(kMlpStageFwd, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, sid_q, sid_k},
-                        MlpDims{Bk, D, H1, H2}, estimator, precision, io, ws, keep, reinterpret_cast<cudaStream_t>(stream));
+  return mi_mlp_block_fwd_rc(X, Y, W1, b1, W2, b2, W3, b3, sid_q, sid_k, Bq, Bk, q_offset, D, H1, H2, estimator, precision, ref,
+                             two_pass, scal_out, nullptr, state, state_bytes, workspace, workspace_bytes, stream);
 }
 int mi_mlp_block_merge(const double* scal_all, int world, int64_t B_global, int estimator, int two_pass, double* loss_out, double* merged,
                        mi_stream_t stream_) {
   MI_TRY(device_check());
-  if (!scal_all || world <= 0 || B_global <= 0 || !loss_out || !merged ||
-      (estimator != MI_EST_DV && estimator != MI_EST_INFONCE_REF && estimator != MI_EST_INFONCE_ROW)) return MI_ERR_BAD_ARG;
+  const bool sym = estimator == MI_EST_INFONCE_SYM;
+  if (!scal_all || world <= 0 || B_global <= 0 || !loss_out || !merged || (sym && !two_pass) ||
+      (estimator != MI_EST_DV && estimator != MI_EST_INFONCE_REF && estimator != MI_EST_INFONCE_ROW && !sym)) return MI_ERR_BAD_ARG;
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   merge_scal_kernel<<<1, 32, 0, stream>>>(scal_all, world, merged);
   MI_LAUNCH_CHECK("merge_scal_kernel");
-  loss_finalize_kernel<<<1, 32, 0, stream>>>(merged, nullptr, B_global, estimator, loss_out, nullptr, nullptr, nullptr);
+  // symmetric InfoNCE: the slots of infonce_row (slot 0 = loss_row, slot 5 = 0); the caller completes 0 and 5 from the
+  // merged columns
+  loss_finalize_kernel<<<1, 32, 0, stream>>>(merged, nullptr, B_global, sym ? MI_EST_INFONCE_ROW : estimator, loss_out, nullptr, nullptr,
+                                             nullptr);
   MI_LAUNCH_CHECK("loss_finalize_kernel");
   if (!two_pass) {
     mlp_block_guard_kernel<<<1, 1, 0, stream>>>(merged, loss_out);
@@ -2425,19 +2437,29 @@ int mi_mlp_block_merge(const double* scal_all, int world, int64_t B_global, int 
   }
   return MI_OK;
 }
+int mi_mlp_block_bwd_rc(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
+                        const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
+                        int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
+                        int two_pass, const double* loss, const double* merged, const float* col_lse, void* state, size_t state_bytes,
+                        float* dX, float* dC_part, float* dW1, float* db1, float* dW2, float* db2, float* dW3, float* db3,
+                        void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+  MI_TRY(device_check());
+  Bump ws(workspace, workspace_bytes, false), keep(state, state_bytes, false);
+  MlpBlockIO io{};
+  io.two_pass = two_pass; io.loss = loss; io.merged = merged; io.col_lse = col_lse; io.dC_part = dC_part;
+  io.gr = MlpGrads{dX, nullptr, dW1, db1, dW2, db2, dW3, db3};
+  return mlp_block_impl(kMlpStageBwd, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, sid_q, sid_k},
+                        MlpDims{Bk, D, H1, H2}, estimator, precision, io, ws, keep, reinterpret_cast<cudaStream_t>(stream));
+}
 int mi_mlp_block_bwd(const float* X, const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
                      const float* W3, const float* b3, const int32_t* sid_q, const int32_t* sid_k,
                      int64_t Bq, int64_t Bk, int64_t q_offset, int64_t D, int64_t H1, int64_t H2, int estimator, int precision,
                      int two_pass, const double* loss, const double* merged, void* state, size_t state_bytes,
                      float* dX, float* dC_part, float* dW1, float* db1, float* dW2, float* db2, float* dW3, float* db3,
                      void* workspace, size_t workspace_bytes, mi_stream_t stream) {
-  MI_TRY(device_check());
-  Bump ws(workspace, workspace_bytes, false), keep(state, state_bytes, false);
-  MlpBlockIO io{};
-  io.two_pass = two_pass; io.loss = loss; io.merged = merged; io.dC_part = dC_part;
-  io.gr = MlpGrads{dX, nullptr, dW1, db1, dW2, db2, dW3, db3};
-  return mlp_block_impl(kMlpStageBwd, X, Y, MlpParams{W1, b1, W2, b2, W3, b3}, MlpBlock{Bq, Bk, q_offset, Bk, sid_q, sid_k},
-                        MlpDims{Bk, D, H1, H2}, estimator, precision, io, ws, keep, reinterpret_cast<cudaStream_t>(stream));
+  return mi_mlp_block_bwd_rc(X, Y, W1, b1, W2, b2, W3, b3, sid_q, sid_k, Bq, Bk, q_offset, D, H1, H2, estimator, precision, two_pass,
+                             loss, merged, nullptr, state, state_bytes, dX, dC_part, dW1, db1, dW2, db2, dW3, db3, workspace,
+                             workspace_bytes, stream);
 }
 size_t mi_mlp_input_grad_workspace_bytes(int64_t R, int64_t D, int64_t H1, int precision) {
   Bump ws(nullptr, 0, true);

@@ -11,7 +11,8 @@
 //
 // Pairs are processed in row panels (rows i in [r0, r0 + R), all columns j; pair index p = (i - r0) B + j):
 //   forward   H[p,:] = bf16 h1  ->  tile engine  Z2 = H W2^T  with the EpiMlpFwd epilogue  ->  S (fp32 [B, B])
-//   loss      row statistics of S over the negatives mask -> DV / InfoNCE exactly as for the separable critics; G = dL/dS
+//   loss      row statistics of S over the negatives mask (symmetric InfoNCE: and column statistics) -> DV / InfoNCE
+//             exactly as for the separable critics; G = dL/dS
 //   backward  recompute Z2 with the EpiMlpDz epilogue -> dZ2 panel (bf16), dw3, db2;
 //             dW2 += dZ2^T H          (both operands read MN-major, contraction over the pairs, split-K)
 //             dZ1  = (dZ2 W2) . [H > 0]  (W2 read MN-major; ReLU mask in the epilogue), reduced over j -> dA_i, over i -> dC_j
@@ -200,6 +201,58 @@ __global__ void mlp_row_stats_kernel(const float* __restrict__ S, const int* __r
     row_out[row] = make_float4(lse_neg, cnt, diag, hi + log1pf(expf(lo - hi)));
   }
 }
+// Columns of S [Bq, Bk] (symmetric InfoNCE), in two launches.  Part 1: thread = column j (consecutive threads read
+// consecutive j of a row), blockIdx.y = a slice of the rows; the same online (max, sum exp) as mlp_row_stats_kernel over
+// the slice's negatives of column j, and their count.  part = {m, s, cnt}, each [gridDim.y][Bk].
+constexpr int kMlpColSplits = 32;                         // most row slices (the part buffer is planned for this many)
+__global__ void mlp_col_part_kernel(const float* __restrict__ S, const int* __restrict__ sid_q, const int* __restrict__ sid_k,
+                                    long long Bq, long long Bk, float* __restrict__ part, const int* __restrict__ run_if) {
+  MI_PRED(run_if);
+  const long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (j >= Bk) return;
+  const long long per = (Bq + gridDim.y - 1) / gridDim.y;
+  const long long i0 = blockIdx.y * per, i1 = i0 + per < Bq ? i0 + per : Bq;
+  const int my = sid_k[j];
+  float m = mi::neg_inf(), s = 0.f, cnt = 0.f;
+  for (long long i = i0; i < i1; ++i) {
+    if (sid_q[i] != my) {
+      const float v = S[i * Bk + j];
+      const float mn = fmaxf(m, v);
+      s = s * expf(m - mn) + expf(v - mn); m = mn; cnt += 1.f;
+    }
+  }
+  const long long o = blockIdx.y * Bk + j, n = static_cast<long long>(gridDim.y) * Bk;
+  part[o] = m; part[n + o] = s; part[2 * n + o] = cnt;
+}
+// Part 2, per column j: merge of the n_split slices, then the positive pair S[j - q_off, j] if it lies in the block.
+// col_lse[j] = log-sum-exp over {i in the block : (i, j) in negatives u positives} (-inf: none).  col_out (square block
+// only): the float4 of mlp_row_stats_kernel's layout for the column, {lse over the negatives, #negatives, S[j, j], col_lse[j]}.
+__global__ void mlp_col_merge_kernel(const float* __restrict__ part, int n_split, const float* __restrict__ S, long long Bq,
+                                     long long Bk, long long q_off, float* __restrict__ col_lse, float4* __restrict__ col_out,
+                                     const int* __restrict__ run_if) {
+  MI_PRED(run_if);
+  const long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (j >= Bk) return;
+  const long long n = static_cast<long long>(n_split) * Bk;
+  float m = mi::neg_inf(), s = 0.f, cnt = 0.f;
+  for (int y = 0; y < n_split; ++y) {
+    const float m2 = part[y * Bk + j], s2 = part[n + y * Bk + j];
+    cnt += part[2 * n + y * Bk + j];
+    const float mn = fmaxf(m, m2);
+    if (mn > mi::neg_inf()) s = s * expf(m - mn) + s2 * expf(m2 - mn);
+    m = mn;
+  }
+  const float lse_neg = (cnt > 0.f && s > 0.f) ? m + logf(s) : mi::neg_inf();
+  const long long i = j - q_off;
+  float diag = mi::neg_inf(), lse = lse_neg;
+  if (i >= 0 && i < Bq) {
+    diag = S[i * Bk + j];
+    const float hi = fmaxf(lse_neg, diag), lo = fminf(lse_neg, diag);
+    lse = hi + log1pf(expf(lo - hi));
+  }
+  col_lse[j] = lse;
+  if (col_out) col_out[j] = make_float4(lse_neg, cnt, diag, lse);
+}
 // the same float4 per row from the single pass' sums: lse over the negatives = ref + log(sum_j g~)
 __global__ void mlp_rows_from_sums_kernel(const float* __restrict__ rowsum, const float* __restrict__ rowcnt,
                                           const float* __restrict__ diag, const float* __restrict__ ref, long long B,
@@ -216,10 +269,12 @@ __global__ void mlp_rows_from_sums_kernel(const float* __restrict__ rowsum, cons
 }
 // G = dL/dS over a block [Bq, Bk] (image rows at q_off) of a batch of Bg.  dv / infonce (mi_critics.py:3-23): softmax
 // over ALL negatives (lse = the global log-sum-exp), -1/Bg on the diagonal; row InfoNCE: (1/Bg) softmax over {positive} u
-// negatives of the row, minus 1/Bg on the diagonal.
+// negatives of the row, minus 1/Bg on the diagonal; symmetric InfoNCE (col_lse != NULL: the log-sum-exp of every column
+// over ALL rows of the batch): the mean of the row and the column softmax, minus 1/Bg on the diagonal.
 __global__ void mlp_g_kernel(const float* __restrict__ S, const int* __restrict__ sid_q, const int* __restrict__ sid_k, long long Bq,
                              long long Bk, long long q_off, long long Bg, int dv_like, const float* __restrict__ lse,
-                             const float4* __restrict__ rows, float* __restrict__ G, const int* __restrict__ run_if) {
+                             const float4* __restrict__ rows, const float* __restrict__ col_lse, float* __restrict__ G,
+                             const int* __restrict__ run_if) {
   MI_PRED(run_if);
   const long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (idx >= Bq * Bk) return;
@@ -229,7 +284,11 @@ __global__ void mlp_g_kernel(const float* __restrict__ S, const int* __restrict_
   const bool pos = j == q_off + i;
   float g = 0.f;
   if (dv_like) g = neg ? expf(S[idx] - lse[0]) : (pos ? -inv_b : 0.f);
-  else if (neg || pos) g = inv_b * expf(S[idx] - rows[i].w) - (pos ? inv_b : 0.f);
+  else if (neg || pos) {
+    const float v = S[idx];
+    const float e = col_lse ? 0.5f * (expf(v - rows[i].w) + expf(v - col_lse[j])) : expf(v - rows[i].w);
+    g = inv_b * e - (pos ? inv_b : 0.f);
+  }
   G[idx] = g;
 }
 // One read of the dZ1 panel gives both reductions.  A block owns a slab [32 rows il] x [all j] x [64 columns]:
@@ -413,7 +472,8 @@ struct MlpCtx {
   MlpParams prm;
   __nv_bfloat16 *X16, *Y16, *W1x, *W1y, *W2h, *Hpan, *DZ2, *DZ1h, *dA16, *dC16;
   float *A32, *C32, *b2p, *w3p, *S, *rows_r, *lse_f, *part, *G, *DZ1, *dA32, *dC32, *acc_w3, *acc_b2, *dW2, *db3v;
-  double* scal;
+  float *col_part, *col_lse, *cols_r;     // symmetric InfoNCE: column partials, column log-sum-exp, column float4s
+  double *scal, *scal_col;
   double* loss_out;
   cudaStream_t stream;
   size_t mk;
@@ -511,7 +571,27 @@ int mlp_tp_fwd(const MlpCtx& c, bool dry) {
   MI_LAUNCH_CHECK("stats_reduce_kernel");
   return MI_OK;
 }
-// backward, once the loss is known (c.lse_f: the global log-sum-exp; c.rows_r: the block's row statistics): G, then Z2
+// column statistics of the block's stored logits (symmetric InfoNCE): col_lse [Bk] as mlp_col_merge_kernel; `square`
+// (the block is the batch): also the columns' float4s (c.cols_r) reduced to the scalar row c.scal_col.  The row slices
+// fill the machine: Bk / 256 column blocks alone are 16 - 32 blocks at Bk = 4096 - 8192.
+int mlp_col_stats(const MlpCtx& c, float* col_lse, bool square) {
+  const unsigned gx = blocks_for(c.Bk, 256);
+  long long ny = cdiv(4LL * num_sms(), gx);
+  if (ny > kMlpColSplits) ny = kMlpColSplits;
+  if (ny > c.Bq) ny = c.Bq;
+  mlp_col_part_kernel<<<dim3(gx, static_cast<unsigned>(ny)), 256, 0, c.stream>>>(c.S, c.sid_q, c.sid_k, c.Bq, c.Bk, c.col_part, t_run_if);
+  MI_LAUNCH_CHECK("mlp_col_part_kernel");
+  float4* cols = square ? reinterpret_cast<float4*>(c.cols_r) : nullptr;
+  mlp_col_merge_kernel<<<gx, 256, 0, c.stream>>>(c.col_part, static_cast<int>(ny), c.S, c.Bq, c.Bk, c.q_off, col_lse, cols, t_run_if);
+  MI_LAUNCH_CHECK("mlp_col_merge_kernel");
+  if (square) {
+    stats_reduce_kernel<<<1, 1024, 0, c.stream>>>(cols, static_cast<int>(c.Bk), c.scal_col, t_run_if);
+    MI_LAUNCH_CHECK("stats_reduce_kernel");
+  }
+  return MI_OK;
+}
+// backward, once the loss is known (c.lse_f: the global log-sum-exp; c.rows_r: the block's row statistics; c.col_lse:
+// symmetric InfoNCE, the log-sum-exp of every column over the batch): G, then Z2
 // recomputed panel by panel.  `resident`: the forward's only panel is still in c.Hpan.
 int mlp_tp_bwd(const MlpCtx& c, bool resident, Bump& ws) {
   const long long Bq = c.Bq, Bk = c.Bk, H2 = c.H2;
@@ -520,8 +600,9 @@ int mlp_tp_bwd(const MlpCtx& c, bool resident, Bump& ws) {
   const long long R = mlp_panel_rows(Bq, Bk);
   if (!dry) {
     const int dv_like = (c.estimator == MI_EST_DV || c.estimator == MI_EST_INFONCE_REF) ? 1 : 0;
+    const float* col_lse = c.estimator == MI_EST_INFONCE_SYM ? c.col_lse : nullptr;
     mlp_g_kernel<<<blocks_for(Bq * Bk, 256), 256, 0, stream>>>(c.S, c.sid_q, c.sid_k, Bq, Bk, c.q_off, c.Bg, dv_like, c.lse_f,
-                                                               reinterpret_cast<const float4*>(c.rows_r), c.G, t_run_if);
+                                                               reinterpret_cast<const float4*>(c.rows_r), col_lse, c.G, t_run_if);
     MI_LAUNCH_CHECK("mlp_g_kernel");
     MI_TRY(mlp_zero_accumulators(c, Bk));
   }
@@ -549,7 +630,10 @@ int mlp_tp_bwd(const MlpCtx& c, bool resident, Bump& ws) {
 int mlp_two_pass(const MlpCtx& c, bool plan, Bump& ws) {
   MI_TRY(mlp_tp_fwd(c, ws.dry));
   if (!ws.dry) {
-    loss_finalize_kernel<<<1, 32, 0, c.stream>>>(c.scal, nullptr, c.Bg, c.estimator, c.loss_out, c.lse_f, nullptr, t_run_if);
+    const bool sym = c.estimator == MI_EST_INFONCE_SYM;
+    if (sym) MI_TRY(mlp_col_stats(c, c.col_lse, true));
+    loss_finalize_kernel<<<1, 32, 0, c.stream>>>(c.scal, sym ? c.scal_col : nullptr, c.Bg, c.estimator, c.loss_out, c.lse_f, nullptr,
+                                                 t_run_if);
     MI_LAUNCH_CHECK("loss_finalize_kernel");
   }
   if (!plan) return MI_OK;
@@ -714,7 +798,7 @@ void mlp_ctx_dims(MlpCtx& c, long long D, long long H1, long long H2, int precis
 bool mlp_dims_ok(const MlpDims& d, int estimator) {
   if (d.B <= 0 || d.D <= 0 || d.H1 <= 0 || d.H2 <= 0 || (d.D % 8) != 0 || (d.H1 % 8) != 0 || (d.H2 % 8) != 0) return false;
   if (d.H2 > mi::EpiMlpDz::kMaxTiles * mi::TILE_N) return false;
-  return estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF || estimator == MI_EST_INFONCE_ROW;
+  return estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF || estimator == MI_EST_INFONCE_ROW || estimator == MI_EST_INFONCE_SYM;
 }
 // fp32 [R, C] (pitch ld_in) -> the bf16 operand (hi, + lo in strict mode) of pitch `pitch`, lo half at column Cp
 int mlp_split(const MlpCtx& c, const float* in, long long ld_in, __nv_bfloat16* out, long long pitch, long long Cp, long long R, long long C) {
@@ -753,6 +837,12 @@ int mlp_setup(MlpCtx& c, MlpSpBuf& sb, const float* X, const float* Y, const Mlp
   c.S = S_out ? S_out : keep.take<float>(Bq * Bk);
   c.rows_r = keep.take<float>(Bq * 4);
   c.scal = ws.take<double>(8);
+  // symmetric InfoNCE: planned by every size query (it does not know the estimator), carved only for this estimator
+  const bool cols = ws.dry || estimator == MI_EST_INFONCE_SYM;
+  c.col_part = cols ? ws.take<float>(3LL * kMlpColSplits * Bk) : nullptr;
+  c.col_lse = cols ? ws.take<float>(Bk) : nullptr;
+  c.cols_r = cols ? ws.take<float>(Bk * 4) : nullptr;
+  c.scal_col = cols ? ws.take<double>(8) : nullptr;
   c.lse_f = ws.take<float>(1);
   c.db3v = ws.take<float>(1);
   c.Hpan = ws.take<bf>(Pmax * pH);
@@ -913,8 +1003,10 @@ struct MlpBlockIO {
   const float* ref;         // stage fwd (single pass): [1] the reference of every block (maximum over the blocks)
   int two_pass;
   double* scal_out;         // stage fwd: [8] the block's scalar row (mi_score_stats layout, slot 7 = its sum of g~)
+  float* col_lse_out;       // stage fwd, symmetric InfoNCE: [Bk] log-sum-exp of every column over the block's rows
   const double* loss;       // stage bwd: [8] loss_out of the batch (mi_mlp_block_merge)
   const double* merged;     // stage bwd: [8] merged scalar row (slot 7 = the batch's sum of g~)
+  const float* col_lse;     // stage bwd, symmetric InfoNCE: [Bk] log-sum-exp of every column over the batch
   float* dC_part;           // stage bwd: [Bk, H1] the block's contribution to dL/dC
   MlpGrads gr;              // stage bwd: dX (the block's rows), dW1 (image half), db1, dW2, db2, dW3, db3 of the block
 };
@@ -922,10 +1014,13 @@ int mlp_block_impl(int stage, const float* X, const float* Y, const MlpParams& p
                    int estimator, int precision, const MlpBlockIO& io, Bump& ws, Bump& keep, cudaStream_t stream) {
   if (!mlp_dims_ok(d, estimator)) return MI_ERR_BAD_ARG;
   const long long H1 = d.H1, H2 = d.H2;
+  const bool sym = estimator == MI_EST_INFONCE_SYM;       // the two-pass sequence only: columns need every row first
   bool args_ok = true;
   if (stage == kMlpStageRef) args_ok = io.ref_out != nullptr;
-  else if (stage == kMlpStageFwd) args_ok = blk.sid_q && blk.sid_k && io.scal_out && (io.two_pass || io.ref);
-  else if (stage == kMlpStageBwd) args_ok = blk.sid_q && blk.sid_k && io.loss && io.dC_part && (io.two_pass || io.merged);
+  else if (stage == kMlpStageFwd)
+    args_ok = blk.sid_q && blk.sid_k && io.scal_out && (io.two_pass || io.ref) && (!sym || (io.two_pass && io.col_lse_out));
+  else if (stage == kMlpStageBwd)
+    args_ok = blk.sid_q && blk.sid_k && io.loss && io.dC_part && (io.two_pass || io.merged) && (!sym || (io.two_pass && io.col_lse));
   else return MI_ERR_BAD_ARG;
   MlpCtx c;
   MlpSpBuf sb{};
@@ -938,7 +1033,11 @@ int mlp_block_impl(int stage, const float* X, const float* Y, const MlpParams& p
   }
   if (stage == kMlpStageFwd) {
     if (!dry) c.scal = io.scal_out;
-    if (io.two_pass) return mlp_tp_fwd(c, dry);
+    if (io.two_pass) {
+      MI_TRY(mlp_tp_fwd(c, dry));
+      if (!dry && sym) MI_TRY(mlp_col_stats(c, io.col_lse_out, false));
+      return MI_OK;
+    }
     sb.ref = const_cast<float*>(io.ref);
     MI_TRY(mlp_sp_panels(c, sb, nullptr, ws));
     if (!dry) {
@@ -949,6 +1048,7 @@ int mlp_block_impl(int stage, const float* X, const float* Y, const MlpParams& p
   }
   if (io.two_pass) {
     if (!dry) {
+      c.col_lse = const_cast<float*>(io.col_lse);
       lse_from_loss_kernel<<<1, 1, 0, stream>>>(io.loss, c.lse_f);
       MI_LAUNCH_CHECK("lse_from_loss_kernel");
     }

@@ -427,6 +427,9 @@ def sharded_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor, W:
 #      rank's contribution dC_part [Bg, H1] to dL/dC of every text row
 #   5. reduce-scatter of dC_part -> dC_r; dY_r and the text half of dW1 (mi_mlp_input_grad); ONE all-reduce of the flat
 #      parameter gradients
+#   infonce_sym (two-pass only): step 2 also gives the block's column partials [Bg] (log-sum-exp of every column over the
+#   rank's rows); ONE all-gather of them, merged in fp64 on every rank, completes the column loss after step 3 and is the
+#   column normaliser of the backward in step 4
 
 MLP_GRAD_NAMES = ("dW1", "db1", "dW2", "db2", "dW3", "db3")
 
@@ -442,17 +445,18 @@ def sharded_mlp_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor
     dv / infonce with gradients take the single pass (unless mi_set_mlp_mode cleared bit 0); its guard is read on the host
     after the scalar exchange and, if it tripped on the global weight sum, every rank repeats the step with the two-pass
     sequence and reports guard = 1.  ``check_guard=False`` skips that host read; the verdict is then left in
-    stats['guard'] for the caller to act on.  infonce_row, forward-only calls and ``two_pass=True`` use the two-pass
-    sequence."""
+    stats['guard'] for the caller to act on.  infonce_row, infonce_sym (stats also hold 'loss_col'), forward-only calls
+    and ``two_pass=True`` use the two-pass sequence."""
     if backend is None:
         from . import ops as backend  # the CUDA path; raises if the library / device is missing
-    if estimator not in ("dv", "infonce", "infonce_ref", "infonce_row"):
-        raise ValueError(f"the MLP critic supports the dv, infonce and infonce_row estimators, not {estimator!r}")
+    if estimator not in ("dv", "infonce", "infonce_ref", "infonce_row", "infonce_sym"):
+        raise ValueError(f"the MLP critic supports the dv, infonce, infonce_row and infonce_sym estimators, not {estimator!r}")
     world, rank = _world(group)
     Bl, D = X_local.shape
     Bg = Bl * world
     off = rank * Bl
-    dv_like = estimator != "infonce_row"
+    sym = estimator == "infonce_sym"
+    dv_like = estimator not in ("infonce_row", "infonce_sym")
     single = need_grads and dv_like and not two_pass and (backend.get_mlp_mode() & 1) != 0
     nccl = world > 1 and dist.get_backend(group) != "gloo"
     X, Y = X_local.detach(), Y_local.detach()
@@ -477,9 +481,19 @@ def sharded_mlp_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor
     Y_all = _all_gather_rows(Y.contiguous(), world, group)
 
     # ---- the block pass and the scalar exchange
-    scal, state = backend.mlp_block_fwd(X, Y_all, params, sid_loc, sid_all, off, estimator, precision, ref, not single)
+    fw = backend.mlp_block_fwd(X, Y_all, params, sid_loc, sid_all, off, estimator, precision, ref, not single)
+    scal, state = fw[0], fw[1]
     scal_all = _all_gather_rows(scal.reshape(1, 8), world, group)
     loss, merged = backend.mlp_block_merge(scal_all, Bg, estimator, not single)
+    col_lse = None
+    if sym:
+        # column j over the batch = log-sum-exp of the ranks' partials (each holds the positive pair in exactly one block);
+        # the merge leaves slots 0 / 5 of loss_out to this side
+        c = torch.logsumexp(_all_gather_rows(fw[2].reshape(1, Bg), world, group).double(), 0)
+        loss = loss.clone()
+        loss[5] = (c.sum() - Bg * loss[1]) / Bg
+        loss[0] = 0.5 * (loss[4] + loss[5])
+        col_lse = c
     if single and check_guard and float(loss[7]) != 0.0:
         # every rank sees the same merged rows: all of them repeat the step with exact statistics
         out, dX, dY, grads = sharded_mlp_critic_loss_fwd_bwd(X_local, Y_local, params, sid_local, estimator, precision,
@@ -488,11 +502,15 @@ def sharded_mlp_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor
         return out, dX, dY, grads
     out = {"loss": loss[0], "pos_mean": loss[1], "lse_neg": loss[2], "n_neg": loss[3], "loss_row": loss[4],
            "rows_without_negatives": loss[6], "guard": loss[7]}
+    if sym:
+        out["loss_col"] = loss[5]
     if not need_grads:
         return out, None, None, None
 
     # ---- backward of the block, exchange of the dC contributions, layer 1 of the own text rows
-    g = backend.mlp_block_bwd(X, Y_all, params, sid_loc, sid_all, off, estimator, precision, not single, loss, merged, state)
+    extra = {"col_lse": col_lse} if sym else {}          # a backend without the symmetric estimator needs no such argument
+    g = backend.mlp_block_bwd(X, Y_all, params, sid_loc, sid_all, off, estimator, precision, not single, loss, merged, state,
+                              **extra)
     ev = None
     if nccl:
         ev = torch.cuda.Event()

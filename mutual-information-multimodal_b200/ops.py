@@ -549,7 +549,8 @@ def mlp_critic_loss_fwd_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid: torch
                             precision: str = "fast", need_grads: bool = True, want_scores: bool = False):
     """The reference's own critic make_mlp(2D, [H1, H2]) (model.py:18-32) on every pair + estimator, fwd+bwd
     (mi_mlp_critic_loss_fwd_bwd).  ``params`` = (W1 [H1,2D], b1, W2 [H2,H1], b2, W3 [1,H2], b3) fp32.
-    Returns (loss_out fp64[8], S or None, grads dict with keys dX, dY, dW1 ... db3 (or None))."""
+    Returns (loss_out fp64[8], S or None, grads dict with keys dX, dY, dW1 ... db3 (or None)); loss_out[4] / [5] are the
+    row / column losses of infonce_sym."""
     _need_cuda(X, Y, sid, *params)
     lib = _lib.load()
     f32 = lambda t: t.detach().to(torch.float32).contiguous()
@@ -559,10 +560,8 @@ def mlp_critic_loss_fwd_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid: torch
     H1, H2 = W1.shape[0], W2.shape[0]
     if W1.shape != (H1, 2 * D) or W2.shape != (H2, H1) or W3.numel() != H2 or b1.numel() != H1 or b2.numel() != H2 or b3.numel() != 1:
         raise MIError("MLP critic parameters do not have the make_mlp(2D, [H1, H2]) shapes")
-    if estimator not in ("dv", "infonce", "infonce_ref", "infonce_row"):
-        raise MIError("the MLP critic supports the dv, infonce and infonce_row estimators")
+    est, prec = _mlp_estimator(estimator), PRECISION[precision]
     sid = sid.to(torch.int32).contiguous()
-    est, prec = ESTIMATOR[estimator], PRECISION[precision]
     dev = X.device
     loss = torch.empty(8, dtype=torch.float64, device=dev)
     S = torch.empty((B, B), dtype=torch.float32, device=dev) if want_scores else None
@@ -617,8 +616,8 @@ def _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev):
 
 
 def _mlp_estimator(estimator):
-    if estimator not in ("dv", "infonce", "infonce_ref", "infonce_row"):
-        raise MIError("the MLP critic supports the dv, infonce and infonce_row estimators")
+    if estimator not in ESTIMATOR:
+        raise MIError(f"unknown estimator {estimator!r}: the MLP critic supports {', '.join(ESTIMATOR)}")
     return ESTIMATOR[estimator]
 
 
@@ -636,8 +635,10 @@ def mlp_block_ref_logit(X: torch.Tensor, Y: torch.Tensor, params, q_offset: int,
 
 def mlp_block_fwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor, sid_k: torch.Tensor, q_offset: int,
                   estimator: str, precision: str, ref: Optional[torch.Tensor], two_pass: bool):
-    """The block's pass over its Bq x Bk pairs (mi_mlp_block_fwd) -> (scalar row fp64 [8], state).  ``state`` is an
-    opaque device buffer that carries the block to ``mlp_block_bwd``."""
+    """The block's pass over its Bq x Bk pairs (mi_mlp_block_fwd_rc) -> (scalar row fp64 [8], state), and for infonce_sym
+    (``two_pass`` only) a third item: the block's column partials fp32 [Bk], the log-sum-exp of every column over the
+    block's negatives and its positive pair.  ``state`` is an opaque device buffer that carries the block to
+    ``mlp_block_bwd``."""
     X, Y, prm, D, H1, H2 = _mlp_operands(X, Y, params)
     _need_cuda(sid_q, sid_k, ref)
     Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), PRECISION[precision]
@@ -647,10 +648,12 @@ def mlp_block_fwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor,
     ws = _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev)
     state = torch.empty(lib.mi_mlp_block_state_bytes(Bq, Bk, D, H1, H2, prec), dtype=torch.uint8, device=dev)
     scal = torch.empty(8, dtype=torch.float64, device=dev)
-    _check(lib.mi_mlp_block_fwd(*(_ptr(t) for t in (X, Y) + prm), _ptr(sid_q), _ptr(sid_k), Bq, Bk, q_offset, D, H1, H2, est, prec,
-                                _ptr(ref), int(two_pass), _ptr(scal), _ptr(state), state.numel(), _ptr(ws), ws.numel(), _stream()),
-           "mi_mlp_block_fwd")
-    return scal, state
+    sym = estimator == "infonce_sym"
+    col = torch.empty(Bk, dtype=torch.float32, device=dev) if sym else None
+    _check(lib.mi_mlp_block_fwd_rc(*(_ptr(t) for t in (X, Y) + prm), _ptr(sid_q), _ptr(sid_k), Bq, Bk, q_offset, D, H1, H2, est,
+                                   prec, _ptr(ref), int(two_pass), _ptr(scal), _ptr(col), _ptr(state), state.numel(), _ptr(ws),
+                                   ws.numel(), _stream()), "mi_mlp_block_fwd_rc")
+    return (scal, state, col) if sym else (scal, state)
 
 
 def mlp_block_merge(scal_all: torch.Tensor, b_global: int, estimator: str, two_pass: bool):
@@ -665,12 +668,16 @@ def mlp_block_merge(scal_all: torch.Tensor, b_global: int, estimator: str, two_p
 
 
 def mlp_block_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor, sid_k: torch.Tensor, q_offset: int,
-                  estimator: str, precision: str, two_pass: bool, loss: torch.Tensor, merged: torch.Tensor, state: torch.Tensor) -> dict:
-    """The block's backward once the loss of the batch is known (mi_mlp_block_bwd).  Returns dX of the block's rows,
-    dC_part [Bk, H1] (the block's contribution to dL/dC of every text row), dW1 (image half filled), db1, dW2, db2, dW3, db3
-    (the block's shares)."""
+                  estimator: str, precision: str, two_pass: bool, loss: torch.Tensor, merged: torch.Tensor, state: torch.Tensor,
+                  col_lse: Optional[torch.Tensor] = None) -> dict:
+    """The block's backward once the loss of the batch is known (mi_mlp_block_bwd_rc; ``col_lse`` fp32 [Bk]: for
+    infonce_sym, the log-sum-exp of every column over the whole batch).  Returns dX of the block's rows, dC_part [Bk, H1]
+    (the block's contribution to dL/dC of every text row), dW1 (image half filled), db1, dW2, db2, dW3, db3 (the block's
+    shares)."""
     X, Y, prm, D, H1, H2 = _mlp_operands(X, Y, params)
-    _need_cuda(sid_q, sid_k, loss, merged, state)
+    _need_cuda(sid_q, sid_k, loss, merged, state, col_lse)
+    if col_lse is not None:
+        col_lse = col_lse.detach().to(torch.float32).contiguous()
     Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), PRECISION[precision]
     dev = X.device
     sid_q, sid_k = sid_q.to(torch.int32).contiguous(), sid_k.to(torch.int32).contiguous()
@@ -678,9 +685,10 @@ def mlp_block_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor,
               "dW3": (1, H2), "db3": (1,)}
     g = {k: torch.empty(v, dtype=torch.float32, device=dev) for k, v in shapes.items()}
     ws = _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev)
-    _check(_lib.load().mi_mlp_block_bwd(*(_ptr(t) for t in (X, Y) + prm), _ptr(sid_q), _ptr(sid_k), Bq, Bk, q_offset, D, H1, H2,
-                                        est, prec, int(two_pass), _ptr(loss), _ptr(merged), _ptr(state), state.numel(),
-                                        *(_ptr(g[k]) for k in shapes), _ptr(ws), ws.numel(), _stream()), "mi_mlp_block_bwd")
+    _check(_lib.load().mi_mlp_block_bwd_rc(*(_ptr(t) for t in (X, Y) + prm), _ptr(sid_q), _ptr(sid_k), Bq, Bk, q_offset, D, H1,
+                                           H2, est, prec, int(two_pass), _ptr(loss), _ptr(merged), _ptr(col_lse), _ptr(state),
+                                           state.numel(), *(_ptr(g[k]) for k in shapes), _ptr(ws), ws.numel(), _stream()),
+           "mi_mlp_block_bwd_rc")
     return g
 
 

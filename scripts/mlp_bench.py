@@ -1,6 +1,8 @@
 """Fused concat-MLP critic (make_mlp(1536, [1024, 512]), SURVEY 8f-1): ms per fwd+bwd step and tensor throughput,
 next to the reference sequence (explicit pair tensor -> nn.Sequential fp32 -> estimator -> backward) on the same GPU.
-python scripts/mlp_bench.py [--torch-max-b 256] > profiles/..."""
+python scripts/mlp_bench.py [--torch-max-b 256] [--estimators dv,infonce_row,infonce_sym] > profiles/...
+Rows of an estimator other than dv name it in the path column; infonce_row / infonce_sym take the two-pass sequence in
+every mode."""
 import argparse
 import os
 import sys
@@ -16,6 +18,7 @@ ap.add_argument("--sizes", default="64,256,1024,4096")
 ap.add_argument("--torch-max-b", type=int, default=256)
 ap.add_argument("--steps", type=int, default=5)
 ap.add_argument("--modes", default="3,1,0", help="mi_set_mlp_mode values to time (3 = default)")
+ap.add_argument("--estimators", default="dv", help="estimators to time (dv, infonce, infonce_row, infonce_sym)")
 a = ap.parse_args()
 dev = torch.device("cuda:0")
 D, H1, H2 = 768, 1024, 512
@@ -48,19 +51,21 @@ for B in [int(v) for v in a.sizes.split(",")]:
     for mode in [int(v) for v in a.modes.split(",")]:
         ops.set_mlp_mode(mode)
         for prec in ("fast", "strict"):
-            ms = timed(lambda: ops.mlp_critic_loss_fwd_bwd(X, Y, params, sid, "dv", prec, True, False), a.steps)
-            # per-kind engine time of one more step (CUDA events around every tile-engine launch)
-            import ctypes
-            lib = _lib.load()
-            lib.mi_set_profiling(1)
-            ops.mlp_critic_loss_fwd_bwd(X, Y, params, sid, "dv", prec, True, False)
-            torch.cuda.synchronize()
-            kms = (ctypes.c_double * 6)(); kn = (ctypes.c_int64 * 6)()
-            lib.mi_profile_read_kinds(kms, kn, 6)
-            lib.mi_set_profiling(0)
-            kinds = "gemm %.2f (%d) | single pass %.2f (%d) | fused dZ1 %.2f (%d) | two-pass epilogues %.2f (%d)" % (
-                kms[2], kn[2], kms[3], kn[3], kms[4], kn[4], kms[5], kn[5])
-            print(f"| {B} | {B*B} | fused {prec}, mode {mode} | {ms:.3f} | {f_alg / ms / 1e9:.1f} | {B * B / ms * 1e3:.3e} | {kinds} |", flush=True)
+            for est in a.estimators.split(","):
+                ms = timed(lambda: ops.mlp_critic_loss_fwd_bwd(X, Y, params, sid, est, prec, True, False), a.steps)
+                # per-kind engine time of one more step (CUDA events around every tile-engine launch)
+                import ctypes
+                lib = _lib.load()
+                lib.mi_set_profiling(1)
+                ops.mlp_critic_loss_fwd_bwd(X, Y, params, sid, est, prec, True, False)
+                torch.cuda.synchronize()
+                kms = (ctypes.c_double * 6)(); kn = (ctypes.c_int64 * 6)()
+                lib.mi_profile_read_kinds(kms, kn, 6)
+                lib.mi_set_profiling(0)
+                kinds = "gemm %.2f (%d) | single pass %.2f (%d) | fused dZ1 %.2f (%d) | two-pass epilogues %.2f (%d)" % (
+                    kms[2], kn[2], kms[3], kn[3], kms[4], kn[4], kms[5], kn[5])
+                path = f"fused {prec}, mode {mode}" + ("" if est == "dv" else f", {est}")
+                print(f"| {B} | {B*B} | {path} | {ms:.3f} | {f_alg / ms / 1e9:.1f} | {B * B / ms * 1e3:.3e} | {kinds} |", flush=True)
     ops.set_mlp_mode(-1)
     if B <= a.torch_max_b:
         study = [str(i) for i in range(B)]

@@ -2,7 +2,7 @@
 mi_b200.dist.sharded_mlp_critic_loss_fwd_bwd at a global batch B_global split over the ranks, next to the single-GPU
 mi_mlp_critic_loss_fwd_bwd at the same B_global timed in the same job.
 
-    torchrun --nproc-per-node N scripts/mlp_sharded_bench.py [--sizes 4096,8192] [--steps 10] > profiles/...
+    torchrun --nproc-per-node N scripts/mlp_sharded_bench.py [--sizes 4096,8192] [--steps 10] [--estimator dv] > profiles/...
     python scripts/mlp_sharded_bench.py                      # N = 1 without a process group
 
 Timing: CUDA events around `--steps` steps after `--warmup` steps, the maximum over ranks.  F_alg = 6 B^2 H1 H2 +
@@ -29,6 +29,7 @@ ap.add_argument("--per-gpu", default="256", help="per-GPU batch sizes (B_global 
 ap.add_argument("--steps", type=int, default=10)
 ap.add_argument("--warmup", type=int, default=3)
 ap.add_argument("--precisions", default="fast,strict")
+ap.add_argument("--estimator", default="dv", help="dv, infonce, infonce_row or infonce_sym")
 a = ap.parse_args()
 
 world, rank = 1, 0
@@ -76,7 +77,7 @@ if rank == 0:
                               capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
     except Exception as e:  # noqa: BLE001
         card = f"{torch.cuda.get_device_name()} (nvidia-smi unavailable: {e})"
-    print(f"card: {card}; ranks: {world}; steps {a.steps} after {a.warmup} warm-up; max over ranks")
+    print(f"card: {card}; ranks: {world}; estimator {a.estimator}; steps {a.steps} after {a.warmup} warm-up; max over ranks")
     print("| B_global | N | precision | path | ms / step | pairs/s | F_alg TFLOP/s | efficiency | engine ms by kind, rank 0 |")
     print("|---|---|---|---|---|---|---|---|---|")
 sizes = [int(v) for v in a.sizes.split(",") if v] + [world * int(v) for v in a.per_gpu.split(",") if v]
@@ -94,8 +95,8 @@ for Bg in sizes:
     Xl, Yl, sl_id = X[sl].contiguous(), Y[sl].contiguous(), sid[sl].contiguous()
     label = " (launch-bound)" if Bl <= 256 else ""
     for prec in a.precisions.split(","):
-        single = lambda: ops.mlp_critic_loss_fwd_bwd(X, Y, params, sid, "dv", prec, True, False)       # noqa: E731
-        sharded = lambda: mdist.sharded_mlp_critic_loss_fwd_bwd(Xl, Yl, params, sl_id, "dv", prec)     # noqa: E731
+        single = lambda: ops.mlp_critic_loss_fwd_bwd(X, Y, params, sid, a.estimator, prec, True, False)       # noqa: E731
+        sharded = lambda: mdist.sharded_mlp_critic_loss_fwd_bwd(Xl, Yl, params, sl_id, a.estimator, prec)     # noqa: E731
         t1 = timed(single)
         tn = timed(sharded)
         kn = kinds(sharded)
