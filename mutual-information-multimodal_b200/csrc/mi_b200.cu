@@ -351,14 +351,18 @@ __global__ void make_refk2_kernel(const float* __restrict__ refk, float ln_wk, f
   if (i < n_pad) dst[i] = (i < n) ? (refk[i] - ln_wk) * mi::kLog2e : 0.f;
 }
 
+// 4 elements / thread.  The float4 load and uint2 store need 16- / 8-byte aligned pointers; a contiguous view at an element
+// offset (x[1:], a slice of a flat parameter buffer) is not, and takes the scalar path for all of its elements.
 __global__ void cast_f32_bf16_kernel(const float* __restrict__ in, __nv_bfloat16* __restrict__ out, long long n) {
   long long i = (blockIdx.x * (long long)blockDim.x + threadIdx.x) * 4;
-  if (i + 3 < n) {
+  const bool vec = ((reinterpret_cast<unsigned long long>(in) & 15ull) | (reinterpret_cast<unsigned long long>(out) & 7ull)) == 0;
+  if (vec && i + 3 < n) {
     const float4 v = *reinterpret_cast<const float4*>(in + i);
     uint2 o; o.x = ptx::pack_bf16(v.x, v.y); o.y = ptx::pack_bf16(v.z, v.w);
     *reinterpret_cast<uint2*>(out + i) = o;
   } else {
-    for (; i < n; ++i) out[i] = __float2bfloat16(in[i]);
+    const long long end = i + 4 < n ? i + 4 : n;
+    for (; i < end; ++i) out[i] = __float2bfloat16(in[i]);
   }
 }
 
