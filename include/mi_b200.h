@@ -114,6 +114,19 @@ int mi_score_stats_rc(const void* Q, int64_t ldq, int q_split, const void* K, in
                       const int32_t* sid_q, const int32_t* sid_k, int64_t q_offset,
                       int64_t Bq, int64_t Bk, int64_t D, float scale, float* row_out, double* scal_out, float* col_lse_out,
                       void* workspace, size_t workspace_bytes, mi_stream_t stream);
+/* mi_score_stats_rc with the schedule and output of the batch-sharded symmetric step (mi_score_stats_rc is this call with
+ * NULL, 0, 0; same workspace size):
+ *   event_k_ready / k_local_valid as in mi_score_single_pass: with k_local_valid = 1, q_offset and Bq multiples of 256 and
+ *     Bq < Bk, the tiles of the own column block [q_offset, q_offset + Bq) are scored before the wait for the event;
+ *     otherwise the call waits before the first tile.
+ *   include_pos = 1: the block's positive pairs are folded into its own columns, col_lse_out[q_offset + r] =
+ *     logaddexp(col_lse_out[q_offset + r], S[r, q_offset + r]).  Column j of the batch is then the plain log-sum-exp of the
+ *     ranks' col_lse_out[j] (mi_merge_sym_stats). */
+int mi_score_stats_rc_ex(const void* Q, int64_t ldq, int q_split, const void* K, int64_t ldk, int k_split,
+                         const int32_t* sid_q, const int32_t* sid_k, int64_t q_offset,
+                         int64_t Bq, int64_t Bk, int64_t D, float scale, float* row_out, double* scal_out, float* col_lse_out,
+                         void* event_k_ready, int k_local_valid, int include_pos,
+                         void* workspace, size_t workspace_bytes, mi_stream_t stream);
 
 /* Fused gradient pass (replaces loss.backward() through mi_critics.py and the pair tensor,
  * main_utils.py:226): recomputes score tiles, forms
@@ -190,6 +203,15 @@ int mi_score_single_pass(const void* Q, int64_t ldq, int q_split, const void* K,
  * Two tiny kernels instead of a chain of framework ops.  scratch8: 8 doubles of device scratch. */
 int mi_merge_scalars(const double* scal_all, int world, int64_t B_global, int estimator, const float* lambda,
                      double* loss_out, float* lse_out, double* scratch8, mi_stream_t stream);
+/* The symmetric estimator's merge (the one the batch-sharded step runs, fp64): the ranks' scalar rows scal_all [world][8]
+ * (mi_score_stats_rc_ex) and column partials col_all [world][col_pitch] (include_pos = 1, first B_global floats of each row
+ * used) -> c_out [B_global] fp32 = the fp64 log-sum-exp of column j over the ranks, rounded once (the column references of
+ * the gradient pass), and loss_out (fp64[8]) in the layout of the single-GPU symmetric call: slot 0 = (row + col) / 2,
+ * 4 = loss_row, 5 = loss_col = (sum_j c_j - sum_i S_ii) / B_global, 7 = 0.  Sums run in a fixed order (no atomics): the
+ * same inputs give the same bits.  scratch: mi_merge_sym_stats_scratch_doubles(B_global) doubles of device scratch. */
+int64_t mi_merge_sym_stats_scratch_doubles(int64_t B_global);
+int mi_merge_sym_stats(const double* scal_all, const float* col_all, int64_t col_pitch, int world, int64_t B_global,
+                       double* loss_out, float* c_out, double* scratch, mi_stream_t stream);
 int mi_single_finalize_q(const float* oq_raw, int64_t rows, int64_t D, const float* ref, const float* wrow, const float* lse,
                          int dv_like, float alpha, float gamma, const void* kdiag, int64_t ldk, int k_split,
                          float* out_f32, void* out_bf16, int64_t ld16, int out_split, mi_stream_t stream);
@@ -239,8 +261,8 @@ int mi_critic_loss_fwd_bwd_from_host(const void* X_host, const void* Y_host, con
 
 /* One host call per step and rank: rank r passes its row shard (X_local, Y_local [B_local, D] bf16, sid_local int32; all ranks
  * the same B_local) and receives the GLOBAL-batch loss (loss_out fp64[8], device, identical on every rank) and the gradients
- * of its rows (dX, dY fp32 [B_local, D]) plus dW (fp32 [D, D], already summed over ranks).  Estimators DV / INFONCE_REF /
- * INFONCE_ROW (the symmetric one is orchestrated on the host side, mi_b200/dist.py).  Inside: all-gather of the ids and of Y
+ * of its rows (dX, dY fp32 [B_local, D]) plus dW (fp32 [D, D], already summed over ranks).  Every estimator; for DV /
+ * INFONCE_REF / INFONCE_ROW inside: all-gather of the ids and of Y
  * (in place, the own column block is scored while the others arrive), references from a sample of the OWN column block and
  * an all-reduce(max) of lambda, the single pass, all-gather of the 8 loss scalars, reduce-scatter of the dY contributions
  * under the dT contraction, all-reduce of dW under the dX GEMM — NCCL called directly on `nccl_comm` (an ncclComm_t, e.g.
@@ -248,7 +270,12 @@ int mi_critic_loss_fwd_bwd_from_host(const void* X_host, const void* Y_host, con
  * resolved from the running process.  check_guard = 1: the host waits (an event, not a stream) until the merged guard count
  * is known — right after the score tiles — and returns MI_GUARD_TRIPPED on every rank when it is non-zero; 0: never
  * synchronises, the count is left in loss_out[7].  A context is bound to one device / communicator and serves one call at a
- * time; the collectives it issues must not interleave with other collectives on the same communicator from other threads. */
+ * time; the collectives it issues must not interleave with other collectives on the same communicator from other threads.
+ * MI_EST_INFONCE_SYM uses exact statistics (no guard: loss_out[7] = 0, never MI_GUARD_TRIPPED, check_guard ignored, no host
+ * read) with the loss_out layout of the single-GPU symmetric call: all-gather of the ids and of Y, the row + column
+ * statistics pass (own column block first, own positive pairs folded into the column partials), ONE all-gather of each
+ * rank's packed record {8 fp64 scalars | B fp32 column partials}, the fp64 merge (mi_merge_sym_stats) on every rank, the
+ * gradient pass with row and column references, then the same reduce-scatter / all-reduce as above. */
 typedef struct mi_dist_ctx mi_dist_ctx;
 int mi_dist_ctx_create(void* nccl_comm, mi_dist_ctx** out);
 void mi_dist_ctx_destroy(mi_dist_ctx* ctx);

@@ -39,6 +39,8 @@ PROTOTYPES = {
     "mi_score_stats_rc_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64]),
     "mi_score_stats_rc": (c_int, [c_vp, c_i64, c_int, c_vp, c_i64, c_int, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_f32,
                                   c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "mi_score_stats_rc_ex": (c_int, [c_vp, c_i64, c_int, c_vp, c_i64, c_int, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_f32,
+                                     c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_sz, c_vp]),
     "mi_score_stats": (c_int, [c_vp, c_i64, c_int, c_vp, c_i64, c_int, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_f32,
                                c_vp, c_vp, c_vp, c_sz, c_vp]),
     "mi_score_grad_workspace_bytes": (c_sz, [c_i64, c_i64, c_i64, c_int]),
@@ -55,6 +57,8 @@ PROTOTYPES = {
                                      c_int, c_int, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                      c_vp, c_int, c_vp, c_sz, c_vp]),
     "mi_merge_scalars": (c_int, [c_vp, c_int, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "mi_merge_sym_stats_scratch_doubles": (c_i64, [c_i64]),
+    "mi_merge_sym_stats": (c_int, [c_vp, c_vp, c_i64, c_int, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "mi_single_finalize_q": (c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_int, c_f32, c_f32, c_vp, c_i64, c_int,
                                      c_vp, c_vp, c_i64, c_int, c_vp]),
     "mi_single_finalize_k": (c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_int, c_f32, c_f32, c_vp, c_i64, c_int, c_vp]),

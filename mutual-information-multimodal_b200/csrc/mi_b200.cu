@@ -795,13 +795,14 @@ __global__ void flag_to_scal_kernel(const int* __restrict__ flag, double* __rest
 
 // ranks' reduced scalars [world][8] -> one row of the same layout (global max / rescaled sum-exp, plain sums).
 // Slot 7 is summed too: the MLP critic's sharded single pass carries each block's sum of g~ there (0 everywhere else).
-__global__ void merge_scal_kernel(const double* __restrict__ scal_all, int world, double* __restrict__ out) {
+// `pitch` (doubles) between the ranks' rows: 8, or the record size of the symmetric step's packed exchange.
+__global__ void merge_scal_kernel(const double* __restrict__ scal_all, int world, double* __restrict__ out, long long pitch = 8) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   double gm = -INFINITY;
-  for (int r = 0; r < world; ++r) gm = fmax(gm, scal_all[r * 8]);
+  for (int r = 0; r < world; ++r) gm = fmax(gm, scal_all[r * pitch]);
   double s = 0, t[6] = {0, 0, 0, 0, 0, 0};
   for (int r = 0; r < world; ++r) {
-    const double* v = scal_all + r * 8;
+    const double* v = scal_all + r * pitch;
     if (isfinite(v[0])) s += v[1] * exp(v[0] - gm);
     for (int k = 0; k < 6; ++k) t[k] += v[2 + k];
   }
@@ -832,6 +833,72 @@ __global__ void loss_finalize_kernel(const double* __restrict__ scal_row, const 
   loss_out[0] = loss; loss_out[1] = pos; loss_out[2] = lse; loss_out[3] = n_neg;
   loss_out[4] = loss_row; loss_out[5] = loss_col; loss_out[6] = scal_row[5]; loss_out[7] = guard;
   if (lse_f) *lse_f = (float)lse;
+}
+
+// ---- symmetric InfoNCE over row blocks (the batch-sharded step): each rank's column partials carry its own positive
+//      pairs (col_pos_fold_kernel), so column j of the batch is the plain log-sum-exp of the ranks' partials and
+//      loss_col = (sum_j c_j - sum_i S_ii) / B, with sum_i S_ii = slot 3 of the merged scalar row.
+// col_lse[i] = logaddexp(col_lse[i], diag[i]), i < n (the caller offsets col_lse to the block's own columns)
+__global__ void col_pos_fold_kernel(float* __restrict__ col_lse, const float* __restrict__ diag, long long n) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float x = col_lse[i], d = diag[i];
+  const float hi = fmaxf(x, d), lo = fminf(x, d);
+  col_lse[i] = hi + log1pf(expf(lo - hi));
+}
+// c_out[j] = (fp32 of) the fp64 log-sum-exp of col_all[r * pitch + j] over the ranks; part[block] = sum of the block's fp64
+// c_j.  256 threads; the fixed tree order makes the sums independent of timing (every rank computes the same bits).
+constexpr int kSymColThreads = 256;
+__global__ void sym_col_kernel(const float* __restrict__ col_all, long long pitch, int world, long long B,
+                               float* __restrict__ c_out, double* __restrict__ part) {
+  __shared__ double sh[kSymColThreads];
+  const long long j = blockIdx.x * (long long)kSymColThreads + threadIdx.x;
+  double c = 0.0;
+  if (j < B) {
+    double m = -INFINITY;
+    for (int r = 0; r < world; ++r) m = fmax(m, (double)col_all[r * pitch + j]);
+    double s = 0.0;
+    for (int r = 0; r < world; ++r) {
+      const double x = col_all[r * pitch + j];
+      if (x > -INFINITY) s += exp(x - m);
+    }
+    c = m > -INFINITY ? m + log(s) : -INFINITY;
+    c_out[j] = (float)c;
+  }
+  sh[threadIdx.x] = c;
+  __syncthreads();
+  for (int o = kSymColThreads / 2; o; o >>= 1) {
+    if (threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) part[blockIdx.x] = sh[0];
+}
+// the column scalar row in the layout of the rows (loss_finalize_kernel reads slot 4): {0, 0, 0, sum S_ii, sum_j c_j - sum S_ii, 0, 0, 0}
+__global__ void sym_col_row_kernel(const double* __restrict__ part, int n_part, const double* __restrict__ row_merged,
+                                   double* __restrict__ col_row) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  double s = 0.0;
+  for (int b = 0; b < n_part; ++b) s += part[b];
+  for (int k = 0; k < 8; ++k) col_row[k] = 0.0;
+  col_row[3] = row_merged[3];
+  col_row[4] = s - row_merged[3];
+}
+inline long long merge_sym_scratch_doubles(long long B) { return 16 + cdiv(B, kSymColThreads); }
+// The ranks' scalar rows (pitch in doubles) and column partials with their own positive pairs folded in (pitch in floats)
+// -> c_out [B] (the column references of the gradient pass) and loss_out in the layout of the single-GPU symmetric call.
+int merge_sym_impl(const double* scal_all, long long scal_pitch, const float* col_all, long long col_pitch, int world, long long B,
+                   double* loss_out, float* c_out, double* scratch, cudaStream_t stream) {
+  const int nb = static_cast<int>(cdiv(B, kSymColThreads));
+  double* rows = scratch; double* cols = scratch + 8; double* part = scratch + 16;
+  sym_col_kernel<<<nb, kSymColThreads, 0, stream>>>(col_all, col_pitch, world, B, c_out, part);
+  MI_LAUNCH_CHECK("sym_col_kernel");
+  merge_scal_kernel<<<1, 32, 0, stream>>>(scal_all, world, rows, scal_pitch);
+  MI_LAUNCH_CHECK("merge_scal_kernel");
+  sym_col_row_kernel<<<1, 32, 0, stream>>>(part, nb, rows, cols);
+  MI_LAUNCH_CHECK("sym_col_row_kernel");
+  loss_finalize_kernel<<<1, 32, 0, stream>>>(rows, cols, B, MI_EST_INFONCE_SYM, loss_out, nullptr, nullptr, nullptr);
+  MI_LAUNCH_CHECK("loss_finalize_kernel");
+  return MI_OK;
 }
 // flag[0] = (loss_out[7] != 0): the device predicate of the exact fallback
 __global__ void guard_to_flag_kernel(const double* __restrict__ loss_out, int* __restrict__ flag, double* __restrict__ guard_a) {
@@ -1116,13 +1183,17 @@ int stats_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid_k,
 // Row AND column statistics of the score block S[q_offset + r, c] = scale <Q_r, K_c>, r < Bq, c < Bk, from ONE pass.
 // Square use (Bq == Bk, q_offset = 0; the 1-GPU symmetric estimator): col_out / scal_col receive the columns in the layout of
 // the rows.  Row-block use (a rank's rows of the batch-sharded step): col_lse receives, for every column, the log-sum-exp
-// over this block's negatives; the caller merges the ranks.
+// over this block's negatives; the caller merges the ranks.  include_pos (row-block use): col_lse also holds the block's
+// positive pairs, col_lse[q_offset + r] = logaddexp(col_lse[q_offset + r], S[r, q_offset + r]).
+// ev_k_ready / k_local_valid schedule the score tiles as single_pass_impl does: the own column block first, then the wait
+// for the other ranks' K rows.  shared_mask: the negatives mask of (sid_q, sid_k), built by the caller.
 int stats_rc_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid_k, long long q_offset, long long Bq, long long Bk,
                   long long D, float scale, float* row_out, double* scal_row, float* col_out, double* scal_col, float* col_lse,
-                  Bump& ws, cudaStream_t stream) {
+                  Bump& ws, cudaStream_t stream, cudaEvent_t ev_k_ready = nullptr, bool k_local_valid = false,
+                  const MaskBuf* shared_mask = nullptr, bool include_pos = false) {
   if (Bq <= 0 || Bk <= 0 || D <= 0 || (D % 8) != 0 || q_offset < 0 || q_offset + Bq > Bk) return MI_ERR_BAD_ARG;
   const bool square = col_lse == nullptr;
-  if (square && (Bq != Bk || q_offset != 0) && !ws.dry) return MI_ERR_BAD_ARG;
+  if (square && (Bq != Bk || q_offset != 0 || include_pos) && !ws.dry) return MI_ERR_BAD_ARG;
   Sched sc;
   sc.n_mblk = static_cast<int>(cdiv(Bq, rows_per_mblk()));
   sc.n_ntile = static_cast<int>(cdiv(Bk, mi::TILE_N));
@@ -1132,8 +1203,10 @@ int stats_rc_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid
   const long long k_pad = static_cast<long long>(sc.n_ntile) * mi::TILE_N;
   const int rows_padded = sc.n_mblk * rows_per_mblk();
   const int n_rb = rows_padded / 32;
-  const MaskBuf mb = take_mask(ws, Bq, k_pad, Bk);
-  float4* part = ws.take<float4>(static_cast<size_t>(sc.n_split) * mi::kColQuarters * rows_padded);
+  const int max_split = sc.n_split;
+  const MaskBuf mb = shared_mask != nullptr ? *shared_mask : take_mask(ws, Bq, k_pad, Bk);
+  // (x3: up to three launches append their row partials — own columns first, the rest once K has arrived)
+  float4* part = ws.take<float4>(3 * static_cast<size_t>(max_split) * mi::kColQuarters * rows_padded);
   float* diag = ws.take<float>(Bq);
   float* colpart = ws.take<float>(static_cast<size_t>(n_rb) * k_pad);
   const RedScratch red = take_red(ws);
@@ -1141,18 +1214,41 @@ int stats_rc_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid
   if (ws.dry) return MI_OK;
   if (!Q.p || !K.p || !sid_q || !sid_k || !row_out || !scal_row || !(scale > 0.f)) return MI_ERR_BAD_ARG;
   if (square && (!col_out || !scal_col)) return MI_ERR_BAD_ARG;
-  MI_TRY(build_mask(mb, sid_q, sid_k, Bq, Bk, k_pad, stream));
+  if (shared_mask == nullptr) MI_TRY(build_mask(mb, sid_q, sid_k, Bq, Bk, k_pad, stream));
+  const long long own_t0 = q_offset / mi::TILE_N, own_t1 = (q_offset + Bq) / mi::TILE_N;
+  const bool own_first = ev_k_ready != nullptr && k_local_valid && (q_offset % mi::TILE_N) == 0 && (Bq % mi::TILE_N) == 0 && Bq < Bk;
+  if (ev_k_ready != nullptr && !own_first) MI_CUDA(cudaStreamWaitEvent(stream, ev_k_ready, 0));
   diag_kernel<<<blocks_for(Bq * 32, 256), 256, 0, stream>>>(Q.p, Q.ld, Q.split, K.p, K.ld, K.split, q_offset, Bq, D,
                                                              round_up(D, kSplitAlign), scale, diag, t_run_if);
   MI_LAUNCH_CHECK("diag_kernel");
-  mi::EpiStatsRC::Params ep;
-  ep.mask = mi::MaskInfo{mb.excl, mb.n_same, sid_q, mb.sidk_pad};
-  ep.q_rows = static_cast<int>(Bq); ep.k_cols = static_cast<int>(Bk);
-  ep.scale = scale; ep.part = part; ep.rows_padded = rows_padded;
-  ep.colpart = colpart; ep.col_pitch = k_pad;
-  MI_TRY(launch_engine<mi::EpiStatsRC>(MapSpec{Q.p, Bq, opnd_k_extent(Q, D), Q.ld}, MapSpec{K.p, Bk, opnd_k_extent(K, D), K.ld},
-                                       sc, ep, stream));
-  stats_merge_kernel<<<blocks_for(Bq, 128), 128, 0, stream>>>(part, sc.n_split * mi::kColQuarters, rows_padded, static_cast<int>(Bq),
+  // a launch covers the N tiles [t0, t1): its row partials are appended, its column partials are its own columns
+  int n_part = 0;
+  auto score_tiles = [&](long long t0, long long t1) -> int {
+    if (t1 <= t0) return MI_OK;
+    Sched s = sc;
+    s.n_ntile = static_cast<int>(t1 - t0);
+    s.n_split = std::min(choose_split(s.n_mblk, s.n_ntile, num_pairs()), max_split);
+    MI_TRY(score_segments(s, Q, K, D));
+    s.nt_base = static_cast<int>(t0);
+    mi::EpiStatsRC::Params ep;
+    ep.mask = mi::MaskInfo{mb.excl, mb.n_same, sid_q, mb.sidk_pad};
+    ep.q_rows = static_cast<int>(Bq); ep.k_cols = static_cast<int>(Bk);
+    ep.scale = scale; ep.part = part + static_cast<size_t>(n_part) * rows_padded; ep.rows_padded = rows_padded;
+    ep.colpart = colpart; ep.col_pitch = k_pad;
+    MI_TRY(launch_engine<mi::EpiStatsRC>(MapSpec{Q.p, Bq, opnd_k_extent(Q, D), Q.ld}, MapSpec{K.p, Bk, opnd_k_extent(K, D), K.ld},
+                                         s, ep, stream));
+    n_part += s.n_split * mi::kColQuarters;
+    return MI_OK;
+  };
+  if (own_first) {
+    MI_TRY(score_tiles(own_t0, own_t1));                               // this rank's own columns: K rows already here
+    MI_CUDA(cudaStreamWaitEvent(stream, ev_k_ready, 0));               // the other ranks' text embeddings
+    MI_TRY(score_tiles(0, own_t0));
+    MI_TRY(score_tiles(own_t1, sc.n_ntile));
+  } else {
+    MI_TRY(score_tiles(0, sc.n_ntile));
+  }
+  stats_merge_kernel<<<blocks_for(Bq, 128), 128, 0, stream>>>(part, n_part, rows_padded, static_cast<int>(Bq),
                                                               mb.n_same, static_cast<int>(Bk), diag, reinterpret_cast<float4*>(row_out));
   MI_LAUNCH_CHECK("stats_merge_kernel");
   MI_TRY(reduce_rows(row_out, Bq, scal_row, red, stream));
@@ -1164,6 +1260,10 @@ int stats_rc_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid
   } else {
     col_lse_kernel<<<static_cast<unsigned>(cdiv(Bk, 32)), dim3(32, 8), 0, stream>>>(colpart, n_rb, k_pad, static_cast<int>(Bk), col_lse);
     MI_LAUNCH_CHECK("col_lse_kernel");
+    if (include_pos) {
+      col_pos_fold_kernel<<<blocks_for(Bq, 256), 256, 0, stream>>>(col_lse + q_offset, diag, Bq);
+      MI_LAUNCH_CHECK("col_pos_fold_kernel");
+    }
   }
   return MI_OK;
 }
@@ -1276,7 +1376,8 @@ int grad_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid_k,
               long long q_offset, long long Bq, long long Bk, long long D, float scale,
               const float* refq, float wq, const float* refk, float wk, int include_diag, int precision,
               float alpha, float gamma, const GradOut& oq, const GradOut* ok, Bump& ws, cudaStream_t stream,
-              cudaEvent_t ev_after_k = nullptr) {
+              cudaEvent_t ev_after_k = nullptr,
+              const MaskBuf* shared_mask = nullptr /* the negatives mask of (sid_q, sid_k), built by the caller */) {
   if (Bq <= 0 || Bk <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
   typedef __nv_bfloat16 bf;
   const bool strict = precision == MI_PREC_BF16_STRICT;
@@ -1288,7 +1389,7 @@ int grad_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid_k,
   const bool k_hl = strict && K.split == 2, q_hl = strict && Q.split == 2;
   const long long mb_panel = panel_mblks(Bq, Bk, D, precision);
   const long long panel_rows = mb_panel * rows_per_mblk();
-  const MaskBuf mb = take_mask(ws, Bq, k_pad, Bk);
+  const MaskBuf mb = shared_mask != nullptr ? *shared_mask : take_mask(ws, Bq, k_pad, Bk);
   float* refk2 = ws.take<float>(k_pad);
   bf* P = ws.take<bf>(static_cast<size_t>(panel_rows) * pitch);
   // strict: the Oq contraction runs as short split-K chains into a raw fp32 panel, finished by an elementwise pass
@@ -1302,7 +1403,7 @@ int grad_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid_k,
   const bool use_q = refq != nullptr && wq > 0.f, use_k = refk != nullptr && wk > 0.f;
   if ((!use_q && !use_k) || !(scale > 0.f)) return MI_ERR_BAD_ARG;
 
-  MI_TRY(build_mask(mb, sid_q, sid_k, Bq, Bk, k_pad, stream));
+  if (shared_mask == nullptr) MI_TRY(build_mask(mb, sid_q, sid_k, Bq, Bk, k_pad, stream));
   if (use_k) {
     make_refk2_kernel<<<blocks_for(k_pad, 256), 256, 0, stream>>>(refk, logf(wk), refk2, Bk, k_pad);
     MI_LAUNCH_CHECK("make_refk2_kernel");
@@ -1966,17 +2067,26 @@ size_t mi_score_stats_rc_workspace_bytes(int64_t Bq, int64_t Bk, int64_t D) {
                     &dummy, ws, nullptr) != MI_OK) return 0;
   return ws.peak + 256;
 }
-int mi_score_stats_rc(const void* Q, int64_t ldq, int q_split, const void* K, int64_t ldk, int k_split,
-                      const int32_t* sid_q, const int32_t* sid_k, int64_t q_offset,
-                      int64_t Bq, int64_t Bk, int64_t D, float scale, float* row_out, double* scal_out, float* col_lse_out,
-                      void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+int mi_score_stats_rc_ex(const void* Q, int64_t ldq, int q_split, const void* K, int64_t ldk, int k_split,
+                         const int32_t* sid_q, const int32_t* sid_k, int64_t q_offset,
+                         int64_t Bq, int64_t Bk, int64_t D, float scale, float* row_out, double* scal_out, float* col_lse_out,
+                         void* event_k_ready, int k_local_valid, int include_pos,
+                         void* workspace, size_t workspace_bytes, mi_stream_t stream) {
   MI_TRY(device_check());
   if (!col_lse_out) return MI_ERR_BAD_ARG;
   Bump ws(workspace, workspace_bytes, false);
   return stats_rc_impl(Opnd{static_cast<const __nv_bfloat16*>(Q), ldq, q_split == 2 ? 2 : 1},
                        Opnd{static_cast<const __nv_bfloat16*>(K), ldk, k_split == 2 ? 2 : 1},
                        sid_q, sid_k, q_offset, Bq, Bk, D, scale, row_out, scal_out, nullptr, nullptr, col_lse_out, ws,
-                       reinterpret_cast<cudaStream_t>(stream));
+                       reinterpret_cast<cudaStream_t>(stream), reinterpret_cast<cudaEvent_t>(event_k_ready), k_local_valid != 0,
+                       nullptr, include_pos != 0);
+}
+int mi_score_stats_rc(const void* Q, int64_t ldq, int q_split, const void* K, int64_t ldk, int k_split,
+                      const int32_t* sid_q, const int32_t* sid_k, int64_t q_offset,
+                      int64_t Bq, int64_t Bk, int64_t D, float scale, float* row_out, double* scal_out, float* col_lse_out,
+                      void* workspace, size_t workspace_bytes, mi_stream_t stream) {
+  return mi_score_stats_rc_ex(Q, ldq, q_split, K, ldk, k_split, sid_q, sid_k, q_offset, Bq, Bk, D, scale, row_out, scal_out,
+                              col_lse_out, nullptr, 0, 0, workspace, workspace_bytes, stream);
 }
 
 size_t mi_score_grad_workspace_bytes(int64_t Bq, int64_t Bk, int64_t D, int precision) {
@@ -2089,6 +2199,15 @@ int mi_merge_scalars(const double* scal_all, int world, int64_t B_global, int es
   loss_finalize_kernel<<<1, 32, 0, stream>>>(scratch8, nullptr, B_global, estimator, loss_out, lse_out, lambda, nullptr);
   MI_LAUNCH_CHECK("loss_finalize_kernel");
   return MI_OK;
+}
+int64_t mi_merge_sym_stats_scratch_doubles(int64_t B_global) { return B_global > 0 ? merge_sym_scratch_doubles(B_global) : 0; }
+int mi_merge_sym_stats(const double* scal_all, const float* col_all, int64_t col_pitch, int world, int64_t B_global,
+                       double* loss_out, float* c_out, double* scratch, mi_stream_t stream) {
+  MI_TRY(device_check());
+  if (!scal_all || !col_all || world <= 0 || B_global <= 0 || col_pitch < B_global || !loss_out || !c_out || !scratch)
+    return MI_ERR_BAD_ARG;
+  return merge_sym_impl(scal_all, 8, col_all, col_pitch, world, B_global, loss_out, c_out, scratch,
+                        reinterpret_cast<cudaStream_t>(stream));
 }
 int mi_single_finalize_q(const float* oq_raw, int64_t rows, int64_t D, const float* ref, const float* wrow, const float* lse,
                          int dv_like, float alpha, float gamma, const void* kdiag, int64_t ldk, int k_split,

@@ -24,6 +24,17 @@
 // The host reads ONE number per step, the merged guard count, as soon as the score tiles are done (it waits for an event on
 // the communication stream, not for the step); a non-zero count makes the call return MI_GUARD_TRIPPED on EVERY rank (the
 // count is the same everywhere) and the caller repeats the step on the exact path.
+//
+// Symmetric InfoNCE (exact references: no guard, no host read) replaces the references and the single pass by:
+//
+//   row+col statistics, OWN column tiles first       (aux stream: the mask, after the ids; other ranks' Y still arriving)
+//   <--ev-- wait Y; the remaining column tiles
+//   fold own diag into own column partials  --ev-->  ONE all-gather of the records {8 fp64 scalars | B fp32 column partials}
+//   <--ev-- c (fp64 log-sum-exp over ranks), loss   merge (fixed order: the same bits on every rank)
+//   gradient pass (refq = row lse, refk = c)  --ev-->  reduce-scatter of the final dY contributions     (under the dT contraction)
+//   dW = X^T dT                                --ev-->  all-reduce dW                                  (under the dX GEMM)
+//
+// The gradient pass needs every column's log-sum-exp, so the merge is a hard barrier between the two score computations.
 #include <dlfcn.h>
 
 namespace {
@@ -39,7 +50,7 @@ struct NcclApi {
   bool ok = false;
 };
 // nccl.h: ncclDataType_t / ncclRedOp_t values (stable across NCCL 2.x)
-constexpr int kNcclInt32 = 2, kNcclFloat32 = 7, kNcclFloat64 = 8, kNcclBf16 = 9, kNcclSum = 0, kNcclMax = 2;
+constexpr int kNcclUint8 = 1, kNcclInt32 = 2, kNcclFloat32 = 7, kNcclFloat64 = 8, kNcclBf16 = 9, kNcclSum = 0, kNcclMax = 2;
 
 const NcclApi& nccl_api() {
   static NcclApi api;
@@ -81,8 +92,9 @@ namespace {
 struct ShardBufs {
   __nv_bfloat16 *T, *Y_all, *dT16;
   int *sid_all, *flag;
-  float *ref, *diag, *lam_loc, *lam, *wrow, *rows, *lse32, *oq_raw, *ok_raw;
+  float *ref, *diag, *lam_loc, *lam, *wrow, *rows, *lse32, *oq_raw, *ok_raw, *c;
   double *scal, *scal_all, *scratch8;
+  uint8_t* rec_all;        // symmetric estimator: the ranks' packed records {8 fp64 scalars | B fp32 column partials | pad}
 };
 
 int sharded_impl(mi_dist_ctx* ctx, int world, int rank, const void* X_, const void* Y_, const void* W_, const int* sid_local,
@@ -90,25 +102,36 @@ int sharded_impl(mi_dist_ctx* ctx, int world, int rank, const void* X_, const vo
                  double* loss_out, float* dX, float* dY, float* dW, Bump& ws, int check_guard, cudaStream_t S) {
   typedef __nv_bfloat16 bf;
   if (Bl <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
-  if (estimator < MI_EST_DV || estimator > MI_EST_INFONCE_ROW) return MI_ERR_BAD_ARG;     // the symmetric form: host-side path
+  if (estimator < MI_EST_DV || estimator > MI_EST_INFONCE_SYM) return MI_ERR_BAD_ARG;
   const bool bilinear = critic == MI_CRITIC_BILINEAR;
-  const bool dv_like = estimator != MI_EST_INFONCE_ROW;
+  const bool sym = estimator == MI_EST_INFONCE_SYM;
+  const bool dv_like = estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF;
   const bool strict = (precision & 1) == MI_PREC_BF16_STRICT;
   if (world < 1 || rank < 0 || rank >= world) return MI_ERR_BAD_ARG;
   const long long Bg = Bl * world, off = static_cast<long long>(rank) * Bl;
   const int tsplit = (bilinear && strict) ? 2 : 1;
   const long long Dp = round_up(D, kSplitAlign);
   const long long ldT = tsplit == 2 ? 2 * Dp : D;
-  ShardBufs b;
+  // symmetric record of one rank: 64 B of scalars, then the column partials, padded to 16 B
+  const size_t rec_bytes = 64 + static_cast<size_t>(round_up(Bg * 4, 16));
+  ShardBufs b{};
   b.T = bilinear ? ws.take<bf>(static_cast<size_t>(Bl) * ldT) : nullptr;
   b.Y_all = ws.take<bf>(static_cast<size_t>(Bg) * D);
   b.dT16 = bilinear ? ws.take<bf>(static_cast<size_t>(Bl) * ldT) : nullptr;
-  b.sid_all = ws.take<int>(Bg); b.flag = ws.take<int>(1);
-  b.ref = ws.take<float>(Bl); b.diag = ws.take<float>(Bl); b.lam_loc = ws.take<float>(1); b.lam = ws.take<float>(1);
-  b.wrow = ws.take<float>(Bl); b.rows = ws.take<float>(static_cast<size_t>(Bl) * 4); b.lse32 = ws.take<float>(1);
-  b.oq_raw = (bilinear || !dX) ? ws.take<float>(static_cast<size_t>(Bl) * D) : nullptr;      // dot: dX doubles as the raw buffer
+  b.sid_all = ws.take<int>(Bg);
+  b.ref = ws.take<float>(Bl); b.rows = ws.take<float>(static_cast<size_t>(Bl) * 4);
+  if (sym) {
+    b.rec_all = ws.take<uint8_t>(static_cast<size_t>(world) * rec_bytes);
+    b.c = ws.take<float>(Bg);
+    b.scratch8 = ws.take<double>(merge_sym_scratch_doubles(Bg));
+  } else {
+    b.flag = ws.take<int>(1);
+    b.diag = ws.take<float>(Bl); b.lam_loc = ws.take<float>(1); b.lam = ws.take<float>(1);
+    b.wrow = ws.take<float>(Bl); b.lse32 = ws.take<float>(1);
+    b.oq_raw = (bilinear || !dX) ? ws.take<float>(static_cast<size_t>(Bl) * D) : nullptr;      // dot: dX doubles as the raw buffer
+    b.scal = ws.take<double>(8); b.scal_all = ws.take<double>(static_cast<size_t>(world) * 8); b.scratch8 = ws.take<double>(8);
+  }
   b.ok_raw = ws.take<float>(static_cast<size_t>(Bg) * D);
-  b.scal = ws.take<double>(8); b.scal_all = ws.take<double>(static_cast<size_t>(world) * 8); b.scratch8 = ws.take<double>(8);
   const long long k_pad_all = cdiv(Bg, mi::TILE_N) * mi::TILE_N;
   const MaskBuf all_mask = take_mask(ws, Bl, k_pad_all, Bg);      // rows: this rank's; columns: everyone's
   if (!ws.ok()) return MI_ERR_WORKSPACE;
@@ -121,10 +144,20 @@ int sharded_impl(mi_dist_ctx* ctx, int world, int rank, const void* X_, const vo
   const Opnd Yloc{static_cast<const bf*>(Y_), D, 1};
   if (ws.dry) {          // planning: the stage scratch of every stage, one after the other
     const Opnd To{nullptr, ldT, tsplit}, Ya{nullptr, D, 1};
-    MI_TRY(ref_sample_impl(To, Yloc, nullptr, nullptr, 0, Bl, Bl, D, 1.f, incl, 0, Bl, stride, margin, nullptr, nullptr, nullptr, ws, nullptr));
-    ws.release(mk);
-    MI_TRY(single_pass_impl(To, Ya, nullptr, nullptr, off, Bl, Bg, D, 1.f, incl, precision, gam, nullptr, nullptr, nullptr,
-                            nullptr, nullptr, nullptr, nullptr, nullptr, ws, nullptr));
+    if (sym) {
+      MI_TRY(stats_rc_impl(To, Ya, nullptr, nullptr, off, Bl, Bg, D, 1.f, nullptr, nullptr, nullptr, nullptr, nullptr, ws, nullptr,
+                           nullptr, false, &all_mask, true));
+      ws.release(mk);
+      // (planned as mi_score_grad_workspace_bytes plans the stage op, for its largest operand variant: a hi/lo K)
+      GradOut oq, okk;
+      MI_TRY(grad_impl(To, Opnd{nullptr, D, 2}, nullptr, nullptr, off, Bl, Bg, D, 1.f, nullptr, 1.f, nullptr, 1.f, 1, precision & 1,
+                       1.f, gam, oq, &okk, ws, nullptr, nullptr, &all_mask));
+    } else {
+      MI_TRY(ref_sample_impl(To, Yloc, nullptr, nullptr, 0, Bl, Bl, D, 1.f, incl, 0, Bl, stride, margin, nullptr, nullptr, nullptr, ws, nullptr));
+      ws.release(mk);
+      MI_TRY(single_pass_impl(To, Ya, nullptr, nullptr, off, Bl, Bg, D, 1.f, incl, precision, gam, nullptr, nullptr, nullptr,
+                              nullptr, nullptr, nullptr, nullptr, nullptr, ws, nullptr));
+    }
     ws.release(mk);
     if (bilinear) {        // dW split-K partials
       GemmArgs g; g.M = D; g.N = D; g.k_blocks = static_cast<int>(round_up(Bl, kSplitAlign) / bk()) * tsplit;
@@ -176,39 +209,72 @@ int sharded_impl(mi_dist_ctx* ctx, int world, int rank, const void* X_, const vo
   }
   const Opnd To = bilinear ? Opnd{b.T, ldT, tsplit} : Opnd{X, D, 1};
   const Opnd Ya{b.Y_all, D, 1};
-  MI_TRY(ref_sample_impl(To, Yloc, sid_local, sid_local, 0, Bl, Bl, D, inv_tau, incl, 0, Bl, stride, margin, b.ref, b.diag, b.lam_loc, ws, S));
-  ws.release(mk);
-  MI_CUDA(cudaEventRecord(ctx->ev_lamloc, S));
-  MI_CUDA(cudaStreamWaitEvent(Cs, ctx->ev_lamloc, 0));
-  if (world > 1) MI_NCCL(nc.all_reduce(b.lam_loc, b.lam, 1, kNcclFloat32, kNcclMax, ctx->comm, Cs));
-  else MI_CUDA(cudaMemcpyAsync(b.lam, b.lam_loc, 4, cudaMemcpyDeviceToDevice, Cs));
-  MI_CUDA(cudaEventRecord(ctx->ev_lam, Cs));
-  // ---- the single pass over this rank's rows against ALL columns
-  MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_mask, 0));
-  MI_CUDA(cudaMemsetAsync(b.flag, 0, sizeof(int), S));
-  float* oq_raw = b.oq_raw ? b.oq_raw : dX;
-  MI_TRY(single_pass_impl(To, Ya, b.sid_all + off, b.sid_all, off, Bl, Bg, D, inv_tau, incl, precision, gam, b.ref, b.lam, b.diag,
-                          b.rows, oq_raw, b.ok_raw, b.wrow, b.flag, ws, S, ctx->ev_k, b.scal, ctx->ev_s, ctx->ev_y, nullptr, nullptr,
-                          /*k_local_valid=*/true, &all_mask, ctx->ev_lam));
-  ws.release(mk);
-  // ---- scalars: exchange and merge on the communication stream, under the contractions; the guard goes to the host.
-  //      (The rows are reduced inside the pass, on the compute stream, BEFORE the dY contraction is launched: the engine's
-  //      persistent grid takes every SM, so a collective that is not already running when it starts waits for it to end —
-  //      measured: deferring the reduction to this stream delayed the scalar all-gather by the whole contraction.)
-  MI_CUDA(cudaStreamWaitEvent(Cs, ctx->ev_s, 0));
-  if (world > 1) MI_NCCL(nc.all_gather(b.scal, b.scal_all, 8, kNcclFloat64, ctx->comm, Cs));
-  else MI_CUDA(cudaMemcpyAsync(b.scal_all, b.scal, 64, cudaMemcpyDeviceToDevice, Cs));
-  merge_scal_kernel<<<1, 32, 0, Cs>>>(b.scal_all, world, b.scratch8);
-  MI_LAUNCH_CHECK("merge_scal_kernel");
-  loss_finalize_kernel<<<1, 32, 0, Cs>>>(b.scratch8, nullptr, Bg, estimator, loss_out, b.lse32, dv_like ? b.lam : nullptr, nullptr);
-  MI_LAUNCH_CHECK("loss_finalize_kernel");
-  if (check_guard) MI_CUDA(cudaMemcpyAsync(ctx->guard_host, loss_out + 7, sizeof(double), cudaMemcpyDeviceToHost, Cs));
-  MI_CUDA(cudaEventRecord(ctx->ev_m, Cs));
-  if (check_guard) {
-    MI_CUDA(cudaEventSynchronize(ctx->ev_m));            // the score tiles are done; the contractions are still running
-    if (ctx->guard_host[0] != 0.0) {                     // same verdict on every rank: abandon the step (no collective is pending)
-      MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_m, 0));
-      return MI_GUARD_TRIPPED;
+  float* oq_raw = b.oq_raw ? b.oq_raw : dX;      // (single pass)
+  if (sym) {
+    // ---- row + column statistics of this rank's rows against ALL columns (exact references: no guard), the own column
+    //      block first; the own positive pairs are folded into the own slots of the column partials, which go straight
+    //      into this rank's record of the packed exchange
+    uint8_t* rec = b.rec_all + static_cast<size_t>(rank) * rec_bytes;
+    MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_mask, 0));
+    MI_TRY(stats_rc_impl(To, Ya, b.sid_all + off, b.sid_all, off, Bl, Bg, D, inv_tau, b.rows, reinterpret_cast<double*>(rec),
+                         nullptr, nullptr, reinterpret_cast<float*>(rec + 64), ws, S, ctx->ev_y, /*k_local_valid=*/true, &all_mask,
+                         /*include_pos=*/true));
+    ws.release(mk);
+    make_ref_kernel<<<blocks_for(Bl, 256), 256, 0, S>>>(b.ref, reinterpret_cast<const float4*>(b.rows), 3, nullptr, Bl);
+    MI_LAUNCH_CHECK("make_ref_kernel");
+    MI_CUDA(cudaEventRecord(ctx->ev_s, S));
+    // ---- ONE all-gather of the records; every rank merges them the same way (fixed order: the same bits everywhere)
+    MI_CUDA(cudaStreamWaitEvent(Cs, ctx->ev_s, 0));
+    if (world > 1) MI_NCCL(nc.all_gather(rec, b.rec_all, rec_bytes, kNcclUint8, ctx->comm, Cs));
+    MI_TRY(merge_sym_impl(reinterpret_cast<const double*>(b.rec_all), static_cast<long long>(rec_bytes / 8),
+                          reinterpret_cast<const float*>(b.rec_all + 64), static_cast<long long>(rec_bytes / 4), world, Bg,
+                          loss_out, b.c, b.scratch8, Cs));
+    MI_CUDA(cudaEventRecord(ctx->ev_m, Cs));
+    // ---- the gradient pass needs every column reference c_j: G = (1/2B)(e^{S - r_i} + e^{S - c_j}), positives included.
+    //      dT (or dX) and this rank's dY contributions come out final; ev_k marks the contributions complete.
+    MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_m, 0));
+    GradOut oq, okk;
+    if (bilinear) { oq.bf16 = b.dT16; oq.ld16 = ldT; oq.split = tsplit; }
+    else { oq.f32 = dX; oq.ld = D; }
+    okk.f32 = b.ok_raw; okk.ld = D;
+    const float w = 0.5f / static_cast<float>(Bg);
+    MI_TRY(grad_impl(To, Ya, b.sid_all + off, b.sid_all, off, Bl, Bg, D, inv_tau, b.ref, w, b.c, w, 1, precision & 1, inv_tau, gam,
+                     oq, &okk, ws, S, ctx->ev_k, &all_mask));
+    ws.release(mk);
+  } else {
+    MI_TRY(ref_sample_impl(To, Yloc, sid_local, sid_local, 0, Bl, Bl, D, inv_tau, incl, 0, Bl, stride, margin, b.ref, b.diag, b.lam_loc, ws, S));
+    ws.release(mk);
+    MI_CUDA(cudaEventRecord(ctx->ev_lamloc, S));
+    MI_CUDA(cudaStreamWaitEvent(Cs, ctx->ev_lamloc, 0));
+    if (world > 1) MI_NCCL(nc.all_reduce(b.lam_loc, b.lam, 1, kNcclFloat32, kNcclMax, ctx->comm, Cs));
+    else MI_CUDA(cudaMemcpyAsync(b.lam, b.lam_loc, 4, cudaMemcpyDeviceToDevice, Cs));
+    MI_CUDA(cudaEventRecord(ctx->ev_lam, Cs));
+    // ---- the single pass over this rank's rows against ALL columns
+    MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_mask, 0));
+    MI_CUDA(cudaMemsetAsync(b.flag, 0, sizeof(int), S));
+    MI_TRY(single_pass_impl(To, Ya, b.sid_all + off, b.sid_all, off, Bl, Bg, D, inv_tau, incl, precision, gam, b.ref, b.lam, b.diag,
+                            b.rows, oq_raw, b.ok_raw, b.wrow, b.flag, ws, S, ctx->ev_k, b.scal, ctx->ev_s, ctx->ev_y, nullptr, nullptr,
+                            /*k_local_valid=*/true, &all_mask, ctx->ev_lam));
+    ws.release(mk);
+    // ---- scalars: exchange and merge on the communication stream, under the contractions; the guard goes to the host.
+    //      (The rows are reduced inside the pass, on the compute stream, BEFORE the dY contraction is launched: the engine's
+    //      persistent grid takes every SM, so a collective that is not already running when it starts waits for it to end —
+    //      measured: deferring the reduction to this stream delayed the scalar all-gather by the whole contraction.)
+    MI_CUDA(cudaStreamWaitEvent(Cs, ctx->ev_s, 0));
+    if (world > 1) MI_NCCL(nc.all_gather(b.scal, b.scal_all, 8, kNcclFloat64, ctx->comm, Cs));
+    else MI_CUDA(cudaMemcpyAsync(b.scal_all, b.scal, 64, cudaMemcpyDeviceToDevice, Cs));
+    merge_scal_kernel<<<1, 32, 0, Cs>>>(b.scal_all, world, b.scratch8);
+    MI_LAUNCH_CHECK("merge_scal_kernel");
+    loss_finalize_kernel<<<1, 32, 0, Cs>>>(b.scratch8, nullptr, Bg, estimator, loss_out, b.lse32, dv_like ? b.lam : nullptr, nullptr);
+    MI_LAUNCH_CHECK("loss_finalize_kernel");
+    if (check_guard) MI_CUDA(cudaMemcpyAsync(ctx->guard_host, loss_out + 7, sizeof(double), cudaMemcpyDeviceToHost, Cs));
+    MI_CUDA(cudaEventRecord(ctx->ev_m, Cs));
+    if (check_guard) {
+      MI_CUDA(cudaEventSynchronize(ctx->ev_m));            // the score tiles are done; the contractions are still running
+      if (ctx->guard_host[0] != 0.0) {                     // same verdict on every rank: abandon the step (no collective is pending)
+        MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_m, 0));
+        return MI_GUARD_TRIPPED;
+      }
     }
   }
   // ---- reduce-scatter of the dY contributions (as soon as they are complete: under the dT contraction)
@@ -218,11 +284,13 @@ int sharded_impl(mi_dist_ctx* ctx, int world, int rank, const void* X_, const vo
   MI_CUDA(cudaEventRecord(ctx->ev_rs, Cs));
   // ---- finalise: dT, dW (all-reduced), dX, dY
   MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_m, 0));
-  finalize_q_kernel<<<blocks_capped(Bl * D / 8, 256), 256, 0, S>>>(oq_raw, D, Bl, b.ref, b.wrow, b.lse32, dv_like ? 1 : 0, inv_tau, gam,
-                                                                   b.Y_all + off * D, D, 1, Dp, bilinear ? nullptr : dX,
-                                                                   bilinear ? b.dT16 : nullptr, (bilinear && tsplit == 2) ? b.dT16 + Dp : nullptr,
-                                                                   ldT, nullptr);
-  MI_LAUNCH_CHECK("finalize_q_kernel");
+  if (!sym) {
+    finalize_q_kernel<<<blocks_capped(Bl * D / 8, 256), 256, 0, S>>>(oq_raw, D, Bl, b.ref, b.wrow, b.lse32, dv_like ? 1 : 0, inv_tau, gam,
+                                                                     b.Y_all + off * D, D, 1, Dp, bilinear ? nullptr : dX,
+                                                                     bilinear ? b.dT16 : nullptr, (bilinear && tsplit == 2) ? b.dT16 + Dp : nullptr,
+                                                                     ldT, nullptr);
+    MI_LAUNCH_CHECK("finalize_q_kernel");
+  }
   if (bilinear) {
     if (dW) {
       GemmArgs g;
@@ -247,9 +315,11 @@ int sharded_impl(mi_dist_ctx* ctx, int world, int rank, const void* X_, const vo
     }
   }
   MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_rs, 0));
-  finalize_k_kernel<<<blocks_capped(Bl * D / 8, 256), 256, 0, S>>>(dY, D, Bl, b.lam, b.lse32, dv_like ? 1 : 0, inv_tau, gam,
-                                                                   To.p, To.ld, To.split, Dp, 0, Bl);
-  MI_LAUNCH_CHECK("finalize_k_kernel");
+  if (!sym) {       // (the symmetric gradient pass wrote its dY contributions final)
+    finalize_k_kernel<<<blocks_capped(Bl * D / 8, 256), 256, 0, S>>>(dY, D, Bl, b.lam, b.lse32, dv_like ? 1 : 0, inv_tau, gam,
+                                                                     To.p, To.ld, To.split, Dp, 0, Bl);
+    MI_LAUNCH_CHECK("finalize_k_kernel");
+  }
   if (bilinear && dW) MI_CUDA(cudaStreamWaitEvent(S, ctx->ev_dw, 0));
   return MI_OK;
 }

@@ -251,14 +251,21 @@ def sharded_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor, W:
     # ---- the exchange step
     nccl = world > 1 and dist.get_backend(group) != "gloo"
     single = need_grads and not sym and not two_pass
-    if (nccl and single and sid_local.dtype == torch.int32 and hasattr(backend, "sharded_step")
+    # symmetric InfoNCE always uses exact statistics; MI_SYM_RC=0 keeps its older op-by-op form (see below) for A/B runs
+    one_call_sym = sym and need_grads and os.environ.get("MI_SYM_RC", "1") != "0"
+    if (nccl and (single or one_call_sym) and sid_local.dtype == torch.int32 and hasattr(backend, "sharded_step")
             and os.environ.get("MI_SHARDED_IMPL", "c") != "python"):
         # the whole step, collectives included, as ONE library call (csrc/sharded.cuh): no per-op host overhead
         st, lo, dX, dY, dW = backend.sharded_step(Xb, Yb, Wb, sid_local, estimator, precision, inv_tau, group=group,
                                                   check_guard=check_guard)
         if st == 0:
-            return ({"loss": lo[0], "pos_mean": lo[1], "lse_neg": lo[2], "n_neg": lo[3], "loss_row": lo[4],
-                     "rows_without_negatives": lo[6], "guard": lo[7]}, dX, dY, dW)
+            out = {"loss": lo[0], "pos_mean": lo[1], "lse_neg": lo[2], "n_neg": lo[3], "loss_row": lo[4],
+                   "rows_without_negatives": lo[6], "guard": lo[7]}
+            if sym:
+                out["loss_col"] = lo[5]
+            return out, dX, dY, dW
+        if sym:
+            raise RuntimeError(f"mi_sharded_critic_loss_fwd_bwd: unexpected status {st} for infonce_sym")
         out, dX, dY, dW = sharded_critic_loss_fwd_bwd(X_local, Y_local, W, sid_local, estimator, precision, inv_tau,
                                                        need_grads, group, backend, two_pass=True)      # guard tripped on every rank
         out["guard"] = torch.ones((), dtype=torch.float64, device=out["loss"].device)

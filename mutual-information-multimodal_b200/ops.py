@@ -224,9 +224,12 @@ def score_stats(Q: Mat, K: Mat, sid_q: torch.Tensor, sid_k: torch.Tensor,
 
 
 def score_stats_rc(Q: Mat, K: Mat, sid_q: torch.Tensor, sid_k: torch.Tensor,
-                   q_offset: int = 0, scale: float = 1.0) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """mi_score_stats_rc: rows / scal as score_stats, plus col_lse [Bk] (fp32) = log-sum-exp of every column over this row
-    block's negatives, from the same score tiles (the symmetric estimator's statistics in the batch-sharded step)."""
+                   q_offset: int = 0, scale: float = 1.0, event_k_ready: Optional["torch.cuda.Event"] = None,
+                   k_local_valid: bool = False, include_pos: bool = False) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """mi_score_stats_rc_ex: rows / scal as score_stats, plus col_lse [Bk] (fp32) = log-sum-exp of every column over this row
+    block's negatives, from the same score tiles (the symmetric estimator's statistics in the batch-sharded step).
+    ``include_pos``: the block's positive pairs are folded into its own columns.  ``event_k_ready`` / ``k_local_valid``: as
+    in score_single_pass (the own column block is scored before the wait for the other ranks' text rows)."""
     _need_cuda(Q, K, sid_q, sid_k)
     lib = _lib.load()
     Qt, ldq, qsp, D = _opnd(Q)
@@ -239,8 +242,10 @@ def score_stats_rc(Q: Mat, K: Mat, sid_q: torch.Tensor, sid_k: torch.Tensor,
     col = torch.empty(Bk, dtype=torch.float32, device=Qt.device)
     nbytes = lib.mi_score_stats_rc_workspace_bytes(Bq, Bk, D)
     ws = workspace(nbytes, Qt.device)
-    _check(lib.mi_score_stats_rc(_ptr(Qt), ldq, qsp, _ptr(Kt), ldk, ksp, _ptr(sid_q), _ptr(sid_k), q_offset, Bq, Bk, D,
-                                 scale, _ptr(rows), _ptr(scal), _ptr(col), _ptr(ws), ws.numel(), _stream()), "mi_score_stats_rc")
+    _check(lib.mi_score_stats_rc_ex(_ptr(Qt), ldq, qsp, _ptr(Kt), ldk, ksp, _ptr(sid_q), _ptr(sid_k), q_offset, Bq, Bk, D,
+                                    scale, _ptr(rows), _ptr(scal), _ptr(col),
+                                    None if event_k_ready is None else C.c_void_p(event_k_ready.cuda_event), int(k_local_valid),
+                                    int(include_pos), _ptr(ws), ws.numel(), _stream()), "mi_score_stats_rc_ex")
     return rows, scal, col
 
 
@@ -374,6 +379,25 @@ def merge_scalars_loss(scal_all: torch.Tensor, estimator: str, b_global: int, la
             "rows_without_negatives": out[6], "guard": out[7], "lse32": lse32}
 
 
+def merge_sym_stats(scal_all: torch.Tensor, col_all: torch.Tensor, b_global: int) -> dict:
+    """mi_merge_sym_stats: the ranks' scalar rows [world, 8] (fp64) and column partials [world, >= b_global] (fp32, own
+    positive pairs folded in: score_stats_rc(include_pos=True)) -> the symmetric loss terms as 0-d fp64 views (the layout of
+    the single-GPU call) and "c" [b_global] fp32, the column log-sum-exps of the batch."""
+    _need_cuda(scal_all, col_all)
+    scal_all = scal_all.to(torch.float64).contiguous()
+    if col_all.dtype != torch.float32 or col_all.stride(1) != 1:
+        col_all = col_all.to(torch.float32).contiguous()
+    dev = scal_all.device
+    lib = _lib.load()
+    out = torch.empty(8, dtype=torch.float64, device=dev)
+    c = torch.empty(b_global, dtype=torch.float32, device=dev)
+    scratch = torch.empty(int(lib.mi_merge_sym_stats_scratch_doubles(b_global)), dtype=torch.float64, device=dev)
+    _check(lib.mi_merge_sym_stats(_ptr(scal_all), _ptr(col_all), col_all.stride(0), scal_all.shape[0], b_global, _ptr(out),
+                                  _ptr(c), _ptr(scratch), _stream()), "mi_merge_sym_stats")
+    return {"loss": out[0], "pos_mean": out[1], "lse_neg": out[2], "n_neg": out[3], "loss_row": out[4], "loss_col": out[5],
+            "rows_without_negatives": out[6], "guard": out[7], "c": c}
+
+
 def single_finalize_q(oq_raw, ref, wrow, lse, dv_like: bool, alpha: float, gamma: float, kdiag: Mat,
                       want_f32: bool = True, want_bf16: bool = False, out_split: bool = False):
     """Oq = alpha (c_q oq_raw - gamma Kdiag): fp32 and/or bf16 (hi/lo) result."""
@@ -468,9 +492,9 @@ def dist_context(group=None):
 
 def sharded_step(X_local: torch.Tensor, Y_local: torch.Tensor, W: Optional[torch.Tensor], sid_local: torch.Tensor,
                  estimator: str, precision: str, inv_tau: float, group=None, check_guard: bool = True):
-    """mi_sharded_critic_loss_fwd_bwd: the whole batch-sharded step (collectives included) as one library call.
-    Returns (status, loss_out fp64[8], dX, dY, dW); status GUARD_TRIPPED (on every rank alike) means the outputs are not
-    valid and the step must be repeated on the exact path."""
+    """mi_sharded_critic_loss_fwd_bwd: the whole batch-sharded step (collectives included) as one library call, for every
+    estimator.  Returns (status, loss_out fp64[8], dX, dY, dW); status GUARD_TRIPPED (on every rank alike) means the outputs
+    are not valid and the step must be repeated on the exact path ("infonce_sym" uses exact statistics: always 0)."""
     _need_cuda(X_local, Y_local, W, sid_local)
     lib = _lib.load()
     ctx, rank, world, _ = dist_context(group)
