@@ -47,8 +47,14 @@ enum mi_critic { MI_CRITIC_DOT = 0, MI_CRITIC_BILINEAR = 1 };
 
 /* estimator codes.  DV and INFONCE_REF restate mi_critics.py:3-12 and :14-23 (the reference's
  * "infonce" is DV + log N_neg); INFONCE_ROW / INFONCE_SYM are the true row / symmetric InfoNCE
- * bounds the north star adds (no counterpart in the reference). */
-enum mi_estimator { MI_EST_DV = 0, MI_EST_INFONCE_REF = 1, MI_EST_INFONCE_ROW = 2, MI_EST_INFONCE_SYM = 3 };
+ * bounds the north star adds (no counterpart in the reference).  JS and NWJ are the f-divergence
+ * bounds (no counterpart in the reference either; minimised, i.e. minus the bound; M = the negatives mask):
+ *   JS   (Jensen-Shannon, Deep InfoMax / f-GAN):  L = mean_{M} softplus(S) + mean_i softplus(-S_ii)
+ *   NWJ  (Nguyen-Wainwright-Jordan, "MINE-f"):    L = e^{-1} mean_{M} e^{S} - mean_i S_ii = e^{LSE_M - ln N_neg - 1} - pos_mean
+ * JS and NWJ run only in the single-GPU separable-critic entries (mi_critic_loss_fwd_bwd and its host forms); every other
+ * entry that takes an estimator rejects them (MI_ERR_BAD_ARG, or a size of 0 from its planner). */
+enum mi_estimator { MI_EST_DV = 0, MI_EST_INFONCE_REF = 1, MI_EST_INFONCE_ROW = 2, MI_EST_INFONCE_SYM = 3,
+                    MI_EST_JS = 4, MI_EST_NWJ = 5 };
 
 enum mi_precision { MI_PREC_BF16_FAST = 0,   /* dS panel rounded once to bf16 */
                     MI_PREC_BF16_STRICT = 1, /* dS = hi + lo bf16 split (fp32-accumulate mode) */
@@ -230,7 +236,19 @@ int mi_single_finalize_k(float* ok, int64_t rows, int64_t D, const float* lambda
  * asynchronous and CUDA-graph capturable, and the results are ALWAYS those of a pass whose guard was clear.
  * guard (loss_out[7]) = number of rows that tripped the sampled pass: > 0 only says that the exact repeat produced the
  * results.  MI_PREC_TWO_PASS asks for exact references from the start.  The symmetric estimator always runs the
- * statistics passes + one gradient pass with exact references. */
+ * statistics passes + one gradient pass with exact references.
+ *
+ * MI_EST_NWJ runs DV's single pass (same references, guard and exact repeat; MI_PREC_TWO_PASS = exact references) and
+ * differs only in its scalar: G = kappa softmax_M(S) - I/B, kappa = e^{LSE_M - ln N_neg - 1} (ln N_neg in fp64).  A kappa
+ * outside the fp32 range is NOT a guard condition (an exact repeat could not change it): the fp64 loss stays finite and the
+ * gradients overflow as an fp32 computation of the same formula would.
+ * MI_EST_JS needs no normaliser: ONE score pass per row panel writes M sigma(S) into the dS panel and sums M softplus(S) per
+ * row; G = M sigma(S) / N_neg - diag(sigma(-S_ii)) / B.  No reference sample, no guard (loss_out[7] = 0), MI_PREC_TWO_PASS
+ * changes nothing.  Forward-only calls run the same pass without the panel.
+ * loss_out of the two:     slot   0     1          2                       3       4                       5   6                  7
+ *                          NWJ    loss  pos_mean   LSE_M                   n_neg   0                       0   rows w/o neg.      guard (as DV)
+ *                          JS     loss  pos_mean   mean_M softplus(S)      n_neg   mean_i softplus(-S_ii)  0   rows w/o neg.      0
+ * Without any negative pair the loss of both is NaN. */
 size_t mi_critic_workspace_bytes(int64_t B, int64_t D, int critic, int estimator, int precision, int need_grads);
 int mi_critic_loss_fwd_bwd(const void* X, const void* Y, const void* W, const int32_t* sid,
                            int64_t B, int64_t D, int critic, int estimator, int precision, float inv_tau,

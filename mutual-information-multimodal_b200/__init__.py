@@ -17,12 +17,12 @@ device is missing.
 from . import _lib  # noqa: F401
 from .critic import (  # noqa: F401
     FusedCritic, FusedMLPCritic, PairBatch, ScoreHandle, create_mi_pairs, create_mi_pairs_tensor, dv_bound_loss, infonce_bound_loss,
-    mi_estimator_loss, select_estimator, sharded_mi_loss,
+    js_bound_loss, mi_estimator_loss, nwj_bound_loss, select_estimator, sharded_mi_loss,
 )
 from .ops import MIError  # noqa: F401
 from .validate import gdv_calculation, gdv_terms  # noqa: F401
 
 __all__ = [
     "FusedCritic", "FusedMLPCritic", "PairBatch", "ScoreHandle", "create_mi_pairs", "create_mi_pairs_tensor", "dv_bound_loss",
-    "infonce_bound_loss", "mi_estimator_loss", "select_estimator", "sharded_mi_loss", "MIError", "gdv_calculation", "gdv_terms",
+    "infonce_bound_loss", "js_bound_loss", "nwj_bound_loss", "mi_estimator_loss", "select_estimator", "sharded_mi_loss", "MIError", "gdv_calculation", "gdv_terms",
 ]

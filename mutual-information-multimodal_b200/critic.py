@@ -29,6 +29,7 @@ from typing import Optional, Sequence, Union
 
 import torch
 import torch.nn as nn
+import torch.nn.functional as F
 
 from . import ops
 
@@ -201,6 +202,7 @@ def sharded_mi_loss(embedding_img, embedding_txt, critic: "FusedCritic", study_i
     DistributedDataParallel's gradient averaging of the encoders yields the gradient of the global loss; parameter
     gradients are those of the global loss, not scaled.  ``critic`` is a ``FusedCritic`` or a ``FusedMLPCritic``."""
     import torch.distributed as tdist
+    ops.reject_separable_only(estimator, "the batch-sharded loss")
     world = tdist.get_world_size(group) if tdist.is_available() and tdist.is_initialized() else 1
     sid = study_id if torch.is_tensor(study_id) else torch.tensor([int(s) for s in study_id], dtype=torch.int64)
     sid = sid.to(embedding_img.device)
@@ -307,6 +309,7 @@ class FusedMLPCritic(nn.Sequential):
 def mi_estimator_loss(handle: ScoreHandle, estimator: str) -> torch.Tensor:
     p, c = handle.pairs, handle.critic
     if isinstance(c, FusedMLPCritic):
+        ops.reject_separable_only(estimator, "the concat-MLP critic (FusedMLPCritic)")
         return _FusedMLPCriticLoss.apply(p.embedding_img, p.embedding_txt, c[0].weight, c[0].bias, c[2].weight, c[2].bias,
                                          c[4].weight, c[4].bias, p.sid, estimator, c.precision, c.check_negatives)
     return _FusedCriticLoss.apply(p.embedding_img, p.embedding_txt, c.W, p.sid, estimator, c.precision,
@@ -350,12 +353,41 @@ def infonce_sym_loss(handle: ScoreHandle, pos_size=None, device=None):
     return mi_estimator_loss(handle, "infonce_sym")
 
 
+def js_bound_loss(discriminator_logits, pos_size, device=None):
+    """Jensen-Shannon bound (Deep InfoMax / f-GAN; no counterpart in the reference), minimised:
+    ``mean_{negatives} softplus(S) + mean_i softplus(-S_ii)``.  A ``ScoreHandle`` runs the fused path; a plain logits
+    tensor (positives first, then negatives, as ``create_mi_pairs_tensor`` orders them) is computed with torch ops.  0-d."""
+    if isinstance(discriminator_logits, ScoreHandle):
+        if pos_size != discriminator_logits.pairs.batch_size:
+            raise ValueError("pos_size must equal the batch size (main_utils.py:224 passes args.batch_size)")
+        return mi_estimator_loss(discriminator_logits, "js")
+    logits = discriminator_logits
+    pos, neg = logits[:pos_size], logits[pos_size:]
+    return torch.mean(F.softplus(neg)) + torch.mean(F.softplus(-pos))
+
+
+def nwj_bound_loss(discriminator_logits, pos_size, device=None):
+    """NWJ bound (Nguyen-Wainwright-Jordan, "MINE-f"; no counterpart in the reference), minimised:
+    ``e^{-1} mean_{negatives} e^{S} - mean_i S_ii = e^{LSE - ln N_neg - 1} - pos_mean`` (ln N_neg in fp64).
+    ``ScoreHandle`` -> fused path; plain logits (positives first) -> torch ops.  0-d."""
+    if isinstance(discriminator_logits, ScoreHandle):
+        if pos_size != discriminator_logits.pairs.batch_size:
+            raise ValueError("pos_size must equal the batch size (main_utils.py:224 passes args.batch_size)")
+        return mi_estimator_loss(discriminator_logits, "nwj")
+    logits = discriminator_logits
+    pos, neg = logits[:pos_size], logits[pos_size:]
+    n_neg = neg.numel()
+    ln_n = math.log(n_neg) if n_neg > 0 else -math.inf
+    return torch.exp(torch.logsumexp(neg.reshape(-1), dim=0) - (ln_n + 1.0)) - torch.mean(pos)
+
+
 def select_estimator(name: str):
     """main_utils.py:141-144: 'dv' -> dv_bound_loss, 'infonce' -> infonce_bound_loss.  The reference
     leaves ``mi_critic`` unbound for any other value (UnboundLocalError at :224); here the two new
     estimators are selectable and anything else raises immediately."""
     table = {"dv": dv_bound_loss, "infonce": infonce_bound_loss,
-             "infonce_row": infonce_row_loss, "infonce_sym": infonce_sym_loss}
+             "infonce_row": infonce_row_loss, "infonce_sym": infonce_sym_loss,
+             "js": js_bound_loss, "nwj": nwj_bound_loss}
     if name not in table:
         raise ValueError(f"unknown mi_estimator {name!r} (reference: main_utils.py:141-144)")
     return table[name]

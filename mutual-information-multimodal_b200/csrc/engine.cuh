@@ -720,6 +720,86 @@ struct EpiPStore {
   }
 };
 
+__device__ __forceinline__ float rcp_approx(float x) {
+  float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y;
+}
+// log1p(e) for e in [0, 1]: degree-8 polynomial e * p(e) on the FMA pipe, |error| < 2e-7 in fp32 (fitted to log1p on [0, 1])
+__device__ __forceinline__ float log1p_unit(float e) {
+  float p = -0.006472604814916849f;
+  p = fmaf(p, e, 0.03617211803793907f);
+  p = fmaf(p, e, -0.09547846019268036f);
+  p = fmaf(p, e, 0.16779260337352753f);
+  p = fmaf(p, e, -0.2408052682876587f);
+  p = fmaf(p, e, 0.331819087266922f);
+  p = fmaf(p, e, -0.49987688660621643f);
+  p = fmaf(p, e, 0.999996542930603f);
+  return p * e;
+}
+
+// ---- Jensen-Shannon dS panel: P[row, col] = M sigma(S) (bf16 hi [+ lo], stored as EpiPStore does) and the fp32 row sums of
+//      M softplus(S) (sum_part; the loss).  Per score: one MUFU.EX2 (e = e^{-|S|}), one MUFU.RCP (r = 1 / (1 + e)),
+//      sigma(S) = r (S >= 0) or e r, softplus(S) = max(S, 0) + log1p(e) with log1p as a polynomial on the FMA pipe.  Safe for
+//      any finite S (e in [0, 1]).  The weights lie in (0, 1): no reference, no running maximum, no guard.
+//      kStore = false: the row sums only (forward-only calls), no panel.  Params as EpiPStore (refq / refk2 / include_diag unused).
+template <bool kStore>
+struct EpiJS {
+  static constexpr bool kJoint = false;
+  static constexpr bool kWalk = false;
+  static constexpr bool kChunk16 = false;
+  static constexpr int kEpiSmemBytes = kStore ? kNumEpiWarps * 2048 : 0;
+  using Params = EpiPStore::Params;
+  struct State { uint8_t* stage_smem; MaskState ms; float s; };
+
+  static __device__ __forceinline__ void init(const Params&, State&) {}
+  static __device__ __forceinline__ void finish(const Params&, State&, int) {
+    if (kStore && (threadIdx.x & 31) == 0) ptx::tma_store_wait_all();
+  }
+  static __device__ __forceinline__ void unit_begin(const Params& p, State& st, const Unit&, int row, int) {
+    st.s = 0.f;
+    mask_begin(p.mask, st.ms, row, p.q_rows);
+  }
+  static __device__ __forceinline__ void chunk(const Params& p, State& st, const Unit&, int row, int col0,
+                                               uint32_t (&v)[32]) {
+    const float sc = p.scale, c2 = -p.scale * kLog2e;   // scale > 0: |S| log2 e = |acc| scale log2 e
+    const int lane = (int)(threadIdx.x & 31);
+    const uint32_t mk = chunk_mask(p.mask, st.ms, col0, p.k_cols);
+    const bool split = kStore && p.lo_col0 > 0;        // strict mode: residual panel, lo_col0 columns to the right
+    float s[4] = {0.f, 0.f, 0.f, 0.f};
+    uint32_t hi[16], lo[16];
+    // pairs of scores, packed as soon as they are formed (v dies as hi / lo fill: no spills at 96 registers)
+#pragma unroll
+    for (int c = 0; c < 32; c += 2) {
+      float sig[2];
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        const float a = __uint_as_float(v[c + j]);
+        const float e = ptx::ex2(fabsf(a) * c2);
+        float sp = fmaf(fmaxf(a, 0.f), sc, log1p_unit(e));
+        if constexpr (kStore) {
+          const float r = rcp_approx(1.f + e);
+          sig[j] = a >= 0.f ? r : e * r;
+        }
+        if ((mk >> (c + j)) & 1u) { sig[j] = 0.f; sp = 0.f; }
+        s[(c + j) & 3] += sp;
+      }
+      if constexpr (kStore) {
+        const uint32_t h = ptx::pack_bf16(sig[0], sig[1]);
+        hi[c / 2] = h;
+        if (split) lo[c / 2] = ptx::pack_bf16(sig[0] - __uint_as_float(h << 16), sig[1] - __uint_as_float(h & 0xffff0000u));
+      }
+    }
+    st.s += (s[0] + s[1]) + (s[2] + s[3]);
+    if constexpr (kStore) {
+      const int row0 = row - lane;
+      EpiPStore::stage_and_store(p, st.stage_smem, lane, hi, col0, row0);
+      if (split) EpiPStore::stage_and_store(p, st.stage_smem, lane, lo, col0 + p.lo_col0, row0);
+    }
+  }
+  static __device__ __forceinline__ void unit_end(const Params& p, State& st, const Unit& un, int row, int colq) {
+    p.sum_part[((size_t)un.s * kColQuarters + colq) * p.rows_padded + row] = st.s;
+  }
+};
+
 // ---- plain GEMM epilogue: C = alpha * (ACC - gamma * SUB) [+ C_prev]
 struct EpiStore {
   static constexpr bool kJoint = false;

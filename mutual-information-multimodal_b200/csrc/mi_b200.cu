@@ -220,6 +220,8 @@ int launch_engine_cg(const MapSpec& a, const MapSpec& b, const Sched& sc, const 
 template <> struct EpiKind<mi::EpiStats> { static constexpr int value = 0; };
 template <> struct EpiKind<mi::EpiStatsRC> { static constexpr int value = 0; };
 template <> struct EpiKind<mi::EpiPStore> { static constexpr int value = 1; };
+template <> struct EpiKind<mi::EpiJS<true>> { static constexpr int value = 1; };    // Jensen-Shannon dS panel
+template <> struct EpiKind<mi::EpiJS<false>> { static constexpr int value = 0; };   // its statistics-only form
 template <> struct EpiKind<mi::EpiStore> { static constexpr int value = 2; };
 template <> struct EpiKind<mi::EpiMlpFwd> { static constexpr int value = 5; };   // MLP critic: two-pass epilogues
 template <> struct EpiKind<mi::EpiMlpDz> { static constexpr int value = 5; };
@@ -822,17 +824,108 @@ __global__ void loss_finalize_kernel(const double* __restrict__ scal_row, const 
   const double pos = scal_row[3] / (double)B;
   const double loss_row = scal_row[4] / (double)B;
   const double loss_col = scal_col ? scal_col[4] / (double)B : 0.0;
+  if (estimator == MI_EST_JS) {   // scal_row in js_reduce_kernel's layout; lse_f = 1 / N_neg, the weight of every negative in G
+    const double sp_neg = scal_row[0] / n_neg, sp_pos = scal_row[4] / (double)B;
+    loss_out[0] = sp_neg + sp_pos; loss_out[1] = pos; loss_out[2] = sp_neg; loss_out[3] = n_neg;
+    loss_out[4] = sp_pos; loss_out[5] = 0.0; loss_out[6] = scal_row[5]; loss_out[7] = 0.0;
+    if (lse_f) *lse_f = (float)(1.0 / n_neg);
+    return;
+  }
   double loss;
   if (estimator == MI_EST_DV) loss = lse - log((double)(float)n_neg) - pos;   // fp32 N_neg as mi_critics.py:10
   else if (estimator == MI_EST_INFONCE_REF) loss = lse - pos;
   else if (estimator == MI_EST_INFONCE_ROW) loss = loss_row;
+  else if (estimator == MI_EST_NWJ) loss = exp(lse - log(n_neg) - 1.0) - pos;   // fp64 ln N_neg (no reference to mirror)
   else loss = 0.5 * (loss_row + loss_col);
+  const bool nwj = estimator == MI_EST_NWJ;
   double guard = scal_row[6];
-  if (lambda != nullptr && (estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF) && n_neg > 0.0 &&
+  if (lambda != nullptr && (estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF || nwj) && n_neg > 0.0 &&
       !(fabs((double)lambda[0] - lse) <= 60.0)) guard += 1.0;
   loss_out[0] = loss; loss_out[1] = pos; loss_out[2] = lse; loss_out[3] = n_neg;
-  loss_out[4] = loss_row; loss_out[5] = loss_col; loss_out[6] = scal_row[5]; loss_out[7] = guard;
-  if (lse_f) *lse_f = (float)lse;
+  loss_out[4] = nwj ? 0.0 : loss_row; loss_out[5] = loss_col; loss_out[6] = scal_row[5]; loss_out[7] = guard;
+  // NWJ: G = kappa softmax_M(S) - I/B with kappa = e^{LSE - ln N_neg - 1}, i.e. DV's G with LSE replaced by 1 + ln N_neg: the
+  // finalisations (c_q = e^{ref_q - lse_f}, e^{lambda - lse_f}) then need no change
+  if (lse_f) *lse_f = nwj ? (float)(log(n_neg) + 1.0) : (float)lse;
+}
+
+// ---- Jensen-Shannon (no normaliser: the weights sigma(S) lie in (0, 1))
+// rows of one panel: row_out = {sum_k M softplus(S) (the partial row sums added), n_neg, S_ii, softplus(-S_ii)}
+__global__ void js_rows_kernel(const float* __restrict__ part, int n_part, int rows_padded, int rows,
+                               const int* __restrict__ n_same, int k_cols, const float* __restrict__ diag_in,
+                               float4* __restrict__ row_out) {
+  const int row = blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= rows) return;
+  float l = 0.f;
+  for (int p = 0; p < n_part; ++p) l += part[(size_t)p * rows_padded + row];
+  const float d = diag_in[row];
+  row_out[row] = make_float4(l, static_cast<float>(k_cols - n_same[row]), d, fmaxf(-d, 0.f) + log1pf(expf(-fabsf(d))));
+}
+// one block of kJsRedThreads, fixed order: scal = {sum M softplus(S), 0, n_neg, sum S_ii, sum softplus(-S_ii), rows w/o negatives, 0, 0}
+constexpr int kJsRedThreads = 256;
+__global__ void js_reduce_kernel(const float4* __restrict__ row_out, long long rows, double* __restrict__ scal) {
+  __shared__ double sh[5][kJsRedThreads];
+  double a[5] = {0, 0, 0, 0, 0};
+  for (long long r = threadIdx.x; r < rows; r += kJsRedThreads) {
+    const float4 v = row_out[r];
+    a[0] += v.x; a[1] += v.y; a[2] += v.z; a[3] += v.w;
+    if (!(v.y > 0.f)) a[4] += 1.0;
+  }
+  for (int k = 0; k < 5; ++k) sh[k][threadIdx.x] = a[k];
+  __syncthreads();
+  for (int o = kJsRedThreads / 2; o; o >>= 1) {
+    if ((int)threadIdx.x < o) for (int k = 0; k < 5; ++k) sh[k][threadIdx.x] += sh[k][threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    scal[0] = sh[0][0]; scal[1] = 0.0; scal[2] = sh[1][0]; scal[3] = sh[2][0]; scal[4] = sh[3][0]; scal[5] = sh[4][0];
+    scal[6] = 0.0; scal[7] = 0.0;
+  }
+}
+// the gradients from the raw contractions: out[i,:] = alpha (w[0] raw[i,:] - (sigma(-S_ii) / B) sub[i,:]), w[0] = 1 / N_neg.
+// The positive pair's weight is per row.  raw may equal out_f32 (in place).  8 elements / thread.
+__global__ void js_finalize_kernel(const float* raw, long long D, long long rows, const float* __restrict__ w,
+                                   const float* __restrict__ diag, float inv_b, float alpha,
+                                   const __nv_bfloat16* __restrict__ sub, long long ld_sub, int sub_split, long long Dp,
+                                   float* out_f32, __nv_bfloat16* __restrict__ out_bf16, __nv_bfloat16* __restrict__ out_lo, long long ld16) {
+  const float c = w[0];
+  for (long long idx = (blockIdx.x * (long long)blockDim.x + threadIdx.x) * 8; idx < rows * D;
+       idx += (long long)gridDim.x * blockDim.x * 8) {
+    const long long i = idx / D, d = idx - i * D;          // D % 8 == 0
+    const float gam = inv_b / (1.f + expf(diag[i]));       // sigma(-S_ii) / B
+    const uint4 kv = *reinterpret_cast<const uint4*>(sub + i * ld_sub + d);
+    const uint32_t kw[4] = {kv.x, kv.y, kv.z, kv.w};
+    float kd[8];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) { kd[2 * j] = __uint_as_float(kw[j] << 16); kd[2 * j + 1] = __uint_as_float(kw[j] & 0xffff0000u); }
+    if (sub_split == 2) {
+      const uint4 lv = *reinterpret_cast<const uint4*>(sub + i * ld_sub + Dp + d);
+      const uint32_t lw[4] = {lv.x, lv.y, lv.z, lv.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) { kd[2 * j] += __uint_as_float(lw[j] << 16); kd[2 * j + 1] += __uint_as_float(lw[j] & 0xffff0000u); }
+    }
+    const float4 r0 = *reinterpret_cast<const float4*>(raw + idx), r1 = *reinterpret_cast<const float4*>(raw + idx + 4);
+    const float rv[8] = {r0.x, r0.y, r0.z, r0.w, r1.x, r1.y, r1.z, r1.w};
+    float o[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) o[j] = alpha * (c * rv[j] - gam * kd[j]);
+    if (out_f32) {
+      *reinterpret_cast<float4*>(out_f32 + idx) = make_float4(o[0], o[1], o[2], o[3]);
+      *reinterpret_cast<float4*>(out_f32 + idx + 4) = make_float4(o[4], o[5], o[6], o[7]);
+    }
+    if (out_bf16) {
+      uint32_t h[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) h[j] = ptx::pack_bf16(o[2 * j], o[2 * j + 1]);
+      *reinterpret_cast<uint4*>(out_bf16 + i * ld16 + d) = make_uint4(h[0], h[1], h[2], h[3]);
+      if (out_lo) {
+        uint32_t l[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          l[j] = ptx::pack_bf16(o[2 * j] - __uint_as_float(h[j] << 16), o[2 * j + 1] - __uint_as_float(h[j] & 0xffff0000u));
+        *reinterpret_cast<uint4*>(out_lo + i * ld16 + d) = make_uint4(l[0], l[1], l[2], l[3]);
+      }
+    }
+  }
 }
 
 // ---- symmetric InfoNCE over row blocks (the batch-sharded step): each rank's column partials carry its own positive
@@ -1687,6 +1780,107 @@ int single_pass_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* 
   return MI_OK;
 }
 
+// Jensen-Shannon on one GPU (square batch, row q pairs with column q): per row panel ONE score computation (EpiJS) writes
+// P = M sigma(S) and the row sums of M softplus(S) (-> row_out in js_rows_kernel's layout, scal_out after the last panel);
+// the two contractions give the RAW gradients  oq_raw = P K  and  ok_raw = P^T Q  (accumulated over the panels).  The
+// weight 1/N_neg and the positive terms are applied by js_finalize_kernel once N_neg is known.  oq_raw == ok_raw == nullptr:
+// the statistics only (EpiJS<false>, no panel).  diag[q] = S[q, q]; with `feed` it is valid for a panel after before_panel.
+int js_pass_impl(const Opnd& Q, const Opnd& K, const int* sid, long long B, long long D, float scale, int precision,
+                 const float* diag, float* row_out, double* scal_out, float* oq_raw, float* ok_raw, const MaskBuf& mb,
+                 Bump& ws, cudaStream_t stream, const PanelFeed* feed = nullptr) {
+  if (B <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
+  typedef __nv_bfloat16 bf;
+  const bool strict = (precision & 1) == MI_PREC_BF16_STRICT;
+  const bool grads = oq_raw != nullptr || ok_raw != nullptr || ws.dry;
+  const int n_ntile = static_cast<int>(cdiv(B, mi::TILE_N));
+  const long long k_pad = static_cast<long long>(n_ntile) * mi::TILE_N;
+  const int kp = static_cast<int>(k_pad / bk());
+  const long long pitch = k_pad * (strict ? 2 : 1);
+  const long long Dp = round_up(D, kSplitAlign);
+  const bool k_hl = strict && K.split == 2, q_hl = strict && Q.split == 2;
+  const long long panel_rows = panel_mblks(B, B, D, precision & 1) * rows_per_mblk();
+  bf* P = grads ? ws.take<bf>(static_cast<size_t>(panel_rows) * pitch) : nullptr;
+  const size_t part_slices = static_cast<size_t>(n_ntile > 64 ? 64 : n_ntile) * mi::kColQuarters;
+  float* part = ws.take<float>(part_slices * panel_rows);
+  const int oq_ksplit = strict ? strict_ksplit(kp * (k_hl ? 3 : 2)) : 1;     // see kStrictChainBlocks
+  const size_t kpart_elems = (grads && oq_ksplit > 1) ? static_cast<size_t>(oq_ksplit) * panel_rows * round_up(D, 4) : 0;
+  float* kpart = kpart_elems ? ws.take<float>(kpart_elems) : nullptr;
+  if (!ws.ok()) return MI_ERR_WORKSPACE;
+  if (ws.dry) return MI_OK;
+  if (!Q.p || !K.p || !sid || !diag || !row_out || !scal_out || !(scale > 0.f)) return MI_ERR_BAD_ARG;
+  const Opnd Qe{Q.p, Q.ld, strict ? Q.split : 1}, Ke{K.p, K.ld, strict ? K.split : 1};
+  Bump none(nullptr, 0, false);
+  for (long long r0 = 0; r0 < B; r0 += panel_rows) {
+    const long long rows = (B - r0 < panel_rows) ? (B - r0) : panel_rows;
+    if (feed != nullptr) MI_TRY(feed->before_panel(r0, rows));
+    // (1) score tiles -> P panel + partial row sums of softplus
+    Sched sc;
+    sc.n_mblk = static_cast<int>(cdiv(rows, rows_per_mblk()));
+    sc.n_ntile = n_ntile;
+    sc.n_split = choose_split(sc.n_mblk, sc.n_ntile, num_pairs());
+    if (sc.n_split > 64) sc.n_split = 64;
+    sc.n_ksplit = 1; sc.order = 0;
+    MI_TRY(score_segments(sc, Qe, Ke, D));
+    const int rows_padded = sc.n_mblk * rows_per_mblk();
+    mi::EpiPStore::Params ep;
+    ep.mask = mi::MaskInfo{mb.excl + r0, mb.n_same + r0, sid + r0, mb.sidk_pad};
+    ep.q_rows = static_cast<int>(rows); ep.k_cols = static_cast<int>(B);
+    ep.q_offset = r0; ep.scale = scale;
+    ep.refq = nullptr; ep.ln_wq = 0.f; ep.use_q = 0; ep.refk2 = nullptr; ep.use_k = 0; ep.include_diag = 0;
+    ep.lo_col0 = strict ? static_cast<int>(k_pad) : 0;
+    ep.sum_part = part; ep.rows_padded = rows_padded;
+    const MapSpec ma{Qe.p + r0 * Qe.ld, rows, opnd_k_extent(Qe, D), Qe.ld}, mbk{Ke.p, B, opnd_k_extent(Ke, D), Ke.ld};
+    if (grads) {
+      MI_TRY(make_tmap_store32(&ep.tmap_p, P, rows, pitch, pitch));
+      MI_TRY(launch_engine<mi::EpiJS<true>>(ma, mbk, sc, ep, stream));
+    } else {
+      std::memset(&ep.tmap_p, 0, sizeof(ep.tmap_p));
+      MI_TRY(launch_engine<mi::EpiJS<false>>(ma, mbk, sc, ep, stream));
+    }
+    js_rows_kernel<<<blocks_for(rows, 128), 128, 0, stream>>>(part, sc.n_split * mi::kColQuarters, rows_padded, static_cast<int>(rows),
+                                                              mb.n_same + r0, static_cast<int>(B), diag + r0,
+                                                              reinterpret_cast<float4*>(row_out) + r0);
+    MI_LAUNCH_CHECK("js_rows_kernel");
+    if (r0 + panel_rows >= B) {
+      js_reduce_kernel<<<1, kJsRedThreads, 0, stream>>>(reinterpret_cast<const float4*>(row_out), B, scal_out);
+      MI_LAUNCH_CHECK("js_reduce_kernel");
+    }
+    if (!grads) continue;
+    // (2) ok_raw += P^T Q[panel]: contraction over the panel rows, P read MN-major
+    if (ok_raw) {
+      GemmArgs g;
+      const int kr = static_cast<int>(cdiv(rows, bk()));
+      g.a_mn = true;
+      g.a = MapSpec{P, rows, pitch, pitch};
+      g.b_mn = true; g.b = MapSpec{Q.p + r0 * Q.ld, rows, q_hl ? Dp + D : D, Q.ld};
+      g.M = B; g.N = D; g.seg_len = kr; g.k_blocks = kr;
+      if (strict) {                                  // P_hi^T Q_hi + P_lo^T Q_hi (+ P_hi^T Q_lo)
+        g.k_blocks = 2 * kr; g.a_moff[1] = static_cast<int>(k_pad);
+        if (q_hl) { g.k_blocks = 3 * kr; g.b_noff[2] = static_cast<int>(Dp); }
+      }
+      g.accumulate = r0 > 0;
+      g.out_f32 = ok_raw; g.ld_out = D;
+      MI_TRY(run_gemm(g, none, stream));
+    }
+    // (3) oq_raw[panel] = P K
+    if (oq_raw) {
+      GemmArgs g;
+      g.a = MapSpec{P, rows, pitch, pitch};
+      g.b_mn = true; g.b = MapSpec{K.p, B, k_hl ? Dp + D : D, K.ld};
+      g.M = rows; g.N = D; g.seg_len = kp; g.k_blocks = kp;
+      if (strict) {
+        g.k_blocks = 2 * kp; g.a_seg[1] = kp;
+        if (k_hl) { g.k_blocks = 3 * kp; g.b_noff[2] = static_cast<int>(Dp); }
+      }
+      g.out_f32 = oq_raw + r0 * D; g.ld_out = D;
+      g.ksplit = oq_ksplit;
+      Bump kws(kpart, kpart_elems * sizeof(float), false);
+      MI_TRY(run_gemm(g, oq_ksplit > 1 ? kws : none, stream));
+    }
+  }
+  return MI_OK;
+}
+
 inline bool single_pass_estimator(int estimator, int precision) {
   return estimator != MI_EST_INFONCE_SYM && (precision & MI_PREC_TWO_PASS) == 0;
 }
@@ -1706,19 +1900,22 @@ int critic_impl(const void* X_, const void* Y_, const void* W_, const int* sid, 
                 const std::function<int(long long, long long)>* x_ready = nullptr,  // single pass only: X rows arrive per panel
                 const Fallback& fb = Fallback()) {
   if (B <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
-  if (estimator < MI_EST_DV || estimator > MI_EST_INFONCE_SYM) return MI_ERR_BAD_ARG;
+  if (estimator < MI_EST_DV || estimator > MI_EST_NWJ) return MI_ERR_BAD_ARG;
   typedef __nv_bfloat16 bf;
   const bf* X = static_cast<const bf*>(X_); const bf* Y = static_cast<const bf*>(Y_); const bf* W = static_cast<const bf*>(W_);
   const bool bilinear = critic == MI_CRITIC_BILINEAR;
   const bool grads = dX != nullptr || dY != nullptr || dW != nullptr;
   const bool plan = ws.dry || grads;
   const bool sym = estimator == MI_EST_INFONCE_SYM;
-  const bool dv_like = estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF;
+  const bool js = estimator == MI_EST_JS;           // its own pass (js_pass_impl): no references, no guard
+  // NWJ is DV with another final scalar (see loss_finalize_kernel): the same passes, references and guard
+  const bool dv_like = estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF || estimator == MI_EST_NWJ;
   const bool strict = (precision & 1) == MI_PREC_BF16_STRICT;
   // one score computation instead of two (see single_pass_impl); the symmetric estimator needs exact column statistics
   // before its gradient pass and stays on the statistics-pass + gradient-pass path.  MI_PREC_TWO_PASS asks for exact
   // references (stride 1) in the single pass: the same statistics, then the pass can never trip its guard.
-  const bool single = !sym && (grads || ws.dry);
+  const bool single = !sym && !js && (grads || ws.dry);
+  const bool js_grads = js && plan;
   const bool exact_refs = (precision & MI_PREC_TWO_PASS) != 0;
   const int tsplit = (bilinear && strict) ? 2 : 1;        // T = X W kept as a hi/lo bf16 pair in strict mode
   const long long Dp = round_up(D, kSplitAlign);
@@ -1732,24 +1929,24 @@ int critic_impl(const void* X_, const void* Y_, const void* W_, const int* sid, 
   float* ref_r = ws.take<float>(B);
   float* ref_c = sym ? ws.take<float>(B) : nullptr;
   bf* dT16 = (bilinear && plan) ? ws.take<bf>(static_cast<size_t>(B) * ldT) : nullptr;
-  float* sp_diag = single ? ws.take<float>(B) : nullptr;
+  float* sp_diag = (single || js) ? ws.take<float>(B) : nullptr;
   float* sp_wrow = single ? ws.take<float>(B) : nullptr;
   float* sp_lambda = single ? ws.take<float>(1) : nullptr;
   int* sp_flags = single ? ws.take<int>(4) : nullptr;     // [0] rows tripped (sampled pass), [1] fallback predicate, [2] rows tripped (repeat)
   double* sp_guard = single ? ws.take<double>(1) : nullptr;
-  float* sp_oq = (single && (bilinear || !dX)) ? ws.take<float>(static_cast<size_t>(B) * D) : nullptr;   // dot: dX doubles as the raw buffer
-  float* sp_ok = (single && !dY) ? ws.take<float>(static_cast<size_t>(B) * D) : nullptr;
+  float* sp_oq = ((single || js_grads) && (bilinear || !dX)) ? ws.take<float>(static_cast<size_t>(B) * D) : nullptr;   // dot: dX doubles as the raw buffer
+  float* sp_ok = ((single || js_grads) && !dY) ? ws.take<float>(static_cast<size_t>(B) * D) : nullptr;
   // the negatives mask of the whole batch: built ONCE per call and shared by the exact reference pass and the single pass(es)
   const long long k_pad_all = cdiv(B, mi::TILE_N) * mi::TILE_N;
   MaskBuf all_mask{};
-  if (single) all_mask = take_mask(ws, B, k_pad_all, B);
+  if (single || js) all_mask = take_mask(ws, B, k_pad_all, B);
   if (!ws.ok()) return MI_ERR_WORKSPACE;
   if (!ws.dry && (!X || !Y || !sid || !loss_out || (bilinear && !W))) return MI_ERR_BAD_ARG;
 
   const Opnd Xo{X, D, 1}, Yo{Y, D, 1};
   const Opnd To = bilinear ? Opnd{T, ldT, tsplit} : Xo;
   size_t mk = ws.mark();
-  const bool streamed = x_ready != nullptr && single && !ws.dry;
+  const bool streamed = x_ready != nullptr && (single || js_grads) && !ws.dry;
   Bump none(nullptr, 0, false);
   // T[r0 : r0 + rows] = X[r0 : r0 + rows] W  (B operand of the engine is [N, K] = W^T: W itself read MN-major)
   auto project = [&](long long r0, long long rows, Bump& w) -> int {
@@ -1842,7 +2039,54 @@ int critic_impl(const void* X_, const void* Y_, const void* W_, const int* sid, 
       MI_TRY(run_pass(1, sp_flags, false));
     }
   }
-  if (!single || ws.dry) {        // statistics pass(es) + gradient pass with exact references (planning covers both paths)
+  if (js) {
+    if (!ws.dry) MI_TRY(build_mask(all_mask, sid, sid, B, B, k_pad_all, stream));
+    // S_ii: one O(B D) row-dot kernel (per panel when the image embeddings arrive panel by panel)
+    auto diag_rows = [&](long long r0, long long rows) -> int {
+      diag_kernel<<<blocks_for(rows * 32, 256), 256, 0, stream>>>(To.p + r0 * To.ld, To.ld, To.split, Y, D, 1, r0, rows, D, Dp,
+                                                                   inv_tau, sp_diag + r0, nullptr);
+      MI_LAUNCH_CHECK("diag_kernel");
+      return MI_OK;
+    };
+    PanelFeed feed;
+    if (streamed) {
+      feed.before_panel = [&](long long r0, long long rows) -> int {
+        MI_TRY((*x_ready)(r0, rows));
+        if (bilinear) MI_TRY(project(r0, rows, none));
+        return diag_rows(r0, rows);
+      };
+    } else if (!ws.dry) {
+      MI_TRY(diag_rows(0, B));
+    }
+    float* oq_raw = js_grads ? (sp_oq ? sp_oq : dX) : nullptr;
+    float* ok_raw = js_grads ? (dY ? dY : sp_ok) : nullptr;
+    MI_TRY(js_pass_impl(To, Yo, sid, B, D, inv_tau, precision, sp_diag, rows_r, scal_r, oq_raw, ok_raw, all_mask, ws, stream,
+                        streamed ? &feed : nullptr));
+    ws.release(mk);
+    if (!ws.dry) {
+      loss_finalize_kernel<<<1, 32, 0, stream>>>(scal_r, nullptr, B, estimator, loss_out, lse_f, nullptr, nullptr);   // lse_f = 1 / N_neg
+      MI_LAUNCH_CHECK("loss_finalize_kernel");
+    }
+    if (!ws.dry && js_grads) {
+      const float inv_b = 1.f / static_cast<float>(B);
+      // dY = inv_tau (P^T T / N_neg - sigma(-S_kk) T_k / B), in place
+      if (dY) {
+        js_finalize_kernel<<<blocks_capped(B * D / 8, 256), 256, 0, stream>>>(dY, D, B, lse_f, sp_diag, inv_b, inv_tau, To.p, To.ld,
+                                                                            To.split, Dp, dY, nullptr, nullptr, 0);
+        MI_LAUNCH_CHECK("js_finalize_kernel");
+        if (ev_dy_final) {
+          MI_CUDA(cudaEventRecord(ev_dy_final, stream));
+          if (ev_recorded) *ev_recorded = true;
+        }
+      }
+      // dT = inv_tau (P Y / N_neg - sigma(-S_qq) Y_q / B): fp32 (dot critic: this is dX) or the bf16 (hi/lo) operand of dX / dW
+      if (bilinear ? (dX || dW) : dX != nullptr) js_finalize_kernel<<<blocks_capped(B * D / 8, 256), 256, 0, stream>>>(oq_raw, D, B, lse_f, sp_diag, inv_b, inv_tau, Y, D, 1, Dp,
+                                                                          bilinear ? nullptr : dX, bilinear ? dT16 : nullptr,
+                                                                          (bilinear && tsplit == 2) ? dT16 + Dp : nullptr, ldT);
+      MI_LAUNCH_CHECK("js_finalize_kernel");
+    }
+  }
+  if ((!single || ws.dry) && !js) {        // statistics pass(es) + gradient pass with exact references (planning covers both paths)
     if (sym) {      // rows and columns from one score computation
       MI_TRY(stats_rc_impl(To, Yo, sid, sid, 0, B, B, D, inv_tau, rows_r, scal_r, rows_c, scal_c, nullptr, ws, stream));
     } else {

@@ -14,7 +14,9 @@ import torch
 from . import _lib
 
 CRITIC = {"dot": 0, "bilinear": 1}
-ESTIMATOR = {"dv": 0, "infonce": 1, "infonce_ref": 1, "infonce_row": 2, "infonce_sym": 3}
+ESTIMATOR = {"dv": 0, "infonce": 1, "infonce_ref": 1, "infonce_row": 2, "infonce_sym": 3, "js": 4, "nwj": 5}
+# the f-divergence bounds run on the single-GPU separable critics only (dot / bilinear, critic_loss_fwd_bwd)
+SEPARABLE_ONLY = ("js", "nwj")
 PRECISION = {"fast": 0, "strict": 1}
 
 
@@ -495,6 +497,7 @@ def sharded_step(X_local: torch.Tensor, Y_local: torch.Tensor, W: Optional[torch
     """mi_sharded_critic_loss_fwd_bwd: the whole batch-sharded step (collectives included) as one library call, for every
     estimator.  Returns (status, loss_out fp64[8], dX, dY, dW); status GUARD_TRIPPED (on every rank alike) means the outputs
     are not valid and the step must be repeated on the exact path ("infonce_sym" uses exact statistics: always 0)."""
+    reject_separable_only(estimator, "the batch-sharded step")
     _need_cuda(X_local, Y_local, W, sid_local)
     lib = _lib.load()
     ctx, rank, world, _ = dist_context(group)
@@ -575,6 +578,7 @@ def mlp_critic_loss_fwd_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid: torch
     (mi_mlp_critic_loss_fwd_bwd).  ``params`` = (W1 [H1,2D], b1, W2 [H2,H1], b2, W3 [1,H2], b3) fp32.
     Returns (loss_out fp64[8], S or None, grads dict with keys dX, dY, dW1 ... db3 (or None)); loss_out[4] / [5] are the
     row / column losses of infonce_sym."""
+    reject_separable_only(estimator, "the MLP critic")
     _need_cuda(X, Y, sid, *params)
     lib = _lib.load()
     f32 = lambda t: t.detach().to(torch.float32).contiguous()
@@ -639,9 +643,19 @@ def _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev):
     return workspace(nbytes, dev)
 
 
+def reject_separable_only(estimator: str, what: str) -> None:
+    """Raise before any launch when ``estimator`` runs only on the single-GPU separable critics."""
+    if estimator in SEPARABLE_ONLY:
+        supported = ", ".join(e for e in ESTIMATOR if e not in SEPARABLE_ONLY)
+        raise MIError(f"estimator {estimator!r} is not implemented for {what}: supported are {supported} "
+                      f"({' and '.join(SEPARABLE_ONLY)} run on the single-GPU dot / bilinear critics)")
+
+
 def _mlp_estimator(estimator):
+    reject_separable_only(estimator, "the MLP critic")
     if estimator not in ESTIMATOR:
-        raise MIError(f"unknown estimator {estimator!r}: the MLP critic supports {', '.join(ESTIMATOR)}")
+        raise MIError(f"unknown estimator {estimator!r}: the MLP critic supports "
+                      f"{', '.join(e for e in ESTIMATOR if e not in SEPARABLE_ONLY)}")
     return ESTIMATOR[estimator]
 
 
