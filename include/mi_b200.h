@@ -58,9 +58,13 @@ enum mi_estimator { MI_EST_DV = 0, MI_EST_INFONCE_REF = 1, MI_EST_INFONCE_ROW = 
 
 enum mi_precision { MI_PREC_BF16_FAST = 0,   /* dS panel rounded once to bf16 */
                     MI_PREC_BF16_STRICT = 1, /* dS = hi + lo bf16 split (fp32-accumulate mode) */
-                    MI_PREC_TWO_PASS = 2     /* flag (OR it in): exact softmax references (a statistics pass over EVERY
+                    MI_PREC_TWO_PASS = 2,    /* flag (OR it in): exact softmax references (a statistics pass over EVERY
                                                 column before the gradient pass) instead of sampled ones
-                                                (mi_critic_loss_fwd_bwd) */ };
+                                                (mi_critic_loss_fwd_bwd) */
+                    MI_PREC_FP32X3 = 4       /* MLP-critic entries only ("fp32"): every operand as three bf16 pieces
+                                                p0 = RN(x), p1 = RN(x - p0), p2 = RN(x - p0 - p1) (24 significant bits),
+                                                six K segments, accumulation chains of <= 8192 K elements; the separable,
+                                                sharded, host-buffer and GDV entries reject it (MI_ERR_BAD_ARG / size 0) */ };
 
 const char* mi_status_string(int status);
 const char* mi_last_cuda_error(void);
@@ -312,8 +316,10 @@ int mi_sharded_critic_loss_fwd_bwd(mi_dist_ctx* ctx, const void* X_local, const 
  * device, in nn.Linear layout:  W1 [H1, 2D] (columns [0,D) act on the image embedding, [D,2D) on the text
  * embedding), b1 [H1], W2 [H2, H1], b2 [H2], W3 [1, H2], b3 [1].   D, H1, H2 multiples of 8, H2 <= 512.
  * estimator: MI_EST_DV, MI_EST_INFONCE_REF, MI_EST_INFONCE_ROW or MI_EST_INFONCE_SYM.  precision: MI_PREC_BF16_FAST
- * (bf16 operands of the tensor-core contractions, fp32 accumulate) or MI_PREC_BF16_STRICT (hi/lo bf16 pairs, 16
- * significant bits).  loss_out (fp64[8]) as mi_critic_loss_fwd_bwd (slot 4 = loss_row, slot 5 = loss_col of
+ * (bf16 operands of the tensor-core contractions, fp32 accumulate), MI_PREC_BF16_STRICT (hi/lo bf16 pairs, 16
+ * significant bits) or MI_PREC_FP32X3 (three bf16 pieces, 24 significant bits: ReLU masks flip as rarely as in an fp32
+ * computation; row panels of 2/3 of mi_set_mlp_panel_pairs; D and H1 <= 1280 so that every contraction that feeds an
+ * epilogue stays one bounded chain — size 0 / MI_ERR_BAD_ARG otherwise; any other value is rejected).  loss_out (fp64[8]) as mi_critic_loss_fwd_bwd (slot 4 = loss_row, slot 5 = loss_col of
  * MI_EST_INFONCE_SYM).  dv / infonce with gradients run as a single pass (softmax weights against
  * the maximum logit of a sample of pairs, Z2 formed once; see mi_set_mlp_mode); if its guard trips, the two-pass sequence
  * repeats the step behind a device-side predicate and loss_out[7] > 0 reports it.  infonce_row and infonce_sym always run

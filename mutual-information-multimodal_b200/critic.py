@@ -233,6 +233,7 @@ class FusedCritic(nn.Module):
         super().__init__()
         if critic not in ("dot", "bilinear"):
             raise ValueError("critic must be 'dot' or 'bilinear'")
+        ops._precision(precision)          # "fast" / "strict" ("fp32" is the MLP critic's only): raises before any launch
         self.dim = dim
         self.critic = critic
         self.precision = precision
@@ -295,6 +296,7 @@ class FusedMLPCritic(nn.Sequential):
         if len(hidden_dims) != 2:
             raise ValueError("the fused path implements the reference's two-hidden-layer critic")
         h1, h2 = int(hidden_dims[0]), int(hidden_dims[1])
+        ops._mlp_precision(precision)      # "fast", "strict" or "fp32" (three bf16 pieces per operand)
         super().__init__(nn.Linear(2 * dim, h1), nn.ReLU(), nn.Linear(h1, h2), nn.ReLU(), nn.Linear(h2, 1))
         self.dim = dim
         self.precision = precision

@@ -50,7 +50,12 @@ struct Cfg {
 
 // Work decomposition.  A "unit" is (m block, N-range split, K split); a CTA (pair) walks units
 // u = pair, pair + n_pairs, ... and inside a unit walks its N tiles, each over its K blocks.
-struct Sched {
+// kSegs: the length of the K-segment table.  Host code plans with Sched (six entries); the fast / strict kernels take
+// SchedT<4> — the kernel parameter of the parent layout, so their register allocation is unchanged — and only the
+// MLP critic's fp32 mode (six segments) launches kernels that take the six-entry table.
+constexpr int kMaxSegs = 6;
+template <int kSegs>
+struct SchedT {
   int n_mblk;     // M blocks of 128*kCG rows
   int n_ntile;    // N tiles of 256 columns
   int n_split;    // contiguous N-range splits per M block
@@ -61,12 +66,13 @@ struct Sched {
   int k_blocks;   // number of K blocks (block_k wide) per tile, all segments
   // K segments: block kb belongs to segment kb / seg_len and reads A at K block a_seg[seg] + kb % seg_len,
   // B at b_seg[seg] + kb % seg_len.  One segment = plain GEMM; more = sums of products of hi/lo splits,
-  // e.g. [P_hi | P_lo] x [V ; V] or [T_hi | T_lo] x [Y ; Y] (fp32-accumulate "strict" mode).
+  // e.g. [P_hi | P_lo] x [V ; V] or [T_hi | T_lo] x [Y ; Y] (fp32-accumulate "strict" mode), or the six terms of two
+  // three-piece operands (the MLP critic's fp32 mode).
   int seg_len;
-  int a_seg[4];
-  int b_seg[4];
-  int a_moff[4];  // MN-major A only: M-coordinate offset of the segment (e.g. the lo half of a [hi | lo] panel)
-  int b_noff[4];  // MN-major B only: N-coordinate offset of the segment
+  int a_seg[kSegs];
+  int b_seg[kSegs];
+  int a_moff[kSegs];  // MN-major A only: M-coordinate offset of the segment (e.g. the lo half of a [hi | lo] panel)
+  int b_noff[kSegs];  // MN-major B only: N-coordinate offset of the segment
   // Device-side launch predicate: when non-null and *run_if == 0 the whole grid returns at once.  The exact
   // fallback of the single pass is enqueued behind such a flag, so it costs a few empty launches unless needed.
   const int* run_if;
@@ -76,17 +82,23 @@ struct Sched {
   // every il and can sum over il in registers (EpiMlpDa).
   int grp, chunk_len, n_chunks, n_il;
 };
+using Sched = SchedT<kMaxSegs>;
 
 // A unit's work items: item `it` is the accumulator tile (M block m + it * m_step, N tile nt0 + it * nt_step).
 struct Unit { int m, s, ks, nt0, nt1, kb0, kb1, n_items, m_step, nt_step; };
 
-__host__ __device__ __forceinline__ int num_units(const Sched& sc) {
+template <int kSegs>
+__host__ __device__ __forceinline__ int num_units(const SchedT<kSegs>& sc) {
   return sc.order == 2 ? sc.n_ntile * sc.grp * sc.n_chunks : sc.n_mblk * sc.n_split * sc.n_ksplit;
 }
-__device__ __forceinline__ int sel4(const int (&a)[4], int i) { return i == 0 ? a[0] : i == 1 ? a[1] : i == 2 ? a[2] : a[3]; }
+template <int kSegs>
+__device__ __forceinline__ int sel_seg(const int (&a)[kSegs], int i) {
+  if constexpr (kSegs == 4) return i == 0 ? a[0] : i == 1 ? a[1] : i == 2 ? a[2] : a[3];
+  else return i == 0 ? a[0] : i == 1 ? a[1] : i == 2 ? a[2] : i == 3 ? a[3] : i == 4 ? a[4] : a[5];
+}
 
-template <bool kWalk>
-__host__ __device__ __forceinline__ Unit decode_unit(const Sched& sc, int u) {
+template <bool kWalk, int kSegs>
+__host__ __device__ __forceinline__ Unit decode_unit(const SchedT<kSegs>& sc, int u) {
   Unit r;
   if (kWalk && sc.order == 2) {
     const int nt = u % sc.n_ntile; int t = u / sc.n_ntile;      // the N tiles of an M block run concurrently (A tile from L2)
@@ -118,10 +130,10 @@ __host__ __device__ __forceinline__ Unit decode_unit(const Sched& sc, int u) {
 // 64-wide M half the K rows are contiguous — and described to the MMA with the MN-major SWIZZLE_128B
 // canonical layout (LBO = bytes between the M halves, SBO = 1 KB between 8-row K groups).
 // kBMN: the same for the B operand (B[n,k] at base[k*ld + n]): per 64-wide N group the K rows are contiguous.
-template <int kCG, class Epi, bool kAMN, bool kBMN>
+template <int kCG, class Epi, bool kAMN, bool kBMN, int kSegs>
 __global__ void __launch_bounds__(kNumThreads, 1)
 tile_engine_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-                   const Sched sc, const __grid_constant__ typename Epi::Params ep) {
+                   const SchedT<kSegs> sc, const __grid_constant__ typename Epi::Params ep) {
   using C = Cfg<kCG>;
   if (sc.run_if != nullptr && *sc.run_if == 0) return;      // grid-uniform: both CTAs of a pair leave together
   extern __shared__ uint8_t smem_raw[];
@@ -179,9 +191,9 @@ tile_engine_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
         const int a_row = ((Epi::kWalk ? un.m + it * un.m_step : un.m) * kCG + (int)cta_rank) * BLOCK_M;
         const int b_row = (Epi::kWalk ? un.nt0 : un.nt0 + it) * TILE_N + (int)cta_rank * C::kBRows;
         int seg = un.kb0 / sc.seg_len, w = un.kb0 - seg * sc.seg_len;
-        int a_k = (sel4(sc.a_seg, seg) + w) * C::kBK, b_k = (sel4(sc.b_seg, seg) + w) * C::kBK;
-        int a_m = a_row + sel4(sc.a_moff, seg);
-        int b_n = b_row + sel4(sc.b_noff, seg);
+        int a_k = (sel_seg(sc.a_seg, seg) + w) * C::kBK, b_k = (sel_seg(sc.b_seg, seg) + w) * C::kBK;
+        int a_m = a_row + sel_seg(sc.a_moff, seg);
+        int b_n = b_row + sel_seg(sc.b_noff, seg);
         for (int kb = un.kb0; kb < un.kb1; ++kb) {
           ptx::mbar_wait_addr(empty0 + stage * 8u, phase ^ 1u, 1);
           if (lane == 0) {
@@ -211,8 +223,8 @@ tile_engine_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
           a_k += C::kBK; b_k += C::kBK;
           if (++w == sc.seg_len) {
             w = 0; ++seg;
-            a_k = sel4(sc.a_seg, seg) * C::kBK; b_k = sel4(sc.b_seg, seg) * C::kBK; a_m = a_row + sel4(sc.a_moff, seg);
-            b_n = b_row + sel4(sc.b_noff, seg);
+            a_k = sel_seg(sc.a_seg, seg) * C::kBK; b_k = sel_seg(sc.b_seg, seg) * C::kBK; a_m = a_row + sel_seg(sc.a_moff, seg);
+            b_n = b_row + sel_seg(sc.b_noff, seg);
           }
           if (++stage == (uint32_t)C::kStages) { stage = 0; phase ^= 1u; }
         }
@@ -1038,23 +1050,27 @@ struct EpiMlpFwd {
 // ---- backward through layer 3 / ReLU 2:  dZ2[pair, n] = g[pair] w3[n] [Z2 + b2 > 0]  (bf16 hi [+ lo]) for the
 //      dW2 / dH1 contractions;  dw3[n] += sum_pairs g relu(Z2 + b2),  db2[n] += sum_pairs dZ2  (column sums over
 //      the warp's rows, kept per lane across the whole launch, one atomicAdd per column at the end).
-struct EpiMlpDz {
+struct EpiMlpDzParams {
+  const float* b2;       // [n_ntile * 256] zero padded
+  const float* w3;       // [n_ntile * 256] zero padded
+  const float* g;        // [rows] dL/dlogit of the pair
+  int rows, cols;
+  __nv_bfloat16* dz;     // [rows, pitch]
+  __nv_bfloat16* dz_lo;  // residual half (strict), second piece (fp32 mode) or nullptr
+  __nv_bfloat16* dz_lo2; // third piece (fp32 mode) or nullptr
+  long long pitch;
+  float* dw3;            // [n_ntile * 256] accumulators (atomicAdd)
+  float* db2;
+};
+// kThird: fp32 mode (three-piece dZ2 stores); the fast / strict instantiation carries none of that code
+template <bool kThird>
+struct EpiMlpDzT {
   static constexpr bool kJoint = false;
   static constexpr bool kWalk = false;
   static constexpr bool kChunk16 = false;
   static constexpr int kEpiSmemBytes = 0;
   static constexpr int kMaxTiles = 2;       // H2 <= 512
-  struct Params {
-    const float* b2;       // [n_ntile * 256] zero padded
-    const float* w3;       // [n_ntile * 256] zero padded
-    const float* g;        // [rows] dL/dlogit of the pair
-    int rows, cols;
-    __nv_bfloat16* dz;     // [rows, pitch]
-    __nv_bfloat16* dz_lo;  // residual half (strict) or nullptr
-    long long pitch;
-    float* dw3;            // [n_ntile * 256] accumulators (atomicAdd)
-    float* db2;
-  };
+  using Params = EpiMlpDzParams;
   struct State { uint8_t* stage_smem; float g; float sw[kMaxTiles][2]; float sb[kMaxTiles][2]; };
   static __device__ __forceinline__ void init(const Params&, State& st) {
 #pragma unroll
@@ -1108,6 +1124,26 @@ struct EpiMlpDz {
           for (int c = 0; c < 32; ++c)
             if (col0 + c < p.cols) dl[c] = __float2bfloat16(dz[c] - __bfloat162float(__float2bfloat16(dz[c])));
         }
+        if (kThird && p.dz_lo2 != nullptr) {          // fp32 mode: the third piece (dz - hi) - lo, both differences exact
+          __nv_bfloat16* d2 = p.dz_lo2 + (size_t)row * p.pitch + col0;
+          if (full) {
+            uint32_t l2[16];
+#pragma unroll
+            for (int c = 0; c < 16; ++c) {
+              const float r0 = dz[2 * c] - __uint_as_float(hi[c] << 16), r1 = dz[2 * c + 1] - __uint_as_float(hi[c] & 0xffff0000u);
+              l2[c] = ptx::pack_bf16(r0 - __uint_as_float(lo[c] << 16), r1 - __uint_as_float(lo[c] & 0xffff0000u));
+            }
+            uint4* d4 = reinterpret_cast<uint4*>(d2);
+#pragma unroll
+            for (int g = 0; g < 4; ++g) d4[g] = make_uint4(l2[4 * g], l2[4 * g + 1], l2[4 * g + 2], l2[4 * g + 3]);
+          } else {
+            for (int c = 0; c < 32; ++c)
+              if (col0 + c < p.cols) {
+                const float r = dz[c] - __bfloat162float(__float2bfloat16(dz[c]));
+                d2[c] = __float2bfloat16(r - __bfloat162float(__float2bfloat16(r)));
+              }
+          }
+        }
       }
     }
     // column sums over this warp's 32 pairs (rows beyond p.rows carry g = 0)
@@ -1138,6 +1174,8 @@ struct EpiMlpDz {
       }
   }
 };
+using EpiMlpDz = EpiMlpDzT<false>;
+using EpiMlpDz3 = EpiMlpDzT<true>;
 
 // ---- single pass (dv-like estimators): forward AND the backward through layer 3 / ReLU 2 from ONE Z2 accumulator.
 //      The softmax weights of the negatives are taken relative to a reference logit `ref` that is fixed BEFORE the
@@ -1151,32 +1189,36 @@ struct EpiMlpDz {
 //      second pass is EpiMlpDz's chunk with that g~.
 constexpr float kMlpSpScale = 1.6940658945086007e-21f;    // 2^-69: g~ = e^{S - max_sample} 2^-69
 constexpr double kMlpSpMargin = 47.82715406979468;        // 69 ln 2
-struct EpiMlpSp {
+struct EpiMlpSpParams {
+  const float* b2;       // [n_ntile * 256] zero padded
+  const float* w3;       // [n_ntile * 256] zero padded
+  const float* b3;       // [1]
+  const float* ref;      // [1] maximum logit of the sample (the reference logit is this + kMlpSpMargin)
+  const int* sid_q;      // [rows] study ids of the image rows (negatives: sid_q[i] != sid_k[j], main_utils.py:105)
+  const int* sid_k;      // [B] study ids of the text rows
+  int B, Bp, r0, rr;     // text rows, padded text rows, first image row of the panel, image rows in the panel
+  int q_off;             // global index of local image row 0
+  int cols;              // H2
+  __nv_bfloat16* dz;     // [rr * Bp, pitch]  g~ w3 [Z2 + b2 > 0]
+  __nv_bfloat16* dz_lo;  // residual half (strict), second piece (fp32 mode) or nullptr
+  __nv_bfloat16* dz_lo2; // third piece (fp32 mode) or nullptr
+  long long pitch;
+  float* dw3;            // [n_ntile * 256] accumulators (atomicAdd), in g~ units
+  float* db2;
+  float* rowsum;         // [rows] += sum_j g~          (atomicAdd)
+  float* rowcnt;         // [rows] += number of negatives of the row
+  float* diag_out;       // [rows] logit of the positive pair
+  float* S_out;          // optional [rows, B]: every logit
+};
+// kThird: fp32 mode (three-piece dZ2 stores); the fast / strict instantiation carries none of that code
+template <bool kThird>
+struct EpiMlpSpT {
   static constexpr bool kJoint = true;
   static constexpr bool kWalk = false;
   static constexpr bool kChunk16 = false;
   static constexpr int kEpiSmemBytes = 2 * kColQuarters * BLOCK_M * 4;     // 2 slots x [4 column quarters][128 rows] fp32
   static constexpr int kMaxTiles = 2;       // H2 <= 512
-  struct Params {
-    const float* b2;       // [n_ntile * 256] zero padded
-    const float* w3;       // [n_ntile * 256] zero padded
-    const float* b3;       // [1]
-    const float* ref;      // [1] maximum logit of the sample (the reference logit is this + kMlpSpMargin)
-    const int* sid_q;      // [rows] study ids of the image rows (negatives: sid_q[i] != sid_k[j], main_utils.py:105)
-    const int* sid_k;      // [B] study ids of the text rows
-    int B, Bp, r0, rr;     // text rows, padded text rows, first image row of the panel, image rows in the panel
-    int q_off;             // global index of local image row 0
-    int cols;              // H2
-    __nv_bfloat16* dz;     // [rr * Bp, pitch]  g~ w3 [Z2 + b2 > 0]
-    __nv_bfloat16* dz_lo;  // residual half (strict) or nullptr
-    long long pitch;
-    float* dw3;            // [n_ntile * 256] accumulators (atomicAdd), in g~ units
-    float* db2;
-    float* rowsum;         // [rows] += sum_j g~          (atomicAdd)
-    float* rowcnt;         // [rows] += number of negatives of the row
-    float* diag_out;       // [rows] logit of the positive pair
-    float* S_out;          // optional [rows, B]: every logit
-  };
+  using Params = EpiMlpSpParams;
   struct State { uint8_t* stage_smem; float acc; float g; int slot; float sw[kMaxTiles][2]; float sb[kMaxTiles][2]; };
   static __device__ __forceinline__ void init(const Params&, State& st) {
     st.slot = 0;
@@ -1276,6 +1318,26 @@ struct EpiMlpSp {
           for (int c = 0; c < 16; ++c)
             if (col0 + c < p.cols) dl[c] = __float2bfloat16(dz[c] - __bfloat162float(__float2bfloat16(dz[c])));
         }
+        if (kThird && p.dz_lo2 != nullptr) {          // fp32 mode: the third piece (dz - hi) - lo, both differences exact
+          __nv_bfloat16* d2 = p.dz_lo2 + (size_t)row * p.pitch + col0;
+          if (full) {
+            uint32_t l2[8];
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+              const float r0 = dz[2 * c] - __uint_as_float(hi[c] << 16), r1 = dz[2 * c + 1] - __uint_as_float(hi[c] & 0xffff0000u);
+              l2[c] = ptx::pack_bf16(r0 - __uint_as_float(lo[c] << 16), r1 - __uint_as_float(lo[c] & 0xffff0000u));
+            }
+            uint4* d4 = reinterpret_cast<uint4*>(d2);
+#pragma unroll
+            for (int g = 0; g < 2; ++g) d4[g] = make_uint4(l2[4 * g], l2[4 * g + 1], l2[4 * g + 2], l2[4 * g + 3]);
+          } else {
+            for (int c = 0; c < 16; ++c)
+              if (col0 + c < p.cols) {
+                const float r = dz[c] - __bfloat162float(__float2bfloat16(dz[c]));
+                d2[c] = __float2bfloat16(r - __bfloat162float(__float2bfloat16(r)));
+              }
+          }
+        }
       }
     }
     // column sums over this warp's 32 pairs; a warp whose rows are all excluded (g~ = 0) has nothing to add.
@@ -1307,6 +1369,8 @@ struct EpiMlpSp {
       }
   }
 };
+using EpiMlpSp = EpiMlpSpT<false>;
+using EpiMlpSp3 = EpiMlpSpT<true>;
 
 // ---- backward through ReLU 1 with both reductions fused:  dZ1 = (dZ2 W2) . [H > 0]  is never stored;
 //      dA[i, k] += sum_j dZ1[(i, j), k]  (column sums over the warp's 32 rows: one image row per M block) and

@@ -76,6 +76,7 @@ __global__ void gdv_finalize_kernel(const double* __restrict__ sums, long long N
 int gdv_impl(const float* pos, const float* neg, long long Np, long long Nn, long long D, int precision, double* out,
              Bump& ws, cudaStream_t stream) {
   if (Np <= 1 || Nn <= 1 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
+  if (precision & MI_PREC_FP32X3) return MI_ERR_BAD_ARG;     // three-piece operands: the MLP critic only
   typedef __nv_bfloat16 bf;
   const int sp = (precision & 1) == MI_PREC_BF16_STRICT ? 2 : 1;
   const long long Dp = round_up(D, kSplitAlign), pitch = sp == 2 ? 2 * Dp : D, ext = sp == 2 ? Dp + D : D;

@@ -166,8 +166,30 @@ struct MapSpec {          // a 2-D bf16 tensor map: `rows` x `k_extent` elements
   const void* ptr; long long rows, k_extent, ld;
 };
 
-template <int kCG, class Epi, bool kAMN, bool kBMN>
-int launch_engine_cg(const MapSpec& a, const MapSpec& b, const Sched& sc, const typename Epi::Params& ep, cudaStream_t stream) {
+// The K-segment tables an epilogue is instantiated for (bit 0: four entries, bit 1: six).  Most epilogues serve fast /
+// strict only; the MLP critic's fp32 mode (six segments) runs EpiMlpFwd, EpiMlpDa and EpiStore with six, and the
+// three-piece dZ2 epilogues with six only.
+template <class Epi> struct EpiSegTables { static constexpr int value = 1; };
+template <> struct EpiSegTables<mi::EpiMlpFwd> { static constexpr int value = 3; };
+template <> struct EpiSegTables<mi::EpiMlpDa> { static constexpr int value = 3; };
+template <> struct EpiSegTables<mi::EpiStore> { static constexpr int value = 3; };
+template <> struct EpiSegTables<mi::EpiMlpDz3> { static constexpr int value = 2; };
+template <> struct EpiSegTables<mi::EpiMlpSp3> { static constexpr int value = 2; };
+
+// the host schedule with the first kSegs entries of its segment table
+template <int kSegs>
+mi::SchedT<kSegs> sched_with_table(const Sched& sc) {
+  mi::SchedT<kSegs> r;
+  r.n_mblk = sc.n_mblk; r.n_ntile = sc.n_ntile; r.n_split = sc.n_split; r.n_ksplit = sc.n_ksplit; r.nt_base = sc.nt_base;
+  r.order = sc.order; r.k_blocks = sc.k_blocks; r.seg_len = sc.seg_len;
+  for (int i = 0; i < kSegs; ++i) { r.a_seg[i] = sc.a_seg[i]; r.b_seg[i] = sc.b_seg[i]; r.a_moff[i] = sc.a_moff[i]; r.b_noff[i] = sc.b_noff[i]; }
+  r.run_if = sc.run_if; r.grp = sc.grp; r.chunk_len = sc.chunk_len; r.n_chunks = sc.n_chunks; r.n_il = sc.n_il;
+  return r;
+}
+
+template <int kCG, class Epi, bool kAMN, bool kBMN, int kSegs>
+int launch_engine_cg(const MapSpec& a, const MapSpec& b, const mi::SchedT<kSegs>& sc, const typename Epi::Params& ep,
+                     cudaStream_t stream) {
   using C = mi::Cfg<kCG>;
   CUtensorMap ta, tb;
   // MN-major A: the map's contiguous dimension is M, its rows are K; fetched as 64 x 64 boxes
@@ -175,7 +197,7 @@ int launch_engine_cg(const MapSpec& a, const MapSpec& b, const Sched& sc, const 
   else MI_TRY(make_tmap(&ta, a.ptr, a.rows, a.k_extent, a.ld, mi::BLOCK_M));
   if (kBMN) MI_TRY(make_tmap(&tb, b.ptr, b.rows, b.k_extent, b.ld, 64));
   else MI_TRY(make_tmap(&tb, b.ptr, b.rows, b.k_extent, b.ld, C::kBRows));
-  auto kern = mi::tile_engine_kernel<kCG, Epi, kAMN, kBMN>;
+  auto kern = mi::tile_engine_kernel<kCG, Epi, kAMN, kBMN, kSegs>;
   constexpr int smem = C::template smem_bytes<Epi>();
   static std::atomic<unsigned long long> attr_devs{0};      // bit d: attribute set on device d (it is per device)
   int dev = 0;
@@ -200,7 +222,7 @@ int launch_engine_cg(const MapSpec& a, const MapSpec& b, const Sched& sc, const 
   attr[0].val.clusterDim.x = kCG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  Sched scp = sc;
+  mi::SchedT<kSegs> scp = sc;
   scp.run_if = t_run_if;
   ProfRec rec; rec.kind = EpiKind<Epi>::value; rec.e0 = nullptr; rec.e1 = nullptr;
   if (g_profiling) {
@@ -225,15 +247,31 @@ template <> struct EpiKind<mi::EpiJS<false>> { static constexpr int value = 0; }
 template <> struct EpiKind<mi::EpiStore> { static constexpr int value = 2; };
 template <> struct EpiKind<mi::EpiMlpFwd> { static constexpr int value = 5; };   // MLP critic: two-pass epilogues
 template <> struct EpiKind<mi::EpiMlpDz> { static constexpr int value = 5; };
+template <> struct EpiKind<mi::EpiMlpDz3> { static constexpr int value = 5; };
 template <> struct EpiKind<mi::EpiMlpSp> { static constexpr int value = 3; };    // single pass (forward + dZ2)
+template <> struct EpiKind<mi::EpiMlpSp3> { static constexpr int value = 3; };
 template <> struct EpiKind<mi::EpiMlpDa> { static constexpr int value = 4; };    // dZ1 with fused reductions
 constexpr int kProfKinds = 6;
 template <> struct EpiKind<mi::EpiDist> { static constexpr int value = 0; };
 
 template <class Epi, bool kAMN = false, bool kBMN = false>
 int launch_engine(const MapSpec& a, const MapSpec& b, const Sched& sc, const typename Epi::Params& ep, cudaStream_t stream) {
-  if (cta_group() == 1) return launch_engine_cg<1, Epi, kAMN, kBMN>(a, b, sc, ep, stream);
-  return launch_engine_cg<2, Epi, kAMN, kBMN>(a, b, sc, ep, stream);
+  constexpr int tables = EpiSegTables<Epi>::value;
+  const long long n_seg = sc.seg_len > 0 ? cdiv(sc.k_blocks, sc.seg_len) : 1;
+  if constexpr ((tables & 1) != 0) {
+    if (n_seg <= 4) {
+      const mi::SchedT<4> s4 = sched_with_table<4>(sc);
+      if (cta_group() == 1) return launch_engine_cg<1, Epi, kAMN, kBMN, 4>(a, b, s4, ep, stream);
+      return launch_engine_cg<2, Epi, kAMN, kBMN, 4>(a, b, s4, ep, stream);
+    }
+  }
+  if constexpr ((tables & 2) != 0) {
+    if (n_seg <= mi::kMaxSegs) {
+      if (cta_group() == 1) return launch_engine_cg<1, Epi, kAMN, kBMN, mi::kMaxSegs>(a, b, sc, ep, stream);
+      return launch_engine_cg<2, Epi, kAMN, kBMN, mi::kMaxSegs>(a, b, sc, ep, stream);
+    }
+  }
+  return MI_ERR_BAD_ARG;
 }
 
 inline int rows_per_mblk() { return mi::BLOCK_M * cta_group(); }
@@ -277,7 +315,7 @@ void single_segment(Sched& sc) {
   sc.nt_base = 0;
   sc.seg_len = sc.k_blocks;
   sc.grp = 1; sc.chunk_len = 1; sc.n_chunks = 1; sc.n_il = 1;
-  for (int i = 0; i < 4; ++i) { sc.a_seg[i] = 0; sc.b_seg[i] = 0; sc.a_moff[i] = 0; sc.b_noff[i] = 0; }
+  for (int i = 0; i < mi::kMaxSegs; ++i) { sc.a_seg[i] = 0; sc.b_seg[i] = 0; sc.a_moff[i] = 0; sc.b_noff[i] = 0; }
 }
 
 // ------------------------------------------------------------------------------------ aux kernels
@@ -1064,7 +1102,7 @@ struct GemmArgs {
   long long M = 0, N = 0;
   int k_blocks = 0;           // total K blocks (all segments)
   int seg_len = 0;            // 0: one segment
-  int a_seg[4] = {0, 0, 0, 0}, b_seg[4] = {0, 0, 0, 0}, a_moff[4] = {0, 0, 0, 0}, b_noff[4] = {0, 0, 0, 0};
+  int a_seg[mi::kMaxSegs] = {}, b_seg[mi::kMaxSegs] = {}, a_moff[mi::kMaxSegs] = {}, b_noff[mi::kMaxSegs] = {};
   int ksplit = 1;
   int order = 1;              // Sched::order of the units: 1 = the K splits of a tile on neighbouring CTA pairs, 0 = the tiles of a
                               // K split on neighbouring pairs (they read the same operand rows at the same time: L2 sharing)
@@ -1091,7 +1129,7 @@ int run_gemm(const GemmArgs& g, Bump& ws, cudaStream_t stream) {
   single_segment(sc);
   if (g.seg_len > 0) {
     sc.seg_len = g.seg_len;
-    for (int i = 0; i < 4; ++i) { sc.a_seg[i] = g.a_seg[i]; sc.b_seg[i] = g.b_seg[i]; sc.a_moff[i] = g.a_moff[i]; sc.b_noff[i] = g.b_noff[i]; }
+    for (int i = 0; i < mi::kMaxSegs; ++i) { sc.a_seg[i] = g.a_seg[i]; sc.b_seg[i] = g.b_seg[i]; sc.a_moff[i] = g.a_moff[i]; sc.b_noff[i] = g.b_noff[i]; }
   }
   float* partial = nullptr;
   const long long ldp = round_up(g.N, 4);      // split-K partials are compact [M, ldp] blocks
@@ -1472,6 +1510,7 @@ int grad_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* sid_k,
               cudaEvent_t ev_after_k = nullptr,
               const MaskBuf* shared_mask = nullptr /* the negatives mask of (sid_q, sid_k), built by the caller */) {
   if (Bq <= 0 || Bk <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
+  if (precision & MI_PREC_FP32X3) return MI_ERR_BAD_ARG;     // three-piece operands: the MLP critic only
   typedef __nv_bfloat16 bf;
   const bool strict = precision == MI_PREC_BF16_STRICT;
   const int n_ntile = static_cast<int>(cdiv(Bk, mi::TILE_N));
@@ -1629,6 +1668,7 @@ int single_pass_impl(const Opnd& Q, const Opnd& K, const int* sid_q, const int* 
                                                   row-sum merge and the CALLER reduces (reduce_rows + flag_to_scal) on another
                                                   stream, so the contractions start without waiting for it */) {
   if (Bq <= 0 || Bk <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
+  if (precision & MI_PREC_FP32X3) return MI_ERR_BAD_ARG;     // three-piece operands: the MLP critic only
   typedef __nv_bfloat16 bf;
   const bool strict = (precision & 1) == MI_PREC_BF16_STRICT;
   const int n_ntile = static_cast<int>(cdiv(Bk, mi::TILE_N));
@@ -1900,6 +1940,7 @@ int critic_impl(const void* X_, const void* Y_, const void* W_, const int* sid, 
                 const std::function<int(long long, long long)>* x_ready = nullptr,  // single pass only: X rows arrive per panel
                 const Fallback& fb = Fallback()) {
   if (B <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
+  if (precision & MI_PREC_FP32X3) return MI_ERR_BAD_ARG;     // three-piece operands: the MLP critic only
   if (estimator < MI_EST_DV || estimator > MI_EST_NWJ) return MI_ERR_BAD_ARG;
   typedef __nv_bfloat16 bf;
   const bf* X = static_cast<const bf*>(X_); const bf* Y = static_cast<const bf*>(Y_); const bf* W = static_cast<const bf*>(W_);
@@ -2521,6 +2562,7 @@ static int host_entry_impl(const void* X_host_, const void* Y_host_, const void*
   const __nv_bfloat16* X_hb = static_cast<const __nv_bfloat16*>(X_host_); const __nv_bfloat16* Y_hb = static_cast<const __nv_bfloat16*>(Y_host_);
   const __nv_bfloat16* W_hb = static_cast<const __nv_bfloat16*>(W_host_);
   if (!X_host || !Y_host || !sid_host || !loss_out_host || !dev_scratch || B <= 0 || D <= 0) return MI_ERR_BAD_ARG;
+  if (precision & MI_PREC_FP32X3) return MI_ERR_BAD_ARG;     // three-piece operands: the MLP critic only
   const bool bilinear = critic == MI_CRITIC_BILINEAR;
   if (bilinear && !W_host) return MI_ERR_BAD_ARG;
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);

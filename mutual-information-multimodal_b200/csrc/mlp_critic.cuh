@@ -17,7 +17,8 @@
 //             dW2 += dZ2^T H          (both operands read MN-major, contraction over the pairs, split-K)
 //             dZ1  = (dZ2 W2) . [H > 0]  (W2 read MN-major; ReLU mask in the epilogue), reduced over j -> dA_i, over i -> dC_j
 //             dX = dA W1x, dY = dC W1y, dW1 = [dA^T X | dC^T Y], db1 = sum_i dA_i
-// Strict ("fp32-accumulate") mode keeps every bf16 operand as a hi/lo pair and adds the cross terms as K segments.
+// Strict ("fp32-accumulate") mode keeps every bf16 operand as a hi/lo pair and adds the cross terms as K segments;
+// fp32 mode keeps three pieces (24 significant bits, six K segments) and bounds every accumulation chain (kFp32ChainK).
 //
 // dv / infonce (global log-sum-exp) run as a SINGLE PASS (mlp_single_pass below): the softmax weights are formed against
 // a reference logit fixed before the pass (maximum over a sample of pairs + margin), so the Z2 accumulator that gives
@@ -26,7 +27,10 @@
 // a softmax weight) are a separate B-pair panel.  A guard that finds the reference outside the safe window repeats the
 // step with the two-pass sequence above behind a device-side predicate.
 // ============================================================================================
-// fp32 [R, C] (pitch ld_in) -> bf16 [R, pitch]: hi in columns [0, C), lo (split == 2) in [Cp, Cp + C), zeros elsewhere
+// fp32 [R, C] (pitch ld_in) -> bf16 [R, pitch]: `split` pieces, p0 = RN(x) in columns [0, C), p1 = RN(x - p0) in
+// [Cp, Cp + C) (split >= 2), p2 = RN(x - p0 - p1) in [2 Cp, 2 Cp + C) (split == 3: the kThird instantiation, so that
+// the fast / strict one carries none of its code), zeros elsewhere
+template <bool kThird>
 __global__ void split_f32_kernel(const float* __restrict__ in, long long ld_in, __nv_bfloat16* __restrict__ out, long long pitch,
                                  int split, long long Cp, long long R, long long C, const int* __restrict__ run_if) {
   MI_PRED(run_if);
@@ -35,9 +39,13 @@ __global__ void split_f32_kernel(const float* __restrict__ in, long long ld_in, 
   const long long r = idx / pitch, c = idx - r * pitch;
   float v = 0.f;
   if (c < C) v = __bfloat162float(__float2bfloat16(in[r * ld_in + c]));
-  else if (split == 2 && c >= Cp && c < Cp + C) {
+  else if (split >= 2 && c >= Cp && c < Cp + C) {
     const float x = in[r * ld_in + (c - Cp)];
     v = x - __bfloat162float(__float2bfloat16(x));
+  } else if (kThird && c >= 2 * Cp && c < 2 * Cp + C) {
+    const float x = in[r * ld_in + (c - 2 * Cp)];
+    const float d = x - __bfloat162float(__float2bfloat16(x));                 // exact
+    v = d - __bfloat162float(__float2bfloat16(d));
   }
   out[idx] = __float2bfloat16(v);
 }
@@ -55,7 +63,16 @@ __global__ void fill_f32_kernel(float* __restrict__ p, long long n, float v) {
   long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i < n) p[i] = v;
 }
-// H[p, k] = relu(A[i, k] + C[j, k]) as bf16 hi (+ lo at column Hp), 8 columns per thread;
+// the third pieces of 8 values v whose first two are packed in hi / lo: RN((v - p0) - p1), both differences exact
+__device__ __forceinline__ uint4 third_pieces8(const float (&v)[8], const uint32_t (&hi)[4], const uint32_t (&lo)[4]) {
+  uint32_t r[4];
+#pragma unroll
+  for (int t = 0; t < 4; ++t)
+    r[t] = ptx::pack_bf16((v[2 * t] - __uint_as_float(hi[t] << 16)) - __uint_as_float(lo[t] << 16),
+                          (v[2 * t + 1] - __uint_as_float(hi[t] & 0xffff0000u)) - __uint_as_float(lo[t] & 0xffff0000u));
+  return make_uint4(r[0], r[1], r[2], r[3]);
+}
+// H[p, k] = relu(A[i, k] + C[j, k]) as bf16 pieces (p0, + p1 at column Hp, + p2 at 2 Hp), 8 columns per thread;
 // pairs p = (i - r0) Bk + j of a row panel, or the positive pairs i = p, j = q_off + p (diag)
 __global__ void mlp_gen_kernel(const float* __restrict__ A, const float* __restrict__ Cm, long long H1, long long Bk, long long r0,
                                long long P, __nv_bfloat16* __restrict__ H, long long pitch, long long Hp, int split, int diag,
@@ -74,12 +91,13 @@ __global__ void mlp_gen_kernel(const float* __restrict__ A, const float* __restr
 #pragma unroll
     for (int t = 0; t < 4; ++t) hi[t] = ptx::pack_bf16(v[2 * t], v[2 * t + 1]);
     *reinterpret_cast<uint4*>(H + p * pitch + k) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-    if (split == 2) {
+    if (split >= 2) {
       uint32_t lo[4];
 #pragma unroll
       for (int t = 0; t < 4; ++t)
         lo[t] = ptx::pack_bf16(v[2 * t] - __uint_as_float(hi[t] << 16), v[2 * t + 1] - __uint_as_float(hi[t] & 0xffff0000u));
       *reinterpret_cast<uint4*>(H + p * pitch + Hp + k) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+      if (split == 3) *reinterpret_cast<uint4*>(H + p * pitch + 2 * Hp + k) = third_pieces8(v, hi, lo);
     }
   }
 }
@@ -89,6 +107,8 @@ __global__ void mlp_gen_kernel(const float* __restrict__ A, const float* __restr
 // blockIdx.y slice: the A row of an image is fetched once per kGenJ pairs, C never again; 4 * wpr threads per text row
 // (the 4 threads of a mask word are consecutive lanes), every 2 KB row segment of H is written by consecutive threads.
 constexpr int kGenJ = 4;
+// kThird: fp32 mode (the third pieces at 2 Hp); the fast / strict instantiation carries none of that code
+template <bool kThird>
 __global__ void __launch_bounds__(256, 3) mlp_gen2_kernel(const float* __restrict__ A, const float* __restrict__ Cm, long long H1, long long B,
                                                        long long Bp, long long r0, long long rr, __nv_bfloat16* __restrict__ H,
                                                        long long pitch, long long Hp, int split, uint32_t* __restrict__ mask, int wpr) {
@@ -140,12 +160,13 @@ __global__ void __launch_bounds__(256, 3) mlp_gen2_kernel(const float* __restric
 #pragma unroll
         for (int e = 0; e < 4; ++e) hi[e] = ptx::pack_bf16(v[2 * e], v[2 * e + 1]);
         *reinterpret_cast<uint4*>(H + p * pitch + k) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-        if (split == 2) {
+        if (split >= 2) {
           uint32_t lo[4];
 #pragma unroll
           for (int e = 0; e < 4; ++e)
             lo[e] = ptx::pack_bf16(v[2 * e] - __uint_as_float(hi[e] << 16), v[2 * e + 1] - __uint_as_float(hi[e] & 0xffff0000u));
           *reinterpret_cast<uint4*>(H + p * pitch + Hp + k) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+          if (kThird) *reinterpret_cast<uint4*>(H + p * pitch + 2 * Hp + k) = third_pieces8(v, hi, lo);
         }
       }
     }
@@ -440,19 +461,45 @@ struct MlpGrads { float *dX, *dY, *dW1, *db1, *dW2, *db2, *dW3, *db3; };
 
 long long g_mlp_max_pairs = 1LL << 20;                    // bounds the panel buffers (H, dZ2, dZ1): 5 GB fast, 10 GB strict
 std::atomic<int> g_mlp_mode{3};                           // bit 0: single pass for dv-like estimators, bit 1: fused dZ1 reductions
-inline long long mlp_panel_rows(long long B, long long cols) {
-  long long R = g_mlp_max_pairs / cols;
+// fp32 mode (sp = 3) takes 2/3 of the pairs per panel: 13 KB per pair (H 6, dZ2 3, dZ1 4) instead of strict's 10 KB
+inline long long mlp_panel_rows(long long B, long long cols, int sp) {
+  long long R = (sp == 3 ? 2 * g_mlp_max_pairs / 3 : g_mlp_max_pairs) / cols;
   if (R < 1) R = 1;
   if (R > B) R = B;
   return R;
 }
 
-// hi*hi (+ lo*hi + hi*lo) K segments of a K-major x K-major product whose operands are [hi | lo] pairs
-void kk_segments(GemmArgs& g, int sp, long long K) {
-  const int kb = static_cast<int>(sp == 2 ? round_up(K, kSplitAlign) / bk() : cdiv(K, bk()));
-  g.k_blocks = kb; g.seg_len = kb;
-  if (sp == 2) { g.k_blocks = 3 * kb; g.a_seg[1] = kb; g.b_seg[2] = kb; }
+// The K segments of a product over K of two operands kept as sp bf16 pieces [p0 | p1 (| p2)] per row (piece t at t times
+// the padded width): the terms of order < sp — p0 p0 (sp = 1); p0 p0, p1 p0, p0 p1 (strict); in fp32 mode the six terms
+// smallest first, p0 p2, p1 p1, p2 p0, p0 p1, p1 p0, p0 p0: the tensor cores truncate every accumulation to the
+// accumulator's precision, so the five correction segments are added while the accumulator is still ~2^-8 of its final
+// size and only the p0 p0 segment's MMAs lose bits at full size.  The pieces of a K-major operand lie kb K blocks apart
+// (a_seg / b_seg); those of an MN-major operand a_off / b_off rows apart (a_moff / b_noff: the padded M / N width).
+// T = GemmArgs or Sched (arrays zeroed by the caller).
+template <class T>
+void piece_segments(T& g, int sp, long long K, bool a_mn, long long a_off, bool b_mn, long long b_off) {
+  static constexpr int ta2[3] = {0, 1, 0}, tb2[3] = {0, 0, 1};
+  static constexpr int ta3[6] = {0, 1, 2, 0, 1, 0}, tb3[6] = {2, 1, 0, 1, 0, 0};
+  const int* ta = sp == 3 ? ta3 : ta2;
+  const int* tb = sp == 3 ? tb3 : tb2;
+  const bool k_pad = sp > 1 && !(a_mn && b_mn);             // K-major pieces start at round_up(K, kSplitAlign)
+  const int kb = static_cast<int>(k_pad ? round_up(K, kSplitAlign) / bk() : cdiv(K, bk()));
+  const int n = sp == 3 ? 6 : sp == 2 ? 3 : 1;
+  g.k_blocks = n * kb; g.seg_len = kb;
+  for (int s = 0; s < n; ++s) {
+    if (a_mn) g.a_moff[s] = static_cast<int>(ta[s] * a_off); else g.a_seg[s] = ta[s] * kb;
+    if (b_mn) g.b_noff[s] = static_cast<int>(tb[s] * b_off); else g.b_seg[s] = tb[s] * kb;
+  }
 }
+void kk_segments(GemmArgs& g, int sp, long long K) { piece_segments(g, sp, K, false, 0, false, 0); }
+
+// fp32 mode: the longest accumulation chain into one TMEM accumulator, in K elements (64 K blocks with CTA pairs, 128
+// single-CTA).  The tensor cores truncate each accumulation (DESIGN 3.4: a chain of n MMAs loses ~n 2^-25 relative), so
+// the contractions over pairs (dW2) and rows (dW1) are cut into split-K partial tiles of at most this length, summed by
+// reduce_partials_kernel in fp32 with round-to-nearest.  The contractions that feed an epilogue (Z2 over H1, dZ1 over H2,
+// layer 1 over D) cannot be split: mlp_dims_ok keeps them within one chain (6 round_up(K, 128) <= kFp32ChainK).
+constexpr long long kFp32ChainK = 8192;
+long long mlp_chain_min_ks(int sp, int k_blocks) { return sp == 3 ? cdiv(static_cast<long long>(k_blocks) * bk(), kFp32ChainK) : 1; }
 
 // memset that respects the launch predicate of this thread
 int zero_async(void* p, size_t bytes, cudaStream_t stream) {
@@ -479,25 +526,27 @@ struct MlpCtx {
   size_t mk;
 };
 
+// the dZ2 epilogues: their three-piece form in fp32 mode
+template <class Epi, class Epi3>
+int mlp_launch_dz(const MlpCtx& c, const MapSpec& a, const MapSpec& b, const Sched& sc, const typename Epi::Params& ep) {
+  return c.sp == 3 ? launch_engine<Epi3>(a, b, sc, ep, c.stream) : launch_engine<Epi>(a, b, sc, ep, c.stream);
+}
 // Z2 = H W2^T over one panel of P pairs, handed to an epilogue policy
 void mlp_z2_sched(const MlpCtx& c, long long P, Sched& sc) {
   sc.n_mblk = static_cast<int>(cdiv(P, rows_per_mblk()));
   sc.n_ntile = c.nt2; sc.n_split = 1; sc.n_ksplit = 1; sc.order = 0;
   single_segment(sc);
-  const int kb = static_cast<int>(c.sp == 2 ? c.Hp / bk() : cdiv(c.H1, bk()));
-  sc.k_blocks = kb; sc.seg_len = kb;
-  if (c.sp == 2) { sc.k_blocks = 3 * kb; sc.a_seg[1] = kb; sc.b_seg[2] = kb; }
+  piece_segments(sc, c.sp, c.H1, false, 0, false, 0);
 }
 // dW2 (+)= dZ2^T H : contraction over the panel's pairs, both operands MN-major
 int mlp_dw2_gemm(const MlpCtx& c, long long P, bool accumulate, Bump& ws) {
   GemmArgs g;
-  const int kb = static_cast<int>(cdiv(P, bk()));
   g.a_mn = true; g.a = MapSpec{c.DZ2, P, c.eZ, c.pZ};
   g.b_mn = true; g.b = MapSpec{c.Hpan, P, c.eH, c.pH};
-  g.M = c.H2; g.N = c.H1; g.k_blocks = kb; g.seg_len = kb;
-  if (c.sp == 2) { g.k_blocks = 3 * kb; g.a_moff[1] = static_cast<int>(c.H2p); g.b_noff[2] = static_cast<int>(c.Hp); }
+  g.M = c.H2; g.N = c.H1;
+  piece_segments(g, c.sp, P, true, c.H2p, true, c.Hp);
   const long long tiles = cdiv(c.H2, rows_per_mblk()) * cdiv(c.H1, mi::TILE_N);
-  g.ksplit = choose_ksplit(tiles, g.k_blocks);
+  g.ksplit = choose_ksplit(tiles, g.k_blocks, mlp_chain_min_ks(c.sp, g.k_blocks));
   g.order = 0;      // the 8 tiles of a K split stream the same rows of dZ2 / H: neighbours share them in L2
   g.out_f32 = c.dW2; g.ld_out = c.H1; g.accumulate = accumulate;
   if (ws.dry) g.out_f32 = reinterpret_cast<float*>(16);
@@ -511,9 +560,7 @@ int mlp_dz1_gemm(const MlpCtx& c, long long P, float* out_f32, __nv_bfloat16* ou
   g.a = MapSpec{c.DZ2, P, c.eZ, c.pZ};
   g.b_mn = true; g.b = MapSpec{c.W2h, c.H2, c.eH, c.pH};
   g.M = P; g.N = c.H1;
-  const int kb = static_cast<int>(c.sp == 2 ? c.H2p / bk() : cdiv(c.H2, bk()));
-  g.k_blocks = kb; g.seg_len = kb;
-  if (c.sp == 2) { g.k_blocks = 3 * kb; g.a_seg[1] = kb; g.b_noff[2] = static_cast<int>(c.Hp); }
+  piece_segments(g, c.sp, c.H2, false, 0, true, c.Hp);
   g.out_f32 = out_f32; g.ld_out = c.H1; g.out_bf16 = out_bf16; g.ld_out16 = c.H1; g.relu_mask = c.Hpan; g.ld_mask = c.pH;
   if (ws.dry) g.out_f32 = reinterpret_cast<float*>(16);
   MI_TRY(run_gemm(g, ws, c.stream));
@@ -552,7 +599,7 @@ int mlp_tp_fwd(const MlpCtx& c, bool dry) {
   if (dry) return MI_OK;
   const long long Bq = c.Bq, Bk = c.Bk, H2 = c.H2;
   cudaStream_t stream = c.stream;
-  const long long R = mlp_panel_rows(Bq, Bk);
+  const long long R = mlp_panel_rows(Bq, Bk, c.sp);
   for (long long r0 = 0; r0 < Bq; r0 += R) {
     const long long rr = (Bq - r0 < R) ? (Bq - r0) : R, P = rr * Bk;
     MI_TRY(mlp_tp_gen_panel(c, r0, P));
@@ -597,7 +644,7 @@ int mlp_tp_bwd(const MlpCtx& c, bool resident, Bump& ws) {
   const long long Bq = c.Bq, Bk = c.Bk, H2 = c.H2;
   const bool dry = ws.dry;
   cudaStream_t stream = c.stream;
-  const long long R = mlp_panel_rows(Bq, Bk);
+  const long long R = mlp_panel_rows(Bq, Bk, c.sp);
   if (!dry) {
     const int dv_like = (c.estimator == MI_EST_DV || c.estimator == MI_EST_INFONCE_REF) ? 1 : 0;
     const float* col_lse = c.estimator == MI_EST_INFONCE_SYM ? c.col_lse : nullptr;
@@ -613,11 +660,11 @@ int mlp_tp_bwd(const MlpCtx& c, bool resident, Bump& ws) {
       Sched sc; mlp_z2_sched(c, P, sc);
       mi::EpiMlpDz::Params ep;
       ep.b2 = c.b2p; ep.w3 = c.w3p; ep.g = c.G + r0 * Bk; ep.rows = static_cast<int>(P); ep.cols = static_cast<int>(H2);
-      ep.dz = c.DZ2; ep.dz_lo = c.sp == 2 ? c.DZ2 + c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
-      MI_TRY(launch_engine<mi::EpiMlpDz>(MapSpec{c.Hpan, P, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
+      ep.dz = c.DZ2; ep.dz_lo = c.sp >= 2 ? c.DZ2 + c.H2p : nullptr; ep.dz_lo2 = c.sp == 3 ? c.DZ2 + 2 * c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
+      MI_TRY((mlp_launch_dz<mi::EpiMlpDz, mi::EpiMlpDz3>(c, MapSpec{c.Hpan, P, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep)));
     }
     MI_TRY(mlp_dw2_gemm(c, P, r0 > 0, ws));
-    MI_TRY(mlp_dz1_gemm(c, P, c.sp == 2 ? c.DZ1 : nullptr, c.sp == 1 ? c.DZ1h : nullptr, ws));
+    MI_TRY(mlp_dz1_gemm(c, P, c.sp >= 2 ? c.DZ1 : nullptr, c.sp == 1 ? c.DZ1h : nullptr, ws));
     if (!dry) MI_TRY(mlp_reduce_panel(c, Bk, rr, r0));
   }
   if (!dry) {
@@ -637,7 +684,7 @@ int mlp_two_pass(const MlpCtx& c, bool plan, Bump& ws) {
     MI_LAUNCH_CHECK("loss_finalize_kernel");
   }
   if (!plan) return MI_OK;
-  return mlp_tp_bwd(c, mlp_panel_rows(c.Bq, c.Bk) >= c.Bq, ws);
+  return mlp_tp_bwd(c, mlp_panel_rows(c.Bq, c.Bk, c.sp) >= c.Bq, ws);
 }
 
 // reference of the single pass: the maximum logit over an n x n strided sample of the block's OWN pairs (image rows
@@ -686,7 +733,7 @@ int mlp_sp_panels(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws) {
   const bool dry = ws.dry;
   cudaStream_t stream = c.stream;
   const long long Bp = round_up(Bk, rows_per_mblk());
-  const long long R = mlp_panel_rows(Bq, Bp);
+  const long long R = mlp_panel_rows(Bq, Bp, c.sp);
   const int wpr = static_cast<int>(round_up(cdiv(H1, 32), 2));          // even: the epilogue reads word pairs
   const bool fused_da = (g_mlp_mode.load(std::memory_order_relaxed) & 2) != 0;
   if (!dry) {
@@ -701,7 +748,8 @@ int mlp_sp_panels(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws) {
         long long ny = cdiv(16LL * num_sms(), gg.x);              // enough blocks in flight to saturate the HBM writes
         if (ny > rr) ny = rr;
         gg.y = static_cast<unsigned>(ny < 1 ? 1 : ny);
-        mlp_gen2_kernel<<<gg, 256, 0, stream>>>(c.A32, c.C32, H1, Bk, Bp, r0, rr, c.Hpan, c.pH, c.Hp, c.sp, sb.mask, wpr);
+        if (c.sp == 3) mlp_gen2_kernel<true><<<gg, 256, 0, stream>>>(c.A32, c.C32, H1, Bk, Bp, r0, rr, c.Hpan, c.pH, c.Hp, c.sp, sb.mask, wpr);
+        else mlp_gen2_kernel<false><<<gg, 256, 0, stream>>>(c.A32, c.C32, H1, Bk, Bp, r0, rr, c.Hpan, c.pH, c.Hp, c.sp, sb.mask, wpr);
         MI_LAUNCH_CHECK("mlp_gen2_kernel");
       }
       Sched sc; mlp_z2_sched(c, P, sc);
@@ -710,9 +758,9 @@ int mlp_sp_panels(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws) {
       ep.B = static_cast<int>(Bk); ep.Bp = static_cast<int>(Bp); ep.r0 = static_cast<int>(r0); ep.rr = static_cast<int>(rr);
       ep.q_off = static_cast<int>(c.q_off);
       ep.cols = static_cast<int>(H2);
-      ep.dz = c.DZ2; ep.dz_lo = c.sp == 2 ? c.DZ2 + c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
+      ep.dz = c.DZ2; ep.dz_lo = c.sp >= 2 ? c.DZ2 + c.H2p : nullptr; ep.dz_lo2 = c.sp == 3 ? c.DZ2 + 2 * c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
       ep.rowsum = sb.rowsum; ep.rowcnt = sb.rowcnt; ep.diag_out = sb.diag; ep.S_out = S_out;
-      MI_TRY(launch_engine<mi::EpiMlpSp>(MapSpec{c.Hpan, P, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
+      MI_TRY((mlp_launch_dz<mi::EpiMlpSp, mi::EpiMlpSp3>(c, MapSpec{c.Hpan, P, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep)));
     }
     MI_TRY(mlp_dw2_gemm(c, P, r0 > 0, ws));
     if (fused_da) {
@@ -724,9 +772,7 @@ int mlp_sp_panels(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws) {
         sc.grp = static_cast<int>(Bp / rows_per_mblk()); sc.n_il = static_cast<int>(rr);
         mlp_da_chunks(rr, static_cast<long long>(sc.n_ntile) * sc.grp, sc.chunk_len, sc.n_chunks);
         sc.n_mblk = sc.grp * sc.n_il; sc.n_split = 1; sc.n_ksplit = 1;
-        const int kb = static_cast<int>(c.sp == 2 ? c.H2p / bk() : cdiv(H2, bk()));
-        sc.k_blocks = kb; sc.seg_len = kb;
-        if (c.sp == 2) { sc.k_blocks = 3 * kb; sc.a_seg[1] = kb; sc.b_noff[2] = static_cast<int>(c.Hp); }
+        piece_segments(sc, c.sp, H2, false, 0, true, c.Hp);
         mi::EpiMlpDa::Params ep;
         ep.mask = sb.mask; ep.wpr = wpr; ep.B = static_cast<int>(Bk); ep.Bp = static_cast<int>(Bp);
         ep.r0 = static_cast<int>(r0); ep.rr = static_cast<int>(rr); ep.cols = static_cast<int>(H1);
@@ -734,7 +780,7 @@ int mlp_sp_panels(const MlpCtx& c, const MlpSpBuf& sb, float* S_out, Bump& ws) {
         MI_TRY((launch_engine<mi::EpiMlpDa, false, true>(MapSpec{c.DZ2, P, c.eZ, c.pZ}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream)));
       }
     } else {
-      MI_TRY(mlp_dz1_gemm(c, P, c.sp == 2 ? c.DZ1 : nullptr, c.sp == 1 ? c.DZ1h : nullptr, ws));
+      MI_TRY(mlp_dz1_gemm(c, P, c.sp >= 2 ? c.DZ1 : nullptr, c.sp == 1 ? c.DZ1h : nullptr, ws));
       if (!dry) MI_TRY(mlp_reduce_panel(c, Bp, rr, r0));
     }
   }
@@ -773,8 +819,8 @@ int mlp_sp_finish(const MlpCtx& c, const MlpSpBuf& sb, const double* total, doub
     Sched sc; mlp_z2_sched(c, Bq, sc);
     mi::EpiMlpDz::Params ep;
     ep.b2 = c.b2p; ep.w3 = c.w3p; ep.g = sb.gd; ep.rows = static_cast<int>(Bq); ep.cols = static_cast<int>(H2);
-    ep.dz = c.DZ2; ep.dz_lo = c.sp == 2 ? c.DZ2 + c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
-    MI_TRY(launch_engine<mi::EpiMlpDz>(MapSpec{c.Hpan, Bq, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep, stream));
+    ep.dz = c.DZ2; ep.dz_lo = c.sp >= 2 ? c.DZ2 + c.H2p : nullptr; ep.dz_lo2 = c.sp == 3 ? c.DZ2 + 2 * c.H2p : nullptr; ep.pitch = c.pZ; ep.dw3 = c.acc_w3; ep.db2 = c.acc_b2;
+    MI_TRY((mlp_launch_dz<mi::EpiMlpDz, mi::EpiMlpDz3>(c, MapSpec{c.Hpan, Bq, c.eH, c.pH}, MapSpec{c.W2h, H2, c.eH, c.pH}, sc, ep)));
   }
   MI_TRY(mlp_dw2_gemm(c, Bq, true, ws));
   MI_TRY(mlp_dz1_gemm(c, Bq, sb.DZ1d, nullptr, ws));
@@ -787,22 +833,30 @@ int mlp_sp_finish(const MlpCtx& c, const MlpSpBuf& sb, const double* total, doub
 
 void mlp_ctx_dims(MlpCtx& c, long long D, long long H1, long long H2, int precision) {
   c.D = D; c.H1 = H1; c.H2 = H2;
-  c.sp = (precision & 1) == MI_PREC_BF16_STRICT ? 2 : 1;
+  c.sp = precision == MI_PREC_FP32X3 ? 3 : (precision & 1) == MI_PREC_BF16_STRICT ? 2 : 1;
   const int sp = c.sp;
   c.Dp = round_up(D, kSplitAlign); c.Hp = round_up(H1, kSplitAlign); c.H2p = round_up(H2, kSplitAlign);
-  c.pX = sp == 2 ? 2 * c.Dp : D; c.pH = sp == 2 ? 2 * c.Hp : H1; c.pZ = sp == 2 ? 2 * c.H2p : H2;
-  c.eX = sp == 2 ? c.Dp + D : D; c.eH = sp == 2 ? c.Hp + H1 : H1; c.eZ = sp == 2 ? c.H2p + H2 : H2;   // TMA extents
+  c.pX = sp > 1 ? sp * c.Dp : D; c.pH = sp > 1 ? sp * c.Hp : H1; c.pZ = sp > 1 ? sp * c.H2p : H2;
+  c.eX = (sp - 1) * c.Dp + D; c.eH = (sp - 1) * c.Hp + H1; c.eZ = (sp - 1) * c.H2p + H2;   // TMA extents
   c.nt2 = static_cast<int>(cdiv(H2, mi::TILE_N));
   c.h2_pad = static_cast<long long>(c.nt2) * mi::TILE_N;
 }
-bool mlp_dims_ok(const MlpDims& d, int estimator) {
+// precision: MI_PREC_BF16_FAST, MI_PREC_BF16_STRICT or MI_PREC_FP32X3; fp32 mode also needs the unsplittable contractions
+// over D and H1 (layer 1, Z2) to stay within one bounded chain (kFp32ChainK): D, H1 <= 1280
+bool mlp_precision_ok(int precision, long long D, long long H1) {
+  if (precision == MI_PREC_BF16_FAST || precision == MI_PREC_BF16_STRICT) return true;
+  return precision == MI_PREC_FP32X3 && 6 * round_up(D, kSplitAlign) <= kFp32ChainK && 6 * round_up(H1, kSplitAlign) <= kFp32ChainK;
+}
+bool mlp_dims_ok(const MlpDims& d, int estimator, int precision) {
   if (d.B <= 0 || d.D <= 0 || d.H1 <= 0 || d.H2 <= 0 || (d.D % 8) != 0 || (d.H1 % 8) != 0 || (d.H2 % 8) != 0) return false;
   if (d.H2 > mi::EpiMlpDz::kMaxTiles * mi::TILE_N) return false;
+  if (!mlp_precision_ok(precision, d.D, d.H1)) return false;
   return estimator == MI_EST_DV || estimator == MI_EST_INFONCE_REF || estimator == MI_EST_INFONCE_ROW || estimator == MI_EST_INFONCE_SYM;
 }
-// fp32 [R, C] (pitch ld_in) -> the bf16 operand (hi, + lo in strict mode) of pitch `pitch`, lo half at column Cp
+// fp32 [R, C] (pitch ld_in) -> the bf16 operand (c.sp pieces, see split_f32_kernel) of pitch `pitch`, piece t at column t Cp
 int mlp_split(const MlpCtx& c, const float* in, long long ld_in, __nv_bfloat16* out, long long pitch, long long Cp, long long R, long long C) {
-  split_f32_kernel<<<blocks_for(R * pitch, 256), 256, 0, c.stream>>>(in, ld_in, out, pitch, c.sp, Cp, R, C, nullptr);
+  if (c.sp == 3) split_f32_kernel<true><<<blocks_for(R * pitch, 256), 256, 0, c.stream>>>(in, ld_in, out, pitch, c.sp, Cp, R, C, nullptr);
+  else split_f32_kernel<false><<<blocks_for(R * pitch, 256), 256, 0, c.stream>>>(in, ld_in, out, pitch, c.sp, Cp, R, C, nullptr);
   MI_LAUNCH_CHECK("split_f32_kernel");
   return MI_OK;
 }
@@ -822,7 +876,7 @@ int mlp_setup(MlpCtx& c, MlpSpBuf& sb, const float* X, const float* Y, const Mlp
   mlp_ctx_dims(c, D, H1, H2, precision);
   const int sp = c.sp;
   const long long Bp = round_up(Bk, rows_per_mblk());
-  const long long Pmax1 = mlp_panel_rows(Bq, Bk) * Bk, Pmax2 = mlp_panel_rows(Bq, Bp) * Bp;
+  const long long Pmax1 = mlp_panel_rows(Bq, Bk, sp) * Bk, Pmax2 = mlp_panel_rows(Bq, Bp, sp) * Bp;
   const long long ns_ref = Bq < kMlpRefSample ? Bq : kMlpRefSample;      // the reference-logit sample is a panel too
   long long Pmax = Pmax1 > Pmax2 ? Pmax1 : Pmax2;
   if (Pmax < ns_ref * ns_ref) Pmax = ns_ref * ns_ref;
@@ -849,8 +903,8 @@ int mlp_setup(MlpCtx& c, MlpSpBuf& sb, const float* X, const float* Y, const Mlp
   c.part = ws.take<float>(mi::kColQuarters * rows_padded_max);
   c.G = plan ? ws.take<float>(Bq * Bk) : nullptr;
   c.DZ2 = plan ? ws.take<bf>(Pmax * pZ) : nullptr;
-  // dZ1 panel: bf16 in fast mode (half the bytes of the HBM-write-bound masked contraction), fp32 in strict mode
-  c.DZ1 = (plan && sp == 2) ? ws.take<float>(Pmax * H1) : nullptr;
+  // dZ1 panel: bf16 in fast mode (half the bytes of the HBM-write-bound masked contraction), fp32 in strict / fp32 mode
+  c.DZ1 = (plan && sp >= 2) ? ws.take<float>(Pmax * H1) : nullptr;
   c.DZ1h = (plan && sp == 1) ? ws.take<bf>(Pmax * H1) : nullptr;
   c.dA32 = plan ? keep.take<float>(Bq * H1) : nullptr; c.dC32 = plan ? keep.take<float>(Bp * H1) : nullptr;
   c.dA16 = plan ? ws.take<bf>(Bq * pH) : nullptr; c.dC16 = plan ? ws.take<bf>(Bk * pH) : nullptr;
@@ -883,9 +937,9 @@ int mlp_setup(MlpCtx& c, MlpSpBuf& sb, const float* X, const float* Y, const Mlp
     MI_LAUNCH_CHECK("pad_f32_kernel");
     pad_f32_kernel<<<blocks_for(c.h2_pad, 256), 256, 0, stream>>>(prm.W3, c.w3p, H2, c.h2_pad);
     MI_LAUNCH_CHECK("pad_f32_kernel");
-    // the gaps between the hi and lo halves / beyond a ragged K are never written by the generators
-    if (sp == 2 || (H1 % bk()) != 0) MI_CUDA(cudaMemsetAsync(c.Hpan, 0, static_cast<size_t>(Pmax) * pH * sizeof(bf), stream));
-    if (c.DZ2 && (sp == 2 || (H2 % bk()) != 0)) MI_CUDA(cudaMemsetAsync(c.DZ2, 0, static_cast<size_t>(Pmax) * pZ * sizeof(bf), stream));
+    // the gaps between the pieces / beyond a ragged K are never written by the generators
+    if (sp >= 2 || (H1 % bk()) != 0) MI_CUDA(cudaMemsetAsync(c.Hpan, 0, static_cast<size_t>(Pmax) * pH * sizeof(bf), stream));
+    if (c.DZ2 && (sp >= 2 || (H2 % bk()) != 0)) MI_CUDA(cudaMemsetAsync(c.DZ2, 0, static_cast<size_t>(Pmax) * pZ * sizeof(bf), stream));
   }
   // ---- layer 1: A = X W1x^T + b1, C = Y W1y^T  (fp32 out)
   for (int side = 0; side < 2; ++side) {
@@ -917,9 +971,7 @@ int mlp_layer1_bwd(const MlpCtx& c, long long R, const float* dZ32, __nv_bfloat1
     g.a = MapSpec{dZ16, R, c.eH, pH};
     g.b_mn = true; g.b = MapSpec{W16, H1, c.eX, pX};
     g.M = R; g.N = D;
-    const int kb = static_cast<int>(sp == 2 ? c.Hp / bk() : cdiv(H1, bk()));
-    g.k_blocks = kb; g.seg_len = kb;
-    if (sp == 2) { g.k_blocks = 3 * kb; g.a_seg[1] = kb; g.b_noff[2] = static_cast<int>(c.Dp); }
+    piece_segments(g, sp, H1, false, 0, true, c.Dp);
     g.out_f32 = dIn; g.ld_out = D;
     if (dry) { g.out_f32 = reinterpret_cast<float*>(16); }
     MI_TRY(run_gemm(g, ws, c.stream));
@@ -927,13 +979,12 @@ int mlp_layer1_bwd(const MlpCtx& c, long long R, const float* dZ32, __nv_bfloat1
   }
   if (dW1_side || dry) {   // dW1[:, side] = dZ^T In : contraction over the rows, both operands MN-major
     GemmArgs g;
-    const int kb = static_cast<int>(cdiv(R, bk()));
     g.a_mn = true; g.a = MapSpec{dZ16, R, c.eH, pH};
     g.b_mn = true; g.b = MapSpec{In16, R, c.eX, pX};
-    g.M = H1; g.N = D; g.k_blocks = kb; g.seg_len = kb;
-    if (sp == 2) { g.k_blocks = 3 * kb; g.a_moff[1] = static_cast<int>(c.Hp); g.b_noff[2] = static_cast<int>(c.Dp); }
+    g.M = H1; g.N = D;
+    piece_segments(g, sp, R, true, c.Hp, true, c.Dp);
     const long long tiles = cdiv(H1, rows_per_mblk()) * cdiv(D, mi::TILE_N);
-    g.ksplit = choose_ksplit(tiles, g.k_blocks);
+    g.ksplit = choose_ksplit(tiles, g.k_blocks, mlp_chain_min_ks(sp, g.k_blocks));
     g.out_f32 = dW1_side; g.ld_out = 2 * D;
     if (dry) { g.out_f32 = reinterpret_cast<float*>(16); }
     MI_TRY(run_gemm(g, ws, c.stream));
@@ -945,7 +996,7 @@ int mlp_layer1_bwd(const MlpCtx& c, long long R, const float* dZ32, __nv_bfloat1
 // ---- the single-GPU step: the block form with Bq = Bk = Bg = B, q_off = 0, one id vector
 int mlp_impl(const float* X, const float* Y, const MlpParams& prm, const int* sid, const MlpDims& d, int estimator, int precision,
              double* loss_out, float* S_out, const MlpGrads& gr, Bump& ws, cudaStream_t stream) {
-  if (!mlp_dims_ok(d, estimator)) return MI_ERR_BAD_ARG;
+  if (!mlp_dims_ok(d, estimator, precision)) return MI_ERR_BAD_ARG;
   const long long B = d.B, D = d.D, H1 = d.H1, H2 = d.H2;
   const bool grads = gr.dX || gr.dY || gr.dW1 || gr.db1 || gr.dW2 || gr.db2 || gr.dW3 || gr.db3;
   const bool plan = grads || ws.dry;
@@ -1012,7 +1063,7 @@ struct MlpBlockIO {
 };
 int mlp_block_impl(int stage, const float* X, const float* Y, const MlpParams& prm, const MlpBlock& blk, const MlpDims& d,
                    int estimator, int precision, const MlpBlockIO& io, Bump& ws, Bump& keep, cudaStream_t stream) {
-  if (!mlp_dims_ok(d, estimator)) return MI_ERR_BAD_ARG;
+  if (!mlp_dims_ok(d, estimator, precision)) return MI_ERR_BAD_ARG;
   const long long H1 = d.H1, H2 = d.H2;
   const bool sym = estimator == MI_EST_INFONCE_SYM;       // the two-pass sequence only: columns need every row first
   bool args_ok = true;
@@ -1071,6 +1122,7 @@ int mlp_block_impl(int stage, const float* X, const float* Y, const MlpParams& p
 int mlp_input_grad_impl(const float* dZ, const float* In, const float* W1, int side, long long R, long long D, long long H1, int precision,
                         float* dIn, float* dW1, float* db1, Bump& ws, cudaStream_t stream) {
   if (R <= 0 || D <= 0 || H1 <= 0 || (D % 8) != 0 || (H1 % 8) != 0 || (side != 0 && side != 1)) return MI_ERR_BAD_ARG;
+  if (!mlp_precision_ok(precision, D, H1)) return MI_ERR_BAD_ARG;
   typedef __nv_bfloat16 bf;
   MlpCtx c;
   c.stream = stream;

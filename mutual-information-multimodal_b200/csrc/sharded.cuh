@@ -102,6 +102,7 @@ int sharded_impl(mi_dist_ctx* ctx, int world, int rank, const void* X_, const vo
                  double* loss_out, float* dX, float* dY, float* dW, Bump& ws, int check_guard, cudaStream_t S) {
   typedef __nv_bfloat16 bf;
   if (Bl <= 0 || D <= 0 || (D % 8) != 0) return MI_ERR_BAD_ARG;
+  if (precision & MI_PREC_FP32X3) return MI_ERR_BAD_ARG;     // three-piece operands: the MLP critic only
   if (estimator < MI_EST_DV || estimator > MI_EST_INFONCE_SYM) return MI_ERR_BAD_ARG;
   const bool bilinear = critic == MI_CRITIC_BILINEAR;
   const bool sym = estimator == MI_EST_INFONCE_SYM;

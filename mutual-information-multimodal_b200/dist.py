@@ -234,6 +234,8 @@ def sharded_critic_loss_fwd_bwd(X_local: torch.Tensor, Y_local: torch.Tensor, W:
     it is non-zero the step is repeated on the exact path (``two_pass=True``: statistics pass + gradient pass).
     ``check_guard=False`` skips that host read (no synchronisation at all); the count is then left in stats['guard'] for the
     caller to act on."""
+    if precision not in ("fast", "strict"):      # before any collective: "fp32" exists for the MLP critic only
+        raise ValueError(f"the batch-sharded dot / bilinear critic supports the fast and strict precisions, not {precision!r}")
     if backend is None:
         from . import ops as backend  # the CUDA path; raises if the library / device is missing
     world, rank = _world(group)

@@ -18,6 +18,9 @@ ESTIMATOR = {"dv": 0, "infonce": 1, "infonce_ref": 1, "infonce_row": 2, "infonce
 # the f-divergence bounds run on the single-GPU separable critics only (dot / bilinear, critic_loss_fwd_bwd)
 SEPARABLE_ONLY = ("js", "nwj")
 PRECISION = {"fast": 0, "strict": 1}
+# the MLP critic's entries also take "fp32": three bf16 pieces per operand (24 significant bits, MI_PREC_FP32X3); the
+# separable, sharded-separable and GDV paths read PRECISION above and reject it before any launch
+MLP_PRECISION = dict(PRECISION, fp32=4)
 
 
 class MIError(RuntimeError):
@@ -261,13 +264,13 @@ def score_grad(Q: Mat, K: Mat, sid_q, sid_k, q_offset: int, scale: float,
     ``event_after_k`` (a recorded torch.cuda.Event) is re-recorded on the current stream as soon as Ok is
     complete, before the Oq contraction runs."""
     _need_cuda(Q, K, sid_q, sid_k, refq, refk)
+    prec = _precision(precision)
     lib = _lib.load()
     Qt, ldq, qsp, D = _opnd(Q)
     Kt, ldk, ksp, Dk = _opnd(K)
     assert D == Dk
     sid_q, sid_k = sid_q.to(torch.int32).contiguous(), sid_k.to(torch.int32).contiguous()
     Bq, Bk = Qt.shape[0], Kt.shape[0]
-    prec = PRECISION[precision]
     dev = Qt.device
     o32 = torch.empty((Bq, D), dtype=torch.float32, device=dev) if want_f32 else None
     o16 = ob = None
@@ -342,6 +345,7 @@ def score_single_pass(Q: Mat, K: Mat, sid_q, sid_k, q_offset: int, scale: float,
     """mi_score_single_pass: statistics and raw gradient contractions from ONE score computation, relative to the
     per-row references ``ref`` (score_ref_sample) and the global constant ``lam`` (dv-like estimators)."""
     _need_cuda(Q, K, sid_q, sid_k, ref, lam, diag)
+    prec = _precision(precision)
     lib = _lib.load()
     Qt, ldq, qsp, D = _opnd(Q)
     Kt, ldk, ksp, Dk = _opnd(K)
@@ -349,7 +353,6 @@ def score_single_pass(Q: Mat, K: Mat, sid_q, sid_k, q_offset: int, scale: float,
     sid_q, sid_k = sid_q.to(torch.int32).contiguous(), sid_k.to(torch.int32).contiguous()
     Bq, Bk = Qt.shape[0], Kt.shape[0]
     dev = Qt.device
-    prec = PRECISION[precision]
     f32 = dict(dtype=torch.float32, device=dev)
     r = {"rows": torch.empty((Bq, 4), **f32), "scal": torch.empty(8, dtype=torch.float64, device=dev),
          "oq_raw": torch.empty((Bq, D), **f32), "ok_raw": torch.empty((Bk, D), **f32) if want_k else None,
@@ -440,13 +443,14 @@ def critic_loss_fwd_bwd(X: torch.Tensor, Y: torch.Tensor, W: Optional[torch.Tens
     sync) — loss_out[7] counts the rows that tripped (informational).  ``two_pass`` asks for exact references from the
     start (MI_PREC_TWO_PASS).  ``workspace_buf``: caller-owned scratch of ``critic_workspace_bytes`` (CUDA graphs)."""
     _need_cuda(X, Y, W, sid)
+    prec = _precision(precision) | (2 if two_pass else 0)
     lib = _lib.load()
     X, Y = as_bf16(X), as_bf16(Y)
     W = None if W is None else as_bf16(W)
     sid = sid.to(torch.int32).contiguous()
     B, D = X.shape
     critic = 1 if W is not None else 0
-    est, prec = ESTIMATOR[estimator], PRECISION[precision] | (2 if two_pass else 0)
+    est = ESTIMATOR[estimator]
     dX = dY = dW = None
     if out is not None:
         loss, dX, dY, dW = out
@@ -499,6 +503,7 @@ def sharded_step(X_local: torch.Tensor, Y_local: torch.Tensor, W: Optional[torch
     are not valid and the step must be repeated on the exact path ("infonce_sym" uses exact statistics: always 0)."""
     reject_separable_only(estimator, "the batch-sharded step")
     _need_cuda(X_local, Y_local, W, sid_local)
+    prec = _precision(precision)
     lib = _lib.load()
     ctx, rank, world, _ = dist_context(group)
     if "MI_RS_RESERVE_SMS" in os.environ:       # (experiment knob) SMs the dT contraction leaves to the overlapped reduce-scatter
@@ -510,7 +515,7 @@ def sharded_step(X_local: torch.Tensor, Y_local: torch.Tensor, W: Optional[torch
     sid = sid_local.contiguous()
     Bl, D = X.shape
     critic = 1 if Wb is not None else 0
-    est, prec = ESTIMATOR[estimator], PRECISION[precision]
+    est = ESTIMATOR[estimator]
     dev = X.device
     loss = torch.empty(8, dtype=torch.float64, device=dev)
     dX = torch.empty((Bl, D), dtype=torch.float32, device=dev)
@@ -534,6 +539,7 @@ class GraphedCriticStep:
 
     def __init__(self, B: int, D: int, bilinear: bool = True, estimator: str = "dv", precision: str = "fast",
                  inv_tau: float = 1.0, device=None):
+        prec = _precision(precision)
         dev = torch.device("cuda" if device is None else device)
         self.args = (estimator, precision, inv_tau)
         self.X = torch.zeros((B, D), dtype=torch.bfloat16, device=dev)
@@ -543,7 +549,7 @@ class GraphedCriticStep:
         self.out = (torch.empty(8, dtype=torch.float64, device=dev), torch.empty((B, D), device=dev),
                     torch.empty((B, D), device=dev), torch.empty((D, D), device=dev) if bilinear else None)
         # the captured graph bakes the scratch pointer in: a PRIVATE workspace that lives as long as the graph does
-        nbytes = _lib.load().mi_critic_workspace_bytes(B, D, 1 if bilinear else 0, ESTIMATOR[estimator], PRECISION[precision], 1)
+        nbytes = _lib.load().mi_critic_workspace_bytes(B, D, 1 if bilinear else 0, ESTIMATOR[estimator], prec, 1)
         self.ws = torch.empty(max(int(nbytes), 256), dtype=torch.uint8, device=dev)
         self.graph = None
 
@@ -580,6 +586,7 @@ def mlp_critic_loss_fwd_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid: torch
     row / column losses of infonce_sym."""
     reject_separable_only(estimator, "the MLP critic")
     _need_cuda(X, Y, sid, *params)
+    prec = _mlp_precision(precision)
     lib = _lib.load()
     f32 = lambda t: t.detach().to(torch.float32).contiguous()
     X, Y = f32(X), f32(Y)
@@ -588,7 +595,7 @@ def mlp_critic_loss_fwd_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid: torch
     H1, H2 = W1.shape[0], W2.shape[0]
     if W1.shape != (H1, 2 * D) or W2.shape != (H2, H1) or W3.numel() != H2 or b1.numel() != H1 or b2.numel() != H2 or b3.numel() != 1:
         raise MIError("MLP critic parameters do not have the make_mlp(2D, [H1, H2]) shapes")
-    est, prec = _mlp_estimator(estimator), PRECISION[precision]
+    est = _mlp_estimator(estimator)
     sid = sid.to(torch.int32).contiguous()
     dev = X.device
     loss = torch.empty(8, dtype=torch.float64, device=dev)
@@ -601,7 +608,7 @@ def mlp_critic_loss_fwd_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid: torch
     g = grads or {}
     nbytes = lib.mi_mlp_critic_workspace_bytes(B, D, H1, H2, prec)
     if nbytes == 0:
-        raise MIError("mi_mlp_critic_workspace_bytes: unsupported shape (D, H1, H2 multiples of 8, H2 <= 512)")
+        raise MIError("mi_mlp_critic_workspace_bytes: unsupported shape (D, H1, H2 multiples of 8, H2 <= 512; fp32: D, H1 <= 1280)")
     ws = workspace(nbytes, dev)
     _check(lib.mi_mlp_critic_loss_fwd_bwd(_ptr(X), _ptr(Y), _ptr(W1), _ptr(b1), _ptr(W2), _ptr(b2), _ptr(W3), _ptr(b3), _ptr(sid),
                                           B, D, H1, H2, est, prec, _ptr(loss), _ptr(S),
@@ -639,7 +646,7 @@ def _mlp_operands(X, Y, params):
 def _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, dev):
     nbytes = _lib.load().mi_mlp_block_workspace_bytes(Bq, Bk, D, H1, H2, prec)
     if nbytes == 0:
-        raise MIError("mi_mlp_block_workspace_bytes: unsupported shape (D, H1, H2 multiples of 8, H2 <= 512)")
+        raise MIError("mi_mlp_block_workspace_bytes: unsupported shape (D, H1, H2 multiples of 8, H2 <= 512; fp32: D, H1 <= 1280)")
     return workspace(nbytes, dev)
 
 
@@ -649,6 +656,20 @@ def reject_separable_only(estimator: str, what: str) -> None:
         supported = ", ".join(e for e in ESTIMATOR if e not in SEPARABLE_ONLY)
         raise MIError(f"estimator {estimator!r} is not implemented for {what}: supported are {supported} "
                       f"({' and '.join(SEPARABLE_ONLY)} run on the single-GPU dot / bilinear critics)")
+
+
+def _precision(precision: str) -> int:
+    """The code of a precision of the separable critics / GDV ("fast", "strict"); "fp32" is the MLP critic's only."""
+    if precision not in PRECISION:
+        extra = " (\"fp32\" is implemented for the MLP critic only)" if precision in MLP_PRECISION else ""
+        raise MIError(f"unknown precision {precision!r}: supported are {', '.join(PRECISION)}{extra}")
+    return PRECISION[precision]
+
+
+def _mlp_precision(precision: str) -> int:
+    if precision not in MLP_PRECISION:
+        raise MIError(f"unknown precision {precision!r}: the MLP critic supports {', '.join(MLP_PRECISION)}")
+    return MLP_PRECISION[precision]
 
 
 def _mlp_estimator(estimator):
@@ -663,7 +684,7 @@ def mlp_block_ref_logit(X: torch.Tensor, Y: torch.Tensor, params, q_offset: int,
     """Maximum logit of a sample of the block's own pairs (image rows X against the text rows of Y at q_offset ..)
     (mi_mlp_block_ref_logit) -> fp32 [1]."""
     X, Y, prm, D, H1, H2 = _mlp_operands(X, Y, params)
-    Bq, Bk, prec = X.shape[0], Y.shape[0], PRECISION[precision]
+    Bq, Bk, prec = X.shape[0], Y.shape[0], _mlp_precision(precision)
     ref = torch.empty(1, dtype=torch.float32, device=X.device)
     ws = _mlp_block_workspace(Bq, Bk, D, H1, H2, prec, X.device)
     _check(_lib.load().mi_mlp_block_ref_logit(*(_ptr(t) for t in (X, Y) + prm), Bq, Bk, q_offset, D, H1, H2, prec, _ptr(ref),
@@ -679,7 +700,7 @@ def mlp_block_fwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor,
     ``mlp_block_bwd``."""
     X, Y, prm, D, H1, H2 = _mlp_operands(X, Y, params)
     _need_cuda(sid_q, sid_k, ref)
-    Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), PRECISION[precision]
+    Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), _mlp_precision(precision)
     lib = _lib.load()
     dev = X.device
     sid_q, sid_k = sid_q.to(torch.int32).contiguous(), sid_k.to(torch.int32).contiguous()
@@ -716,7 +737,7 @@ def mlp_block_bwd(X: torch.Tensor, Y: torch.Tensor, params, sid_q: torch.Tensor,
     _need_cuda(sid_q, sid_k, loss, merged, state, col_lse)
     if col_lse is not None:
         col_lse = col_lse.detach().to(torch.float32).contiguous()
-    Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), PRECISION[precision]
+    Bq, Bk, est, prec = X.shape[0], Y.shape[0], _mlp_estimator(estimator), _mlp_precision(precision)
     dev = X.device
     sid_q, sid_k = sid_q.to(torch.int32).contiguous(), sid_k.to(torch.int32).contiguous()
     shapes = {"dX": (Bq, D), "dC_part": (Bk, H1), "dW1": (H1, 2 * D), "db1": (H1,), "dW2": (H2, H1), "db2": (H2,),
@@ -746,10 +767,10 @@ def mlp_input_grad(dZ: torch.Tensor, In: torch.Tensor, W1: torch.Tensor, side: i
         raise MIError("mlp_input_grad: dW1 must be a contiguous fp32 [H1, 2D] tensor")
     dIn = torch.empty((R, D), dtype=torch.float32, device=In.device)
     db1 = torch.empty(H1, dtype=torch.float32, device=In.device) if want_db1 else None
-    prec = PRECISION[precision]
+    prec = _mlp_precision(precision)
     nbytes = _lib.load().mi_mlp_input_grad_workspace_bytes(R, D, H1, prec)
     if nbytes == 0:
-        raise MIError("mi_mlp_input_grad_workspace_bytes: unsupported shape (D, H1 multiples of 8)")
+        raise MIError("mi_mlp_input_grad_workspace_bytes: unsupported shape (D, H1 multiples of 8; fp32: D, H1 <= 1280)")
     ws = workspace(nbytes, In.device)
     _check(_lib.load().mi_mlp_input_grad(_ptr(dZ), _ptr(In), _ptr(W1), int(side), R, D, H1, prec, _ptr(dIn), _ptr(dW1), _ptr(db1),
                                          _ptr(ws), ws.numel(), _stream()), "mi_mlp_input_grad")
@@ -759,17 +780,18 @@ def mlp_input_grad(dZ: torch.Tensor, In: torch.Tensor, W1: torch.Tensor, side: i
 def gdv(pos: torch.Tensor, neg: torch.Tensor, precision: str = "strict") -> torch.Tensor:
     """mi_gdv: fp64[4] = {gdv, intra_pos, intra_neg, inter} of two [N, D] fp32 embedding sets (validate.py:16-49)."""
     _need_cuda(pos, neg)
+    prec = _precision(precision)
     pos, neg = pos.detach().to(torch.float32).contiguous(), neg.detach().to(torch.float32).contiguous()
     if pos.dim() != 2 or neg.dim() != 2 or pos.shape[1] != neg.shape[1]:
         raise MIError("gdv needs two [N, D] matrices with the same D")
     lib = _lib.load()
     Np, Nn, D = pos.shape[0], neg.shape[0], pos.shape[1]
-    nbytes = lib.mi_gdv_workspace_bytes(Np, Nn, D, PRECISION[precision])
+    nbytes = lib.mi_gdv_workspace_bytes(Np, Nn, D, prec)
     if nbytes == 0:
         raise MIError("mi_gdv: unsupported shape (D multiple of 8, at least 2 samples per class)")
     ws = workspace(nbytes, pos.device)
     out = torch.empty(4, dtype=torch.float64, device=pos.device)
-    _check(lib.mi_gdv(_ptr(pos), _ptr(neg), Np, Nn, D, PRECISION[precision], _ptr(out), _ptr(ws), ws.numel(), _stream()), "mi_gdv")
+    _check(lib.mi_gdv(_ptr(pos), _ptr(neg), Np, Nn, D, prec, _ptr(out), _ptr(ws), ws.numel(), _stream()), "mi_gdv")
     return out
 
 
